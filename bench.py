@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W [--workload cg16384|gmres4096|...]
     python bench.py --impl reference --gpus N --steps K --warmup W
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR
 
 A "step" is ONE Krylov iteration.  The primary workload is BASELINE.json configs[3]:
 CG on the 16384 x 16384 Poisson grid (268 M unknowns), strong-scaled over N GPUs by
@@ -20,6 +21,12 @@ before the timed region; vectors (2.1 GB each) are far larger than the 126 MB L2
 L2 flush is needed between iterations.  Timing: CUDA events on the launching stream
 around exactly K iterations (tol = 0 so nothing converges early), barrier + device sync
 on both sides, MAX over ranks.
+
+`--dump-outputs DIR`: after the timed call, what it returned is written as DIR/<name>.npy (float64): the solution
+x (for more than 2^21 unknowns, its entries at up to 2^21 seeded random positions, which x_index lists), the iteration
+count, the final residual, the status and the residual history (GMRES: final_err, v_err, n_out, restart_out as
+well).  The inputs carry no randomness, so two builds run with the same arguments can be compared file by file.
+With several ranks, each writes its own slab's files with a _rank<r> suffix.
 
 `--impl reference`: the reference is Fortran and no Fortran compiler exists on the
 build or GPU box, so this arm times the C/OpenMP restatement of the reference's
@@ -158,6 +165,32 @@ def history_parity(name, hist, r0):
             "against": ref.get("source", ""), "detail": out}
 
 
+DUMP_SAMPLE = 1 << 21   # solution entries kept by --dump-outputs when x is longer (16 MB of float64)
+
+
+def solver_outputs(r):
+    """What a caller of the timed solver call receives (x and the result fields beside it) as float64 host arrays.
+    An x longer than DUMP_SAMPLE is reduced to the entries at a fixed, seeded set of positions, stored as x_index."""
+    import dataclasses
+    import numpy as np
+    import torch
+
+    out = {}
+    for f in dataclasses.fields(r):
+        v = getattr(r, f.name)
+        if f.name == "stats":
+            continue
+        if f.name == "x":
+            if v.numel() > DUMP_SAMPLE:
+                idx = np.unique(np.random.default_rng(0).integers(0, v.numel(), DUMP_SAMPLE))
+                out["x_index"] = idx.astype(np.float64)
+                v = v[torch.from_numpy(idx).to(v.device)]
+            out["x"] = v.cpu().numpy().astype(np.float64)
+        else:
+            out[f.name] = np.asarray(v, dtype=np.float64)
+    return out
+
+
 def make_ops(kl, w):
     A = kl.aniso(*w["aniso"]) if w.get("aniso") else kl.stvec
     M = kl.cbpr2 if w["pc"] == "cbpr2" else (kl.cheb(int(w["pc"][4:])) if (w["pc"] or "").startswith("cheb") else None)
@@ -227,7 +260,7 @@ def gpu_arm(args):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         return float(t.item())
 
-    def measure(name, steps, warmup, with_e2e, with_profile):
+    def measure(name, steps, warmup, with_e2e, with_profile, keep_outputs=False):
         w = WORKLOADS[name]
         nx = w["nx"]
         ny = w["ny"] * (world if w["scaling"] == "weak" else 1)   # global lines
@@ -249,6 +282,7 @@ def gpu_arm(args):
         r = run_gpu_solver(kl, h, w, b, nx, ny, steps_eff)               # timed: events inside the library
         barrier()
         clocks = smp.stop() if rank == 0 else None
+        outputs = solver_outputs(r) if keep_outputs else None
         ms = max_over_ranks(r.stats["solve_ms"])
         its = r.stats["iterations"]
         launches = r.stats["kernel_launches"]
@@ -257,7 +291,7 @@ def gpu_arm(args):
         out = dict(workload=name, iterations=its, ms=ms, ms_per_step=ms / max(its, 1), parity=parity,
                    its_per_s=its / (ms * 1e-3), launches=int(launches), clocks=clocks,
                    bytes_per_iter=r.stats["algorithmic_bytes"] / max(its, 1) * world,
-                   n_unknowns=nx * ny, nx=nx, ny=ny)
+                   n_unknowns=nx * ny, nx=nx, ny=ny, outputs=outputs)
         peak, which = load_peaks()
         out["roofline_iter"] = dict(
             bound="hbm", achieved=r.stats["algorithmic_bytes"] / (ms * 1e-3) / 1e9, peak=peak, unit="GB/s",
@@ -333,7 +367,12 @@ def gpu_arm(args):
                                    "value_pageable_host = the same with ordinary (pageable) host arrays")
         return out
 
-    primary = measure(args.workload, args.steps, args.warmup, True, True)
+    primary = measure(args.workload, args.steps, args.warmup, True, True, keep_outputs=bool(args.dump_outputs))
+    if args.dump_outputs:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        suffix = f"_rank{rank}" if world > 1 else ""
+        for k, v in primary["outputs"].items():
+            np.save(os.path.join(args.dump_outputs, f"{k}{suffix}.npy"), v)
     extras = {}
     if world == 1 and args.extras:
         for name, st in (("gmres4096", 95), ("gmres4096sel", 95), ("pcg16384", args.steps), ("bicgstab8192", args.steps),
@@ -429,7 +468,7 @@ def cpu_baseline(workload, budget_s=20.0, threads=None, with_six=True):
            "sample": f"{w['solver']} on {ns}x{ns}: ({i1}-{i0}) iterations, time difference of two runs "
                      f"({t_long:.2f}s - {t_short:.2f}s) so that allocation/first-touch cancels; "
                      f"oracle/krylov_oracle.c, gcc -O3 -fopenmp -march=native -funroll-loops built on this box "
-                     f"({os.path.relpath(so, ROOT)}), OMP threads = {cores}"}
+                     f"({os.path.basename(so)}), OMP threads = {cores}"}
     if with_six and cores > 6:
         r6, j0, j1, _, _ = rate(6, budget_s * 0.4)
         out["value_6_threads"] = r6
@@ -471,7 +510,12 @@ def main():
     ap.add_argument("--only-extras", default="", help="comma-separated subset of the extra workloads")
     ap.add_argument("--no-cpu-baseline", dest="cpu_baseline", action="store_false")
     ap.add_argument("--cpu-budget", type=float, default=20.0)
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write what the timed solver call returned (x, iteration counts, residual history) "
+                         "as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU implementation")
     if args.impl == "reference":
         reference_arm(args)
     else:

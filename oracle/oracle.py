@@ -9,6 +9,7 @@ from __future__ import annotations
 import ctypes as C
 import os
 import subprocess
+import tempfile
 from dataclasses import dataclass, field
 
 import numpy as np
@@ -34,15 +35,19 @@ def build(force: bool = False) -> str:
 _lib = None
 
 
+_native_dir = None
+
+
 def build_native() -> str:
     """A copy built with -march=native (the reference's own flag, CMakeLists.txt:5) on THIS machine, for timing
-    the CPU baseline on the box it runs on.  The portable x86-64-v3 build stays the checker.  Returns the path
-    (or the portable library's path if the compiler is missing)."""
-    global _SO, _lib
-    out_dir = os.path.join(_HERE, "_native")
-    so = os.path.join(out_dir, "libkrylov_oracle.so")
+    the CPU baseline on the box it runs on.  The portable x86-64-v3 build stays the checker.  The copy goes to a
+    temporary directory (removed at exit), so that the source tree may be read-only.  Returns the path (or the
+    portable library's path if the compiler is missing)."""
+    global _SO, _lib, _native_dir
     try:
-        os.makedirs(out_dir, exist_ok=True)
+        if _native_dir is None:
+            _native_dir = tempfile.TemporaryDirectory(prefix="krylov_oracle_native_")
+        so = os.path.join(_native_dir.name, "libkrylov_oracle.so")
         subprocess.check_call(
             ["gcc", "-O3", "-fopenmp", "-march=native", "-funroll-loops", "-ffp-contract=off", "-fPIC", "-std=gnu11",
              "-shared", "-o", so, os.path.join(_HERE, "krylov_oracle.c"), os.path.join(_HERE, "krylov_extras.c"), "-lm"],
@@ -56,7 +61,7 @@ def build_native() -> str:
 def lib():
     global _lib
     if _lib is None:
-        if not _SO.endswith(os.path.join("_native", "libkrylov_oracle.so")):
+        if _native_dir is None or not _SO.startswith(_native_dir.name):
             build()
         L = C.CDLL(_SO)
         for name in ("ko_get_stvec", "ko_get_stv_poisson", "ko_get_aniso"):

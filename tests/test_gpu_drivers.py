@@ -92,13 +92,14 @@ def test_restart_sweep_and_grid_sweep_and_strong_scaling(ko):
 
 def test_fortran_shim_compiles_and_reference_driver_runs():
     """fortran/krylov_b200.f90 (ISO_C_BINDING shim with the reference's module names) + the reference's own
-    tests/test_poisson_mf.f90, when a Fortran compiler and the reference tree are present."""
+    tests/test_poisson_mf.f90, when a Fortran compiler exists and KRYLOV_REFERENCE names the reference's source tree
+    (it is not part of this repository)."""
     fc = shutil.which("gfortran") or shutil.which("flang") or shutil.which("nvfortran")
-    ref = os.environ.get("KRYLOV_REFERENCE", "/root/reference")
+    ref = os.environ.get("KRYLOV_REFERENCE", "")
     if not fc:
         pytest.skip("no Fortran compiler in this image (gfortran / flang / nvfortran all absent)")
-    if not os.path.exists(os.path.join(ref, "tests", "test_poisson_mf.f90")):
-        pytest.skip("reference tree not present on this box")
+    if not ref or not os.path.exists(os.path.join(ref, "tests", "test_poisson_mf.f90")):
+        pytest.skip("set KRYLOV_REFERENCE to the reference's source tree (AlexanderGSC/gmres) to run its driver")
     import tempfile
     with tempfile.TemporaryDirectory() as td:
         exe = os.path.join(td, "test_poisson_mf")
