@@ -4,7 +4,8 @@
 // All four share one device implementation (the serial and OpenMP variants
 // compute the same quantities; only their summation order differs).
 //
-// Plain CG (default): 64n B per iteration, see FCgDirX2 / FCgRUpdate below (A applied twice, A p never stored).
+// Plain CG, one GPU, from 2^20 unknowns on (default): 48n B per iteration, ONE temporally blocked pass (ChCg below).
+// Plain CG otherwise: 64n B per iteration, see FCgDirX2 / FCgRUpdate below (A applied twice, A p never stored).
 // KL_OPT_CHAIN = 0 and PCG + cbpr2 -- per iteration 72n B for CG and 80n B for PCG + cbpr2:
 //   K1  x += alpha_prev*p ; p' = z + beta*p ; ax = A p' ; ax.p'   reads z,p,x  writes p',ax,x   48n B
 //   K2  r -= alpha ax ; r.r                                       reads r,ax   writes r         24n B
@@ -135,6 +136,87 @@ struct FCgRUpdate : StencilBase<2, 1> {
     }
 };
 
+// ---- plain CG in ONE pass per iteration (48n B, KL_OPT_CG_ONEPASS) ----------------------------------------
+// A two-level temporally blocked chain (kl_chain_tma.cuh).  State at the start of pass k: r_k, p_k, x_k in HBM,
+// alpha_k and beta_k in S[]:
+//   level 0: u = p_k
+//   level 1: A p_k ; r_{k+1} = r_k - alpha_k A p_k ; p_{k+1} = r_{k+1} + beta_k p_k       stores r_{k+1}, p_{k+1}
+//   level 2: A p_{k+1} ; x_{k+1} = x_k + alpha_k p_k (x_k: side input, p_k re-read from the ring)   stores x_{k+1}
+//            sums rho = r'.r', gamma = p'.Ap', sigma = r'.Ap', delta = Ap'.Ap'
+// reads r, p, x and writes r', p', x'.  The point-wise operations are the two-kernel path's fmas on the same
+// operands; only beta differs: PostCgOnePass predicts ||r_{k+2}||^2 from the sums of this pass instead of taking
+// it from the next one (one reduction per iteration), see DESIGN.md section 3.2.
+struct ChCg : ChainBase<2, 2, 1, 4> {
+    static constexpr int NSIDE = 1;     // side[0] = x_k (read at the last level's output points only)
+    double *r_new, *p_new, *x_new;
+    const double *S;
+    double alpha, beta;
+    __device__ __forceinline__ void init() {
+        alpha = S[S_ALPHA];
+        beta = S[S_BETA];
+    }
+    __device__ __forceinline__ void level0(bool, size_t, const double (&raw)[2][2], double (&u)[2],
+                                           double (&cc)[1][2], double *) const {
+#pragma unroll
+        for (int e = 0; e < 2; ++e) {
+            u[e] = raw[1][e];
+            cc[0][e] = 0.0;
+        }
+    }
+    template <class RAW>
+    __device__ __forceinline__ void level(int lv, bool out, size_t idx, const double (&up)[2], const double (&au)[2],
+                                          const double (&cin)[1][2], RAW raw, const double (&sd)[1][2], double (&u)[2],
+                                          double (&cout)[1][2], double *acc) const {
+        if (lv == 1) {
+            const double2 rv = raw(0), pv = raw(1);
+            const double r2[2] = {rv.x, rv.y}, p2[2] = {pv.x, pv.y};
+#pragma unroll
+            for (int e = 0; e < 2; ++e) {
+                cout[0][e] = fma(-alpha, au[e], r2[e]);                                  // cg.f90:130
+                u[e] = fma(beta, p2[e], cout[0][e]);                                     // direction update
+            }
+            if (out) {
+                stg2(r_new + idx, cout[0][0], cout[0][1]);
+                stg2(p_new + idx, u[0], u[1]);
+            }
+        } else {
+            u[0] = u[1] = 0.0;
+            cout[0][0] = cout[0][1] = 0.0;
+            if (out) {
+                const double2 pv = raw(1);
+                const double p2[2] = {pv.x, pv.y};
+                double xn[2];
+#pragma unroll
+                for (int e = 0; e < 2; ++e) {
+                    xn[e] = fma(alpha, p2[e], sd[0][e]);                                 // cg.f90:128
+                    acc[0] = fma(cin[0][e], cin[0][e], acc[0]);                          // rho   = r'.r'
+                    acc[1] = fma(au[e], up[e], acc[1]);                                  // gamma = p'.Ap'
+                    acc[2] = fma(au[e], cin[0][e], acc[2]);                              // sigma = r'.Ap'
+                    acc[3] = fma(au[e], au[e], acc[3]);                                  // delta = Ap'.Ap'
+                }
+                stg2(x_new + idx, xn[0], xn[1]);
+            }
+        }
+    }
+};
+
+// Prologue of the one-pass path: the four sums of ChCg's last level for p_0 = r_0 (= b), no store.
+struct FCgOnePassInit : StencilBase<1, 4> {
+    __device__ __forceinline__ void init() {}
+    __device__ __forceinline__ double point(const double (&v)[1]) const { return v[0]; }
+    template <int VEC>
+    __device__ __forceinline__ void store(size_t, const double (&)[1][VEC], const double (&cu)[VEC],
+                                          const double (&au)[VEC], double *acc) const {
+#pragma unroll
+        for (int v = 0; v < VEC; ++v) {
+            acc[0] = fma(cu[v], cu[v], acc[0]);
+            acc[1] = fma(au[v], cu[v], acc[1]);
+            acc[2] = fma(au[v], cu[v], acc[2]);
+            acc[3] = fma(au[v], au[v], acc[3]);
+        }
+    }
+};
+
 // K2 without x: r -= alpha ax ; acc0 = sum r*r     (cg.f90:130-133)
 struct PCgUpdateR : PwBase<1> {
     double *r;
@@ -188,6 +270,11 @@ struct FPcgUpdateR : StencilBase<2, 2> {
     }
 };
 
+// KL_OPT_CG_ONEPASS = -1: the one-pass path from this many unknowns on.  It won at every size of the sweep, 1.33x at
+// 1024^2 .. 1.79x at 2048^2 (scripts/cg_onepass_sweep.py, profiles/r03_cg_onepass_sweep.json); the grids below 1 Mi
+// unknowns (vectors resident in L2, not swept) keep the two-kernel iteration.
+constexpr size_t kCgOnePassMin = (size_t)1 << 20;
+
 static int cg_solve(Ctx *c, const kl_operator_t *A, const double *b, double *x, int nx, int ny,
                     double tol, int *iter, double *res_out, const kl_precond_t *M, const double *params,
                     int nparams) {
@@ -207,6 +294,10 @@ static int cg_solve(Ctx *c, const kl_operator_t *A, const double *b, double *x, 
     const bool fuse_pc = fused && P.pc.kind == KL_PC_CBPR2;   // update + cbpr2 in one pass
     const bool defer_x = fused && (!prec || fuse_pc);         // x update folded into the next K1 (72n / 80n B)
     const bool twice = defer_x && !prec && c->opt_chain;       // plain CG: apply A twice, never store A p (64n B)
+    // plain CG in one chain pass per iteration (48n B): single GPU (the chain needs a two-line halo, which the
+    // multi-GPU producer-push protocol does not deliver)
+    const bool onepass = twice && c->nranks == 1 && chain_ok(&P, 2) &&
+                         (c->opt_cg_onepass > 0 || (c->opt_cg_onepass < 0 && n >= kCgOnePassMin));
     const int nvec = 4 + (dev ? 0 : 1) + (prec ? 3 : 0) + ((fuse_pc || twice) ? 1 : 0) + (twice ? 1 : 0);
     KL_TRY(ws_reserve(c, nvec * ws_need(n)));
     ws_reset(c);
@@ -216,6 +307,9 @@ static int cg_solve(Ctx *c, const kl_operator_t *A, const double *b, double *x, 
     double *z = r, *aux = nullptr, *aux2 = nullptr;
     double *r_alt = (fuse_pc || twice) ? ws_take<double>(c, n) : nullptr;
     double *x_cur = dx, *x_alt = twice ? ws_take<double>(c, n) : nullptr;
+    // one-pass: x is ping-ponged from the first iteration on; start it where an odd / even maxit ends in dx
+    if (onepass && (maxit & 1)) std::swap(x_cur, x_alt);
+    double *const x_start = x_cur, *const x_other = x_alt;
     const Cbpr2Coef cf = fuse_pc ? cbpr2_coef(P.params) : Cbpr2Coef{1.0, 0.0};
     if (prec) {
         z = ws_take<double>(c, n);
@@ -224,7 +318,7 @@ static int cg_solve(Ctx *c, const kl_operator_t *A, const double *b, double *x, 
     }
     // x0 = 0 ; r0 = b ; p0 = r0 (cg.f90:102-108)
     KL_TRY(stage_in(c, r, b, n));
-    KL_CUDA(c, cudaMemsetAsync(dx, 0, n * sizeof(double), c->stream));
+    KL_CUDA(c, cudaMemsetAsync(x_cur, 0, n * sizeof(double), c->stream));
     KL_CUDA(c, cudaMemsetAsync(p0, 0, n * sizeof(double), c->stream));
     KL_CUDA(c, cudaMemsetAsync(c->d_I, 0, sizeof(int) * I_COUNT, c->stream));
     {
@@ -244,8 +338,16 @@ static int cg_solve(Ctx *c, const kl_operator_t *A, const double *b, double *x, 
         KL_TRY(comm_push_lines(c, 2, first, last, slots, 0, P.nx));
     }
     // rr = r.z  (z = M^-1 r for pcg, cg.f90:182 ; z = r otherwise)
+    // one-pass: rr, p.Ap, r.Ap and Ap.Ap for p_0 = r_0, then alpha_0 and the predicted beta_0
     if (prec) {
         KL_TRY(pc_apply(&P, r, z, aux, aux2, 2, false, PostStoreRed{c->d_S, S_RR, 0}));
+    } else if (onepass) {
+        Halo H{};
+        const double *vecs[1] = {r};
+        FCgOnePassInit d;
+        set_io(d, &P, vecs, H);
+        set_gate(d, c, false);
+        KL_TRY(launch_stencil(c, &P.op, d, P.nx, P.nyl, PostCgOnePassInit{c->d_S}));
     } else {
         PDot2 d;
         set_gate(d, c, false);
@@ -263,6 +365,24 @@ static int cg_solve(Ctx *c, const kl_operator_t *A, const double *b, double *x, 
     auto enqueue_iterations = [&](const int done0, const int batch) -> int {
         const int done = done0;
         for (int k = 0; k < batch; ++k) {
+            if (onepass) {
+                // pass 0 reads r_0 as p_0 as well; from then on p alternates between p1 (odd passes write it)
+                // and p0
+                ProfScope ps(c, 0, "cg_onepass (chain: r-=alpha*A p; p=r+beta*p; x+=alpha*p; A p; 4 dots)", 48.0 * n);
+                Halo H{};
+                const double *vecs[2] = {r, done + k == 0 ? r : pold};
+                ChCg f;
+                set_io(f, &P, vecs, H);
+                set_gate(f, c, true);
+                f.side[0] = x_cur;
+                f.r_new = r_alt; f.p_new = pnew; f.x_new = x_alt; f.S = c->d_S;
+                KL_TRY(launch_chain(c, &P.op, f, P.nx, P.nyl, PostCgOnePass{c->d_S, c->d_I, c->d_hist, c->hist_cap}));
+                std::swap(r, r_alt);
+                std::swap(x_cur, x_alt);
+                std::swap(pold, pnew);
+                z = r;
+                continue;
+            }
             // ---- K1
             if (twice) {
                 Halo H;
@@ -389,7 +509,8 @@ static int cg_solve(Ctx *c, const kl_operator_t *A, const double *b, double *x, 
             GraphKey gk;
             gk.add('C').add(nx).add(ny).add(batch).add(P.op.kind).add(P.op.eps_x).add(P.op.eps_y).add(P.pc.kind)
                 .add(P.pc.degree).add(P.params).add(c->opt_tma).add(c->opt_chain).add(c->opt_stencil_rows)
-                .add(c->opt_stencil_tail).add(c->opt_stencil_stagger).add(c->opt_pdl).add(c->ws).add(dx).add(r).add(pold);
+                .add(c->opt_stencil_tail).add(c->opt_stencil_stagger).add(c->opt_pdl).add(c->ws).add(dx).add(r).add(pold)
+                .add(x_cur).add(onepass).add(onepass && done == 0);     // (one-pass: iteration 1 reads r as p)
             ge = graph_find(c, gk.s);
             if (!ge && polls >= 1) {     // the first batch of a handle's first solve runs eagerly
                 const long long l0 = c->stats.kernel_launches;
@@ -419,7 +540,14 @@ static int cg_solve(Ctx *c, const kl_operator_t *A, const double *b, double *x, 
             break;
         }
     }
-    if (defer_x) {
+    if (onepass) {
+        // no deferred update: after `its` passes x is in x_start (even) or the other buffer (odd); the passes
+        // after the convergence step were gated off
+        if (status == KL_NOT_CONVERGED) KL_TRY(read_back(c));     // (maxit = 0: no poll ran)
+        const int its_done = c->h_pinned_i[I_ITER];
+        const double *xres = (its_done & 1) ? x_other : x_start;
+        if (xres != dx) KL_CUDA(c, cudaMemcpyAsync(dx, xres, n * sizeof(double), cudaMemcpyDeviceToDevice, c->stream));
+    } else if (defer_x) {
         // flush the pending x += alpha p of the last executed iteration (kernels after the convergence step
         // were gated off, so S_ALPHA and the p buffer of that iteration are intact).  Iteration i wrote its
         // direction into p1 for odd i and into p0 for even i.
@@ -450,7 +578,7 @@ static int cg_solve(Ctx *c, const kl_operator_t *A, const double *b, double *x, 
     c->stats.cycles = polls;
     c->stats.solve_ms = ms;
     c->stats.total_ms = ms_tot;
-    c->stats.algorithmic_bytes = (double)its * (fuse_pc ? 80.0 : (prec ? 96.0 : (twice ? 64.0 : (defer_x ? 72.0 : 80.0)))) * (double)n;
+    c->stats.algorithmic_bytes = (double)its * (fuse_pc ? 80.0 : (prec ? 96.0 : (onepass ? 48.0 : (twice ? 64.0 : (defer_x ? 72.0 : 80.0))))) * (double)n;
     *res_out = c->h_pinned[S_RES];
     if (status == KL_OK) *iter = c->h_pinned_i[I_CONV_AT];   // count on exit; unchanged if not converged
     return status;

@@ -156,6 +156,7 @@ struct kl_context_s {
     int opt_stencil_stagger = 0; // staggered tile heights (KL_OPT_STENCIL_STAGGER): measured neutral, off by default
     int opt_stencil_tail = -1;  // lines per CTA in the tapered tail (-1 auto, 0 off), KL_OPT_STENCIL_TAIL
     int opt_pdl = 1;            // programmatic dependent launch between the fused CG kernels (KL_OPT_PDL)
+    int opt_cg_onepass = -1;    // plain CG in one chain pass per iteration (KL_OPT_CG_ONEPASS): -1 auto, 0 off, 1 on
     // comm
     int rank = 0, nranks = 1;
     void *nccl_comm = nullptr;

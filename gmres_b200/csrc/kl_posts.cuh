@@ -42,6 +42,18 @@ struct PostCgAlpha {  // cg.f90:124-126  alpha = rr / (ax.p)
     }
 };
 
+// end of a CG iteration: residual, history, convergence test (cg.f90:135-149)
+__device__ __forceinline__ void cg_record(double *S, int *I, double *hist, int hist_cap, double res) {
+    S[S_RES] = res;
+    int it = I[I_ITER] + 1;
+    I[I_ITER] = it;
+    int hl = I[I_HIST];
+    if (hl < hist_cap) hist[hl] = res;
+    I[I_HIST] = hl + 1;
+    if (res < S[S_TOL]) I[I_CONV_AT] = it;          // cg.f90:144-149
+    else if (!(res == res)) { I[I_BREAKDOWN] = 1; I[I_CONV_AT] = it; }
+}
+
 struct PostCgEnd {
     double *S;
     int *I;
@@ -52,17 +64,36 @@ struct PostCgEnd {
     __device__ __forceinline__ void run() const {
         double num = precond == 2 ? S[S_RED + 1] : S[S_RED];
         double rr2 = precond == 1 ? S[S_TMP0] : S[S_RED];
-        double res = sqrt(rr2);
         S[S_BETA] = num / S[S_RR];
         S[S_RR] = num;
-        S[S_RES] = res;
-        int it = I[I_ITER] + 1;
-        I[I_ITER] = it;
-        int hl = I[I_HIST];
-        if (hl < hist_cap) hist[hl] = res;
-        I[I_HIST] = hl + 1;
-        if (res < S[S_TOL]) I[I_CONV_AT] = it;          // cg.f90:144-149
-        else if (!(res == res)) { I[I_BREAKDOWN] = 1; I[I_CONV_AT] = it; }
+        cg_record(S, I, hist, hist_cap, sqrt(rr2));
+    }
+};
+
+// One-pass CG (ChCg, kl_cg.cu).  S_RED = rho = r.r, gamma = p.Ap, sigma = r.Ap, delta = Ap.Ap of the iterate the
+// pass produced.  alpha = rho / gamma is the reference's formula on true dot products (cg.f90:124-126).  beta needs
+// ||r - alpha Ap||^2, the next pass's r.r; it is predicted by expanding the square, rho - 2 alpha sigma +
+// alpha^2 delta, so that the next pass can form the direction in the same sweep.
+__device__ __forceinline__ void cg_onepass_scalars(double *S) {
+    const double rho = S[S_RED], gam = S[S_RED + 1], sig = S[S_RED + 2], del = S[S_RED + 3];
+    const double alpha = rho / gam;
+    S[S_PAP] = gam;
+    S[S_ALPHA] = alpha;
+    S[S_BETA] = (rho - 2.0 * alpha * sig + alpha * alpha * del) / rho;
+    S[S_RR] = rho;
+}
+struct PostCgOnePassInit {   // after the prologue (sums of r_0 = p_0): alpha_0, beta_0
+    double *S;
+    __device__ __forceinline__ void run() const { cg_onepass_scalars(S); }
+};
+struct PostCgOnePass {       // after a pass: PostCgEnd's bookkeeping on the true ||r||, then alpha and beta
+    double *S;
+    int *I;
+    double *hist;
+    int hist_cap;
+    __device__ __forceinline__ void run() const {
+        cg_onepass_scalars(S);
+        cg_record(S, I, hist, hist_cap, sqrt(S[S_RED]));
     }
 };
 
@@ -141,7 +172,7 @@ struct PostLanBeta {
     }
 };
 
-enum PostKind { PK_NoPost, PK_PostStoreRed, PK_PostCgAlpha, PK_PostCgEnd, PK_PostBeta, PK_PostMgs, PK_PostHh, PK_PostBiAlpha, PK_PostBiOmega, PK_PostBiEnd, PK_PostLanAlpha, PK_PostLanBeta };
+enum PostKind { PK_NoPost, PK_PostStoreRed, PK_PostCgAlpha, PK_PostCgEnd, PK_PostCgOnePassInit, PK_PostCgOnePass, PK_PostBeta, PK_PostMgs, PK_PostHh, PK_PostBiAlpha, PK_PostBiOmega, PK_PostBiEnd, PK_PostLanAlpha, PK_PostLanBeta };
 struct PostAny {
     int kind;
     union U {
@@ -149,6 +180,8 @@ struct PostAny {
         PostStoreRed v_PostStoreRed;
         PostCgAlpha v_PostCgAlpha;
         PostCgEnd v_PostCgEnd;
+        PostCgOnePassInit v_PostCgOnePassInit;
+        PostCgOnePass v_PostCgOnePass;
         PostBeta v_PostBeta;
         PostMgs v_PostMgs;
         PostHh v_PostHh;
@@ -167,6 +200,8 @@ struct PostAny {
             case PK_PostStoreRed: u.v_PostStoreRed.run(); break;
             case PK_PostCgAlpha: u.v_PostCgAlpha.run(); break;
             case PK_PostCgEnd: u.v_PostCgEnd.run(); break;
+            case PK_PostCgOnePassInit: u.v_PostCgOnePassInit.run(); break;
+            case PK_PostCgOnePass: u.v_PostCgOnePass.run(); break;
             case PK_PostBeta: u.v_PostBeta.run(); break;
             case PK_PostMgs: u.v_PostMgs.run(); break;
             case PK_PostHh: u.v_PostHh.run(); break;
@@ -201,6 +236,18 @@ inline PostAny to_any(const PostCgEnd &p) {
     PostAny a;
     a.kind = PK_PostCgEnd;
     a.u.v_PostCgEnd = p;
+    return a;
+}
+inline PostAny to_any(const PostCgOnePassInit &p) {
+    PostAny a;
+    a.kind = PK_PostCgOnePassInit;
+    a.u.v_PostCgOnePassInit = p;
+    return a;
+}
+inline PostAny to_any(const PostCgOnePass &p) {
+    PostAny a;
+    a.kind = PK_PostCgOnePass;
+    a.u.v_PostCgOnePass = p;
     return a;
 }
 inline PostAny to_any(const PostBeta &p) {
