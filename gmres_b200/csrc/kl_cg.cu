@@ -4,7 +4,9 @@
 // All four share one device implementation (the serial and OpenMP variants
 // compute the same quantities; only their summation order differs).
 //
-// Plain CG, one GPU, from 2^20 unknowns on (default): 48n B per iteration, ONE temporally blocked pass (ChCg below).
+// Plain CG, one GPU, from 2^24 unknowns on (default): 36n B per iteration, PAIRS of temporally blocked passes
+//   (24n + 48n, ChCgPass<kCgPairA / kCgPairB> below; p and x are stored every second iteration only).
+// Plain CG, one GPU, 2^20 .. 2^24 unknowns (default): 48n B per iteration, ONE temporally blocked pass (ChCg below).
 // Plain CG otherwise: 64n B per iteration, see FCgDirX2 / FCgRUpdate below (A applied twice, A p never stored).
 // KL_OPT_CHAIN = 0 and PCG + cbpr2 -- per iteration 72n B for CG and 80n B for PCG + cbpr2:
 //   K1  x += alpha_prev*p ; p' = z + beta*p ; ax = A p' ; ax.p'   reads z,p,x  writes p',ax,x   48n B
@@ -136,7 +138,7 @@ struct FCgRUpdate : StencilBase<2, 1> {
     }
 };
 
-// ---- plain CG in ONE pass per iteration (48n B, KL_OPT_CG_ONEPASS) ----------------------------------------
+// ---- plain CG in ONE pass per iteration (48n B, KL_OPT_CG_ONEPASS = 1) -------------------------------------
 // A two-level temporally blocked chain (kl_chain_tma.cuh).  State at the start of pass k: r_k, p_k, x_k in HBM,
 // alpha_k and beta_k in S[]:
 //   level 0: u = p_k
@@ -146,20 +148,38 @@ struct FCgRUpdate : StencilBase<2, 1> {
 // reads r, p, x and writes r', p', x'.  The point-wise operations are the two-kernel path's fmas on the same
 // operands; only beta differs: PostCgOnePass predicts ||r_{k+2}||^2 from the sums of this pass instead of taking
 // it from the next one (one reduction per iteration), see DESIGN.md section 3.2.
-struct ChCg : ChainBase<2, 2, 1, 4> {
-    static constexpr int NSIDE = 1;     // side[0] = x_k (read at the last level's output points only)
+//
+// ---- plain CG in PAIRS of passes (36n B per iteration, KL_OPT_CG_ONEPASS = 2) ------------------------------
+// p_{k+1} = fma(beta_k, p_k, r_{k+1}) is one fma of two vectors that are in HBM anyway, and x feeds nothing in the
+// recurrence.  So only every second pass stores p and x:
+//   pass A (k -> k+1): the one-pass levels without the p and x stores           reads r_k, p_k        writes r_{k+1}
+//   pass B (k+1 -> k+2): level 0 rebuilds u = p_{k+1} = fma(beta_k, p_k, r_{k+1}); level 1 as above with p_{k+1}
+//     = u; level 2 rebuilds p_{k+1} at its output points and stores x_{k+2} = x_k + alpha_k p_k + alpha_{k+1} p_{k+1}
+//     as the two fmas of two one-pass iterations              reads r_{k+1}, p_k, x_k   writes r_{k+2}, p_{k+2}, x_{k+2}
+// 24n + 48n B per pair.  Every stored value and every sum is the one-pass path's fma chain on the same operands,
+// and NIN, L (hence the CTA grid and the block-partial reduction order) are ChCg's: the results are bit-identical.
+// Pass B takes alpha_k, beta_k from S_ALPHA_PREV / S_BETA_PREV (cg_onepass_scalars).
+enum CgPass { kCgOne, kCgPairA, kCgPairB };
+template <int MODE>
+struct ChCgPass : ChainBase<2, 2, 1, 4> {
+    static constexpr int NSIDE = MODE == kCgPairA ? 0 : 1;   // side[0] = x_k (read at the last level's output points)
     double *r_new, *p_new, *x_new;
     const double *S;
     double alpha, beta;
+    double alpha0, beta0;     // pass B: alpha_k, beta_k of the pair's first iteration
     __device__ __forceinline__ void init() {
         alpha = S[S_ALPHA];
         beta = S[S_BETA];
+        if (MODE == kCgPairB) {
+            alpha0 = S[S_ALPHA_PREV];
+            beta0 = S[S_BETA_PREV];
+        }
     }
     __device__ __forceinline__ void level0(bool, size_t, const double (&raw)[2][2], double (&u)[2],
                                            double (&cc)[1][2], double *) const {
 #pragma unroll
         for (int e = 0; e < 2; ++e) {
-            u[e] = raw[1][e];
+            u[e] = MODE == kCgPairB ? fma(beta0, raw[1][e], raw[0][e]) : raw[1][e];       // p_{k+1} : p_k
             cc[0][e] = 0.0;
         }
     }
@@ -173,32 +193,44 @@ struct ChCg : ChainBase<2, 2, 1, 4> {
 #pragma unroll
             for (int e = 0; e < 2; ++e) {
                 cout[0][e] = fma(-alpha, au[e], r2[e]);                                  // cg.f90:130
-                u[e] = fma(beta, p2[e], cout[0][e]);                                     // direction update
+                u[e] = fma(beta, MODE == kCgPairB ? up[e] : p2[e], cout[0][e]);          // direction update
             }
             if (out) {
                 stg2(r_new + idx, cout[0][0], cout[0][1]);
-                stg2(p_new + idx, u[0], u[1]);
+                if (MODE != kCgPairA) stg2(p_new + idx, u[0], u[1]);
             }
         } else {
             u[0] = u[1] = 0.0;
             cout[0][0] = cout[0][1] = 0.0;
             if (out) {
-                const double2 pv = raw(1);
-                const double p2[2] = {pv.x, pv.y};
-                double xn[2];
 #pragma unroll
                 for (int e = 0; e < 2; ++e) {
-                    xn[e] = fma(alpha, p2[e], sd[0][e]);                                 // cg.f90:128
                     acc[0] = fma(cin[0][e], cin[0][e], acc[0]);                          // rho   = r'.r'
                     acc[1] = fma(au[e], up[e], acc[1]);                                  // gamma = p'.Ap'
                     acc[2] = fma(au[e], cin[0][e], acc[2]);                              // sigma = r'.Ap'
                     acc[3] = fma(au[e], au[e], acc[3]);                                  // delta = Ap'.Ap'
                 }
-                stg2(x_new + idx, xn[0], xn[1]);
+                if (MODE != kCgPairA) {
+                    const double2 pv = raw(1);
+                    const double p2[2] = {pv.x, pv.y};
+                    double xn[2];
+                    if (MODE == kCgPairB) {
+                        const double2 rv = raw(0);
+                        const double r2[2] = {rv.x, rv.y};
+#pragma unroll
+                        for (int e = 0; e < 2; ++e)                                      // cg.f90:128, twice
+                            xn[e] = fma(alpha, fma(beta0, p2[e], r2[e]), fma(alpha0, p2[e], sd[0][e]));
+                    } else {
+#pragma unroll
+                        for (int e = 0; e < 2; ++e) xn[e] = fma(alpha, p2[e], sd[0][e]);    // cg.f90:128
+                    }
+                    stg2(x_new + idx, xn[0], xn[1]);
+                }
             }
         }
     }
 };
+using ChCg = ChCgPass<kCgOne>;
 
 // Prologue of the one-pass path: the four sums of ChCg's last level for p_0 = r_0 (= b), no store.
 struct FCgOnePassInit : StencilBase<1, 4> {
@@ -274,6 +306,9 @@ struct FPcgUpdateR : StencilBase<2, 2> {
 // 1024^2 .. 1.79x at 2048^2 (scripts/cg_onepass_sweep.py, profiles/r03_cg_onepass_sweep.json); the grids below 1 Mi
 // unknowns (vectors resident in L2, not swept) keep the two-kernel iteration.
 constexpr size_t kCgOnePassMin = (size_t)1 << 20;
+// ... and pairs of passes (36n B per iteration) from this many on (scripts/cg_pair_sweep.py,
+// profiles/r04_cg_pair_sweep.json).
+constexpr size_t kCgPairMin = (size_t)1 << 24;
 
 static int cg_solve(Ctx *c, const kl_operator_t *A, const double *b, double *x, int nx, int ny,
                     double tol, int *iter, double *res_out, const kl_precond_t *M, const double *params,
@@ -294,10 +329,12 @@ static int cg_solve(Ctx *c, const kl_operator_t *A, const double *b, double *x, 
     const bool fuse_pc = fused && P.pc.kind == KL_PC_CBPR2;   // update + cbpr2 in one pass
     const bool defer_x = fused && (!prec || fuse_pc);         // x update folded into the next K1 (72n / 80n B)
     const bool twice = defer_x && !prec && c->opt_chain;       // plain CG: apply A twice, never store A p (64n B)
-    // plain CG in one chain pass per iteration (48n B): single GPU (the chain needs a two-line halo, which the
-    // multi-GPU producer-push protocol does not deliver)
-    const bool onepass = twice && c->nranks == 1 && chain_ok(&P, 2) &&
-                         (c->opt_cg_onepass > 0 || (c->opt_cg_onepass < 0 && n >= kCgOnePassMin));
+    // plain CG in one chain pass per iteration (48n B) or in pairs of passes (36n B): single GPU (the chain needs a
+    // two-line halo, which the multi-GPU producer-push protocol does not deliver)
+    const int cg_pass = !(twice && c->nranks == 1 && chain_ok(&P, 2)) ? 0
+                        : c->opt_cg_onepass >= 0 ? c->opt_cg_onepass
+                        : (n >= kCgPairMin ? 2 : (n >= kCgOnePassMin ? 1 : 0));
+    const bool onepass = cg_pass == 1, pair = cg_pass == 2;
     const int nvec = 4 + (dev ? 0 : 1) + (prec ? 3 : 0) + ((fuse_pc || twice) ? 1 : 0) + (twice ? 1 : 0);
     KL_TRY(ws_reserve(c, nvec * ws_need(n)));
     ws_reset(c);
@@ -308,7 +345,8 @@ static int cg_solve(Ctx *c, const kl_operator_t *A, const double *b, double *x, 
     double *r_alt = (fuse_pc || twice) ? ws_take<double>(c, n) : nullptr;
     double *x_cur = dx, *x_alt = twice ? ws_take<double>(c, n) : nullptr;
     // one-pass: x is ping-ponged from the first iteration on; start it where an odd / even maxit ends in dx
-    if (onepass && (maxit & 1)) std::swap(x_cur, x_alt);
+    // pairs: x moves once per pair; start it where maxit / 2 pairs end in dx (an odd maxit ends in a flush to dx)
+    if ((onepass && (maxit & 1)) || (pair && ((maxit / 2) & 1))) std::swap(x_cur, x_alt);
     double *const x_start = x_cur, *const x_other = x_alt;
     const Cbpr2Coef cf = fuse_pc ? cbpr2_coef(P.params) : Cbpr2Coef{1.0, 0.0};
     if (prec) {
@@ -319,7 +357,9 @@ static int cg_solve(Ctx *c, const kl_operator_t *A, const double *b, double *x, 
     // x0 = 0 ; r0 = b ; p0 = r0 (cg.f90:102-108)
     KL_TRY(stage_in(c, r, b, n));
     KL_CUDA(c, cudaMemsetAsync(x_cur, 0, n * sizeof(double), c->stream));
-    KL_CUDA(c, cudaMemsetAsync(p0, 0, n * sizeof(double), c->stream));
+    // pairs: p_0 = r_0 gets a buffer of its own, as pass B of the first pair overwrites r_0's with r_2
+    if (pair) KL_CUDA(c, cudaMemcpyAsync(p0, r, n * sizeof(double), cudaMemcpyDeviceToDevice, c->stream));
+    else KL_CUDA(c, cudaMemsetAsync(p0, 0, n * sizeof(double), c->stream));
     KL_CUDA(c, cudaMemsetAsync(c->d_I, 0, sizeof(int) * I_COUNT, c->stream));
     {
         double S0[32] = {0};
@@ -341,7 +381,7 @@ static int cg_solve(Ctx *c, const kl_operator_t *A, const double *b, double *x, 
     // one-pass: rr, p.Ap, r.Ap and Ap.Ap for p_0 = r_0, then alpha_0 and the predicted beta_0
     if (prec) {
         KL_TRY(pc_apply(&P, r, z, aux, aux2, 2, false, PostStoreRed{c->d_S, S_RR, 0}));
-    } else if (onepass) {
+    } else if (onepass || pair) {
         Halo H{};
         const double *vecs[1] = {r};
         FCgOnePassInit d;
@@ -365,6 +405,37 @@ static int cg_solve(Ctx *c, const kl_operator_t *A, const double *b, double *x, 
     auto enqueue_iterations = [&](const int done0, const int batch) -> int {
         const int done = done0;
         for (int k = 0; k < batch; ++k) {
+            if (pair && ((done + k) & 1) == 0) {
+                // pass A: p_0 is in p0 from the prologue on, p alternates between p1 (written by the first pair) and p0
+                ProfScope ps(c, 0, "cg_pair_a (chain: r-=alpha*A p; p=r+beta*p; A p; 4 dots)", 24.0 * n);
+                Halo H{};
+                const double *vecs[2] = {r, pold};
+                ChCgPass<kCgPairA> f;
+                set_io(f, &P, vecs, H);
+                set_gate(f, c, true);
+                f.r_new = r_alt; f.p_new = nullptr; f.x_new = nullptr; f.S = c->d_S;
+                KL_TRY(launch_chain(c, &P.op, f, P.nx, P.nyl, PostCgOnePass{c->d_S, c->d_I, c->d_hist, c->hist_cap}));
+                std::swap(r, r_alt);
+                z = r;
+                continue;
+            }
+            if (pair) {
+                ProfScope ps(c, 1, "cg_pair_b (chain: p=r+beta0*p0; r-=alpha*A p; p=r+beta*p; x+=alpha0*p0+alpha*p; A p; 4 dots)",
+                             48.0 * n);
+                Halo H{};
+                const double *vecs[2] = {r, pold};
+                ChCgPass<kCgPairB> f;
+                set_io(f, &P, vecs, H);
+                set_gate(f, c, true);
+                f.side[0] = x_cur;
+                f.r_new = r_alt; f.p_new = pnew; f.x_new = x_alt; f.S = c->d_S;
+                KL_TRY(launch_chain(c, &P.op, f, P.nx, P.nyl, PostCgOnePass{c->d_S, c->d_I, c->d_hist, c->hist_cap}));
+                std::swap(r, r_alt);
+                std::swap(x_cur, x_alt);
+                std::swap(pold, pnew);
+                z = r;
+                continue;
+            }
             if (onepass) {
                 // pass 0 reads r_0 as p_0 as well; from then on p alternates between p1 (odd passes write it)
                 // and p0
@@ -510,7 +581,7 @@ static int cg_solve(Ctx *c, const kl_operator_t *A, const double *b, double *x, 
             gk.add('C').add(nx).add(ny).add(batch).add(P.op.kind).add(P.op.eps_x).add(P.op.eps_y).add(P.pc.kind)
                 .add(P.pc.degree).add(P.params).add(c->opt_tma).add(c->opt_chain).add(c->opt_stencil_rows)
                 .add(c->opt_stencil_tail).add(c->opt_stencil_stagger).add(c->opt_pdl).add(c->ws).add(dx).add(r).add(pold)
-                .add(x_cur).add(onepass).add(onepass && done == 0);     // (one-pass: iteration 1 reads r as p)
+                .add(x_cur).add(cg_pass).add(onepass && done == 0);     // (one-pass: iteration 1 reads r as p)
             ge = graph_find(c, gk.s);
             if (!ge && polls >= 1) {     // the first batch of a handle's first solve runs eagerly
                 const long long l0 = c->stats.kernel_launches;
@@ -540,7 +611,23 @@ static int cg_solve(Ctx *c, const kl_operator_t *A, const double *b, double *x, 
             break;
         }
     }
-    if (onepass) {
+    if (pair) {
+        // after `its` passes (the passes after the convergence step were gated off) x_{2m}, m = its / 2, is in
+        // x_start (m even) or the other buffer (m odd), and p_{2m} in p0 (m even) or p1 (m odd).  An odd `its` ended
+        // on a pass A: x_{its} = x_{2m} + alpha_{2m} p_{2m}, the one-pass path's fma, with alpha_{2m} in
+        // S_ALPHA_PREV.
+        if (status == KL_NOT_CONVERGED) KL_TRY(read_back(c));     // (maxit = 0: no poll ran)
+        const int its_done = c->h_pinned_i[I_ITER], m = its_done / 2;
+        const double *xres = (m & 1) ? x_other : x_start;
+        if (its_done & 1) {
+            PAxpy u;
+            set_gate(u, c, false);
+            u.a = xres; u.b = (m & 1) ? p1 : p0; u.y = dx; u.S = c->d_S; u.s_idx = S_ALPHA_PREV; u.sign = 1.0;
+            KL_TRY(launch_pointwise(c, u, n, NoPost{}));
+        } else if (xres != dx) {
+            KL_CUDA(c, cudaMemcpyAsync(dx, xres, n * sizeof(double), cudaMemcpyDeviceToDevice, c->stream));
+        }
+    } else if (onepass) {
         // no deferred update: after `its` passes x is in x_start (even) or the other buffer (odd); the passes
         // after the convergence step were gated off
         if (status == KL_NOT_CONVERGED) KL_TRY(read_back(c));     // (maxit = 0: no poll ran)
@@ -578,7 +665,8 @@ static int cg_solve(Ctx *c, const kl_operator_t *A, const double *b, double *x, 
     c->stats.cycles = polls;
     c->stats.solve_ms = ms;
     c->stats.total_ms = ms_tot;
-    c->stats.algorithmic_bytes = (double)its * (fuse_pc ? 80.0 : (prec ? 96.0 : (onepass ? 48.0 : (twice ? 64.0 : (defer_x ? 72.0 : 80.0))))) * (double)n;
+    c->stats.algorithmic_bytes = pair ? (24.0 * ((its + 1) / 2) + 48.0 * (its / 2) + 24.0 * (its & 1)) * (double)n
+                                      : (double)its * (fuse_pc ? 80.0 : (prec ? 96.0 : (onepass ? 48.0 : (twice ? 64.0 : (defer_x ? 72.0 : 80.0))))) * (double)n;
     *res_out = c->h_pinned[S_RES];
     if (status == KL_OK) *iter = c->h_pinned_i[I_CONV_AT];   // count on exit; unchanged if not converged
     return status;

@@ -499,7 +499,7 @@ int kl_create(kl_handle_t *h, int device) {
     if (const char *e = getenv("KL_STENCIL_TAIL")) c->opt_stencil_tail = atoi(e);
     if (const char *e = getenv("KL_STENCIL_STAGGER")) c->opt_stencil_stagger = atoi(e) != 0;
     if (const char *e = getenv("KL_REVERSE")) c->opt_reverse = atoi(e) != 0;
-    if (const char *e = getenv("KL_CG_ONEPASS")) c->opt_cg_onepass = atoi(e) < 0 ? -1 : (atoi(e) != 0);
+    if (const char *e = getenv("KL_CG_ONEPASS")) c->opt_cg_onepass = atoi(e) < 0 ? -1 : std::min(atoi(e), 2);
     if (const char *e = getenv("KL_COOP")) c->opt_coop = atoi(e) != 0;
     if (const char *e = getenv("KL_PERSISTENT")) c->opt_persistent = atoi(e) != 0;
     if (const char *e = getenv("KL_PERSIST_OCC")) c->opt_persist_occ = atoi(e);
@@ -646,7 +646,7 @@ int kl_set_option(kl_handle_t h, int key, int value) {
         case KL_OPT_PERSISTENT: h->opt_persistent = value != 0; break;
         case KL_OPT_PUSH_HALO: h->opt_push_halo = value != 0; break;
         case KL_OPT_CG_ONEPASS:
-            if (value < -1 || value > 1) return KL_ERR_INVALID;
+            if (value < -1 || value > 2) return KL_ERR_INVALID;
             h->opt_cg_onepass = value;
             break;
         default: return KL_ERR_INVALID;

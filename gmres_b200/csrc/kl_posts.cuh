@@ -73,10 +73,14 @@ struct PostCgEnd {
 // One-pass CG (ChCg, kl_cg.cu).  S_RED = rho = r.r, gamma = p.Ap, sigma = r.Ap, delta = Ap.Ap of the iterate the
 // pass produced.  alpha = rho / gamma is the reference's formula on true dot products (cg.f90:124-126).  beta needs
 // ||r - alpha Ap||^2, the next pass's r.r; it is predicted by expanding the square, rho - 2 alpha sigma +
-// alpha^2 delta, so that the next pass can form the direction in the same sweep.
+// alpha^2 delta, so that the next pass can form the direction in the same sweep.  The alpha and beta being replaced
+// are kept in S_ALPHA_PREV / S_BETA_PREV: the second pass of a pair (ChCgPass<kCgPairB>) rebuilds the direction
+// and the x update of the iteration before it.
 __device__ __forceinline__ void cg_onepass_scalars(double *S) {
     const double rho = S[S_RED], gam = S[S_RED + 1], sig = S[S_RED + 2], del = S[S_RED + 3];
     const double alpha = rho / gam;
+    S[S_ALPHA_PREV] = S[S_ALPHA];
+    S[S_BETA_PREV] = S[S_BETA];
     S[S_PAP] = gam;
     S[S_ALPHA] = alpha;
     S[S_BETA] = (rho - 2.0 * alpha * sig + alpha * alpha * del) / rho;

@@ -150,8 +150,10 @@ enum {
                                  tile -- the hardware's dynamic CTA scheduling balances better (measured)            */
     KL_OPT_CG_ONEPASS = 22,   /* plain CG on one GPU with a built-in 5-point operator: 1 = one temporally blocked pass per
                                  iteration (48n B, one reduction; beta predicted from three dot products of the same
-                                 pass), 0 = two stencil passes (64n B), -1 (default) = one pass from 2^20 unknowns
-                                 on (1.3-1.8x faster there on B200; smaller grids, which fit in L2, keep two passes)  */
+                                 pass), 2 = pairs of such passes that store p and x every second iteration only (36n B,
+                                 bit-identical to 1), 0 = two stencil passes (64n B), -1 (default) = one pass from 2^20
+                                 unknowns on (1.3-1.8x faster there on B200; smaller grids, which fit in L2, keep two
+                                 passes), pairs from 2^24 on                                                          */
     KL_OPT_PUSH_HALO = 16,    /* multi-GPU with peer memory: 1 (default) = the kernel that PRODUCES a vector pushes its
                                  boundary lines into the neighbours' halo slots (no halo kernel; the all-reduce that
                                  ends the kernel is the barrier); 0 = separate halo push before every operator apply */
