@@ -580,7 +580,8 @@ static int cg_solve(Ctx *c, const kl_operator_t *A, const double *b, double *x, 
             GraphKey gk;
             gk.add('C').add(nx).add(ny).add(batch).add(P.op.kind).add(P.op.eps_x).add(P.op.eps_y).add(P.pc.kind)
                 .add(P.pc.degree).add(P.params).add(c->opt_tma).add(c->opt_chain).add(c->opt_stencil_rows)
-                .add(c->opt_stencil_tail).add(c->opt_stencil_stagger).add(c->opt_pdl).add(c->ws).add(dx).add(r).add(pold)
+                .add(c->opt_stencil_tail).add(c->opt_stencil_stagger).add(c->opt_pdl).add(c->opt_reverse).add(c->opt_persistent)
+                .add(c->ws).add(dx).add(r).add(pold)
                 .add(x_cur).add(cg_pass).add(onepass && done == 0);     // (one-pass: iteration 1 reads r as p)
             ge = graph_find(c, gk.s);
             if (!ge && polls >= 1) {     // the first batch of a handle's first solve runs eagerly

@@ -122,3 +122,17 @@ def test_onepass_auto_threshold(kl, h):
         b = h.apply(kl.stvec, torch.ones(ns * ns, dtype=torch.float64, device="cuda"), ns, ns)
         g = h.cg_omp(kl.stvec, b, 0.0, 4, nx=ns, ny=ns)
         assert _bytes_per_point(g, ns, ns) == pytest.approx(want), ns
+
+
+@pytest.mark.parametrize("nx,ny", [(1024, 1024), (1000, 64), (128, 515)])
+@pytest.mark.parametrize("aniso", [False, True])
+def test_onepass_matches_two_kernel_path_random_rhs(kl, h, nx, ny, aniso):
+    """As above with a random b, which has support on the whole grid from the first iteration on."""
+    op = kl.aniso(1.0, 0.01) if aniso else kl.stvec
+    b = np.random.default_rng(nx * 3 + ny).standard_normal(nx * ny)
+    for its in (1, 2, 7, 40):
+        g = _with(h, 1, lambda: h.cg_omp(op, b, 0.0, its, nx=nx, ny=ny))
+        s = _with(h, 0, lambda: h.cg_omp(op, b, 0.0, its, nx=nx, ny=ny))
+        assert g.history.size == s.history.size == its
+        assert np.allclose(g.history, s.history, rtol=1e-12, atol=0), (its, np.abs(g.history / s.history - 1).max())
+        assert np.abs(g.x - s.x).max() < 1e-12 * np.abs(s.x).max(), (its, np.abs(g.x - s.x).max())

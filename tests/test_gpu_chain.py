@@ -178,3 +178,35 @@ def test_cooperative_cgs2_step_bit_identical_to_three_kernels(kl, h, ns, m):
     assert g.status in (0, 1) and (g.status, g.n_out, g.restart_out) == (u.status, u.n_out, u.restart_out)
     assert np.abs(g.history / u.history - 1).max() < 1e-11 and np.abs(g.x - u.x).max() < 1e-12
     assert g.stats["kernel_launches"] < u.stats["kernel_launches"]
+
+
+@pytest.mark.parametrize("nx,ny", [(1024, 1024), (1000, 64), (128, 515)])
+def test_cg_operator_twice_matches_stored_ap_random_rhs(kl, h, nx, ny):
+    """As test_cg_operator_twice_matches_stored_ap with a random b (support on the whole grid)."""
+    b = np.random.default_rng(nx + 2 * ny).standard_normal(nx * ny)
+    h.set_option(22, 0)          # KL_OPT_CG_ONEPASS off: the two-kernel iteration at every size
+    try:
+        for its in (1, 2, 7, 40):
+            g = h.cg_omp(kl.stvec, b, 0.0, its, nx=nx, ny=ny)
+            s = _no_chain(kl, h, lambda: h.cg_omp(kl.stvec, b, 0.0, its, nx=nx, ny=ny))
+            assert np.abs(g.x - s.x).max() < 1e-12 * np.abs(s.x).max(), (its, np.abs(g.x - s.x).max())
+            assert np.allclose(g.history, s.history, rtol=1e-12, atol=0)
+    finally:
+        h.set_option(22, -1)
+
+
+@pytest.mark.parametrize("nx,ny,m", [(1024, 1024, 30), (2048, 640, 20), (130, 76, 12)])
+def test_gmres_one_pass_step_bit_identical_to_two_kernels_random_rhs(kl, h, nx, ny, m):
+    """As test_gmres_one_pass_step_bit_identical_to_two_kernels with a random b (support on the whole grid)."""
+    P = (8.2, 0.2)
+    b = np.random.default_rng(nx + ny + m).standard_normal(nx * ny)
+    h.set_option(2, 3)
+    try:
+        for op in (kl.stvec, kl.aniso(1.0, 0.05)):
+            run = lambda: h.gmres_mgsr_omp(op, b, m, 0.0, kl.cbpr2, P, nx=nx, ny=ny)
+            g = run()
+            u = _no_chain(kl, h, run)
+            assert (g.n_out, g.restart_out) == (u.n_out, u.restart_out) and g.history.size == 3 * m
+            assert np.array_equal(g.history, u.history) and np.array_equal(g.x, u.x)
+    finally:
+        h.set_option(2, 1000)
