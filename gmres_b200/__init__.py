@@ -41,6 +41,7 @@ from .api import (  # noqa: F401
     KL_OPT_STENCIL_ROWS,
     KL_OPT_PROFILE,
     KL_OPT_CHECK_EVERY,
+    KL_OPT_X0,
 )
 
 __all__ = [

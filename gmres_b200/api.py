@@ -14,6 +14,9 @@ Every solver method keeps the reference procedure's name and argument order
 intent(out) arguments become fields of the returned result object.  Vectors may be
 numpy float64 arrays (host pointer mode; copied to and from the device inside the
 call) or CUDA torch.float64 tensors (device pointer mode; they stay in HBM).
+
+Every solver method also takes `x0=None`: an initial guess of b's kind and length
+(KL_OPT_X0).  The reference starts from x = 0, and so does a call without x0.
 """
 from __future__ import annotations
 
@@ -34,6 +37,7 @@ KL_POINTER_HOST, KL_POINTER_DEVICE = 0, 1
 (KL_OPT_ORTHO, KL_OPT_MAX_RESTARTS, KL_OPT_VERR, KL_OPT_CHECK_EVERY, KL_OPT_USE_GRAPH,
  KL_OPT_HH_MODE, KL_OPT_FUSE, KL_OPT_PROFILE) = range(1, 9)
 KL_OPT_TMA, KL_OPT_PEER, KL_OPT_REORTH_ETA, KL_OPT_CHAIN, KL_OPT_STENCIL_ROWS, KL_OPT_INLINE_ALLREDUCE = 9, 10, 11, 12, 13, 14
+KL_OPT_X0 = 23
 ORTHO_MGS2, ORTHO_CGS2, ORTHO_CGS2_SELECTIVE = 0, 1, 2
 HH_SEQUENTIAL, HH_BLOCKED = 0, 1
 KL_UNIQUE_ID_BYTES = 128
@@ -417,6 +421,38 @@ class Handle:
         return o, C.c_void_p(o.ctypes.data)
 
     @staticmethod
+    def _check_x0(x0, b):
+        """x0 must be b's kind (a CUDA float64 tensor on b's device, or a numpy array) and length; checked before any
+        call into the library."""
+        if x0 is None:
+            return
+        if _is_torch_cuda(b):
+            import torch
+            if not (_is_torch_cuda(x0) and x0.dtype == torch.float64 and x0.device == b.device):
+                raise KrylovError("x0 must be a CUDA float64 tensor on b's device when b is one")
+            nb, n0 = b.numel(), x0.numel()
+        else:
+            if not isinstance(x0, np.ndarray):
+                raise KrylovError("x0 must be a numpy array when b is not a CUDA tensor")
+            nb, n0 = np.asarray(b).size, x0.size
+        if n0 != nb:
+            raise KrylovError(f"x0 has {n0} values, b has {nb}")
+
+    def _x_out(self, ba, dev, x0):
+        """The solver's x buffer (see _out_like).  KL_OPT_X0 is set on every call, so that a value left on the handle
+        can never make a call read an uninitialised buffer; with x0 given, x0 is copied into the buffer (the caller's
+        x0 is not written) and the library starts from it."""
+        self._chk(self._L.kl_set_option(self._h, KL_OPT_X0, 0 if x0 is None else 1))
+        x, xp = self._out_like(ba, dev)
+        if x0 is not None:
+            if dev:
+                x.view(-1).copy_(x0.reshape(-1))
+                self._order_in()     # the library's stream waits for the copy on torch's current stream
+            else:
+                x.reshape(-1)[:] = x0.reshape(-1)
+        return x, xp
+
+    @staticmethod
     def _grid(b, nx, ny):
         n = b.numel() if hasattr(b, "numel") else b.size
         if nx is None:
@@ -449,10 +485,11 @@ class Handle:
         return z
 
     # -- GMRES
-    def _gmres(self, fn, A, b, m, tol, M, params, nx, ny, with_pc=True):
+    def _gmres(self, fn, A, b, m, tol, M, params, nx, ny, with_pc=True, x0=None):
+        self._check_x0(x0, b)
         ba, bp, dev = self._in(b)
         nx, ny = self._grid(ba, nx, ny)
-        x, xp = self._out_like(ba, dev)
+        x, xp = self._x_out(ba, dev, x0)
         fe = np.zeros(m)
         ve = np.zeros(m + 1)
         n_out, rs = C.c_int(0), C.c_int(0)
@@ -468,17 +505,17 @@ class Handle:
             self._order_out()
         return GmresResult(x, fe, ve, n_out.value, rs.value, rc, self.history(), self.stats())
 
-    def gmres_mgsr_omp(self, Ax_vec, b, m, tol, M_inv=None, params=None, nx=None, ny=None):
-        return self._gmres(self._L.kl_gmres_mgsr_omp, Ax_vec, b, m, tol, M_inv, params, nx, ny)
+    def gmres_mgsr_omp(self, Ax_vec, b, m, tol, M_inv=None, params=None, nx=None, ny=None, x0=None):
+        return self._gmres(self._L.kl_gmres_mgsr_omp, Ax_vec, b, m, tol, M_inv, params, nx, ny, x0=x0)
 
-    def gmres_mgsr_mf(self, Ax_vec, b, m, tol, M_inv=None, params=None, nx=None, ny=None):
-        return self._gmres(self._L.kl_gmres_mgsr_mf, Ax_vec, b, m, tol, M_inv, params, nx, ny)
+    def gmres_mgsr_mf(self, Ax_vec, b, m, tol, M_inv=None, params=None, nx=None, ny=None, x0=None):
+        return self._gmres(self._L.kl_gmres_mgsr_mf, Ax_vec, b, m, tol, M_inv, params, nx, ny, x0=x0)
 
-    def gmres_hh_omp(self, Ax_vec, b, m, tol, nx=None, ny=None):
-        return self._gmres(self._L.kl_gmres_hh_omp, Ax_vec, b, m, tol, None, None, nx, ny, with_pc=False)
+    def gmres_hh_omp(self, Ax_vec, b, m, tol, nx=None, ny=None, x0=None):
+        return self._gmres(self._L.kl_gmres_hh_omp, Ax_vec, b, m, tol, None, None, nx, ny, with_pc=False, x0=x0)
 
-    def gmres_hh_prec_omp(self, Ax_vec, b, m, tol, m_inv=None, params=None, nx=None, ny=None):
-        return self._gmres(self._L.kl_gmres_hh_prec_omp, Ax_vec, b, m, tol, m_inv, params, nx, ny)
+    def gmres_hh_prec_omp(self, Ax_vec, b, m, tol, m_inv=None, params=None, nx=None, ny=None, x0=None):
+        return self._gmres(self._L.kl_gmres_hh_prec_omp, Ax_vec, b, m, tol, m_inv, params, nx, ny, x0=x0)
 
     # -- dense-operator variants (src/gmres_mgsr.f90:11, src/gmres_hh.f90:10, src/problems/hilbert.f90:6)
     def _dense_in(self, A, n):
@@ -509,11 +546,12 @@ class Handle:
             self._order_out()
         return y
 
-    def _gmres_dense(self, fn, A, b, m, tol):
+    def _gmres_dense(self, fn, A, b, m, tol, x0=None):
+        self._check_x0(x0, b)
         ba, bp, dev = self._in(b)
         n = ba.numel() if dev else ba.size
         Aa, Ap = self._dense_in(A, n)
-        x, xp = self._out_like(ba, dev)
+        x, xp = self._x_out(ba, dev, x0)
         fe = np.zeros(m)
         ve = np.zeros(m + 1)
         n_out, rs = C.c_int(0), C.c_int(0)
@@ -524,17 +562,18 @@ class Handle:
             self._order_out()
         return GmresResult(x, fe, ve, n_out.value, rs.value, rc, self.history(), self.stats())
 
-    def gmres_mgsr_dense(self, A, b, m, tol):
-        return self._gmres_dense(self._L.kl_gmres_mgsr_dense, A, b, m, tol)
+    def gmres_mgsr_dense(self, A, b, m, tol, x0=None):
+        return self._gmres_dense(self._L.kl_gmres_mgsr_dense, A, b, m, tol, x0)
 
-    def gmres_hh_dense(self, A, b, m, tol):
-        return self._gmres_dense(self._L.kl_gmres_hh_dense, A, b, m, tol)
+    def gmres_hh_dense(self, A, b, m, tol, x0=None):
+        return self._gmres_dense(self._L.kl_gmres_hh_dense, A, b, m, tol, x0)
 
     # -- CG / BiCGSTAB
-    def _cg(self, fn, A, b, tol, it, M, params, nx, ny, with_pc):
+    def _cg(self, fn, A, b, tol, it, M, params, nx, ny, with_pc, x0=None):
+        self._check_x0(x0, b)
         ba, bp, dev = self._in(b)
         nx, ny = self._grid(ba, nx, ny)
-        x, xp = self._out_like(ba, dev)
+        x, xp = self._x_out(ba, dev, x0)
         itc, res = C.c_int(int(it)), C.c_double(0.0)
         o, keep = A._c()
         args = [self._h, C.byref(o), bp, xp, nx, ny, float(tol), C.byref(itc), C.byref(res)]
@@ -547,26 +586,26 @@ class Handle:
             self._order_out()
         return CgResult(x, itc.value, res.value, rc, self.history(), self.stats())
 
-    def cg(self, Ax_op, b, tol, iter, nx=None, ny=None):
-        return self._cg(self._L.kl_cg, Ax_op, b, tol, iter, None, None, nx, ny, False)
+    def cg(self, Ax_op, b, tol, iter, nx=None, ny=None, x0=None):
+        return self._cg(self._L.kl_cg, Ax_op, b, tol, iter, None, None, nx, ny, False, x0)
 
-    def cg_omp(self, Ax_op, b, tol, iter, nx=None, ny=None):
-        return self._cg(self._L.kl_cg_omp, Ax_op, b, tol, iter, None, None, nx, ny, False)
+    def cg_omp(self, Ax_op, b, tol, iter, nx=None, ny=None, x0=None):
+        return self._cg(self._L.kl_cg_omp, Ax_op, b, tol, iter, None, None, nx, ny, False, x0)
 
-    def pcg(self, Ax_op, b, tol, iter, M_inv, params, nx=None, ny=None):
-        return self._cg(self._L.kl_pcg, Ax_op, b, tol, iter, M_inv, params, nx, ny, True)
+    def pcg(self, Ax_op, b, tol, iter, M_inv, params, nx=None, ny=None, x0=None):
+        return self._cg(self._L.kl_pcg, Ax_op, b, tol, iter, M_inv, params, nx, ny, True, x0)
 
-    def pcg_omp(self, Ax_op, b, tol, iter, M_inv, params, nx=None, ny=None):
-        return self._cg(self._L.kl_pcg_omp, Ax_op, b, tol, iter, M_inv, params, nx, ny, True)
+    def pcg_omp(self, Ax_op, b, tol, iter, M_inv, params, nx=None, ny=None, x0=None):
+        return self._cg(self._L.kl_pcg_omp, Ax_op, b, tol, iter, M_inv, params, nx, ny, True, x0)
 
-    def bicgstab(self, ax_op, b, tol, iter, nx=None, ny=None):
-        return self._cg(self._L.kl_bicgstab, ax_op, b, tol, iter, None, None, nx, ny, False)
+    def bicgstab(self, ax_op, b, tol, iter, nx=None, ny=None, x0=None):
+        return self._cg(self._L.kl_bicgstab, ax_op, b, tol, iter, None, None, nx, ny, False, x0)
 
-    def pbicgstab(self, ax_op, b, tol, iter, m_inv, params, nx=None, ny=None):
-        return self._cg(self._L.kl_pbicgstab, ax_op, b, tol, iter, m_inv, params, nx, ny, True)
+    def pbicgstab(self, ax_op, b, tol, iter, m_inv, params, nx=None, ny=None, x0=None):
+        return self._cg(self._L.kl_pbicgstab, ax_op, b, tol, iter, m_inv, params, nx, ny, True, x0)
 
-    def pbicgstab_omp(self, ax_op, b, tol, max_iter, m_inv, params, nx=None, ny=None):
-        return self._cg(self._L.kl_pbicgstab_omp, ax_op, b, tol, max_iter, m_inv, params, nx, ny, True)
+    def pbicgstab_omp(self, ax_op, b, tol, max_iter, m_inv, params, nx=None, ny=None, x0=None):
+        return self._cg(self._L.kl_pbicgstab_omp, ax_op, b, tol, max_iter, m_inv, params, nx, ny, True, x0)
 
     # -- Lanczos
     def lanczos(self, A: Operator, nx: int, ny: int, steps: int = 30):

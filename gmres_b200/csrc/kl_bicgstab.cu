@@ -259,6 +259,7 @@ static int bicgstab_solve(Ctx *c, const kl_operator_t *A, const double *b, doubl
                           double tol, int *iter, double *res_out, const kl_precond_t *M,
                           const double *params, int nparams) {
     if (!c || !A || !b || !x || !iter || !res_out) return KL_ERR_INVALID;
+    KL_TRY(x0_check(c, b, x));
     Prob P;
     KL_TRY(prob_init(&P, c, A, M, params, nparams, nx, ny));
     const bool prec = P.pc.kind != KL_PC_NONE;
@@ -287,10 +288,28 @@ static int bicgstab_solve(Ctx *c, const kl_operator_t *A, const double *b, doubl
     Cbpr2Coef cf{1.0, 0.0};
     if (cb) cf = cbpr2_coef(P.params);
     // x = 0 ; r = b ; r0 = r ; p = r0 (:114-118).  p_old = ap_old = 0 with beta = omega = 0
-    // makes the first direction update produce p = r exactly.
-    KL_TRY(stage_in(c, r, b, n));
+    // makes the first direction update produce p = r exactly.  KL_OPT_X0: x = x0 ; r = b - A x0.
+    if (c->opt_x0) {
+        KL_TRY(stage_in(c, dx, x, n));
+        const double *db = b;
+        if (!dev) {     // r0 is set from r below
+            KL_TRY(stage_in(c, r0, b, n));
+            db = r0;
+        }
+        KL_TRY(op_resid(&P, dx, db, r, false));
+        double r_norm = 0.0;
+        KL_TRY(x0_norm(c, r, n, &r_norm));
+        if (r_norm < tol || r_norm == 0.0) {     // x0 already passes the test (r = 0 would make alpha 0/0)
+            KL_TRY(x0_zero_step(c));
+            *iter = 0;
+            *res_out = r_norm;
+            return KL_OK;
+        }
+    } else {
+        KL_TRY(stage_in(c, r, b, n));
+        KL_CUDA(c, cudaMemsetAsync(dx, 0, n * sizeof(double), c->stream));
+    }
     KL_CUDA(c, cudaMemcpyAsync(r0, r, n * sizeof(double), cudaMemcpyDeviceToDevice, c->stream));
-    KL_CUDA(c, cudaMemsetAsync(dx, 0, n * sizeof(double), c->stream));
     KL_CUDA(c, cudaMemsetAsync(p0, 0, n * sizeof(double), c->stream));
     KL_CUDA(c, cudaMemsetAsync(ap0, 0, n * sizeof(double), c->stream));
     KL_CUDA(c, cudaMemsetAsync(c->d_I, 0, sizeof(int) * I_COUNT, c->stream));

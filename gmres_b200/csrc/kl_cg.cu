@@ -314,6 +314,7 @@ static int cg_solve(Ctx *c, const kl_operator_t *A, const double *b, double *x, 
                     double tol, int *iter, double *res_out, const kl_precond_t *M, const double *params,
                     int nparams) {
     if (!c || !A || !b || !x || !iter || !res_out) return KL_ERR_INVALID;
+    KL_TRY(x0_check(c, b, x));
     Prob P;
     KL_TRY(prob_init(&P, c, A, M, params, nparams, nx, ny));
     const bool prec = P.pc.kind != KL_PC_NONE;
@@ -354,9 +355,29 @@ static int cg_solve(Ctx *c, const kl_operator_t *A, const double *b, double *x, 
         aux = ws_take<double>(c, n);
         aux2 = ws_take<double>(c, n);
     }
-    // x0 = 0 ; r0 = b ; p0 = r0 (cg.f90:102-108)
-    KL_TRY(stage_in(c, r, b, n));
-    KL_CUDA(c, cudaMemsetAsync(x_cur, 0, n * sizeof(double), c->stream));
+    // x0 = 0 ; r0 = b ; p0 = r0 (cg.f90:102-108).  KL_OPT_X0: r0 = b - A x0 with x0 in the buffer the iterations
+    // start from (the two-kernel paths' first x update adds alpha = 0 times p = 0 to it, which leaves it as it is)
+    if (c->opt_x0) {
+        KL_TRY(stage_in(c, dx, x, n));
+        const double *db = b;
+        if (!dev) {     // ax is not read before the first iteration writes it
+            KL_TRY(stage_in(c, ax, b, n));
+            db = ax;
+        }
+        KL_TRY(op_resid(&P, dx, db, r, false));
+        if (x_cur != dx) KL_CUDA(c, cudaMemcpyAsync(x_cur, dx, n * sizeof(double), cudaMemcpyDeviceToDevice, c->stream));
+        double r0_norm = 0.0;
+        KL_TRY(x0_norm(c, r, n, &r0_norm));
+        if (r0_norm < tol || r0_norm == 0.0) {     // x0 already passes the test (r0 = 0 would make alpha 0/0)
+            KL_TRY(x0_zero_step(c));
+            *iter = 0;
+            *res_out = r0_norm;
+            return KL_OK;
+        }
+    } else {
+        KL_TRY(stage_in(c, r, b, n));
+        KL_CUDA(c, cudaMemsetAsync(x_cur, 0, n * sizeof(double), c->stream));
+    }
     // pairs: p_0 = r_0 gets a buffer of its own, as pass B of the first pair overwrites r_0's with r_2
     if (pair) KL_CUDA(c, cudaMemcpyAsync(p0, r, n * sizeof(double), cudaMemcpyDeviceToDevice, c->stream));
     else KL_CUDA(c, cudaMemsetAsync(p0, 0, n * sizeof(double), c->stream));

@@ -649,6 +649,10 @@ int kl_set_option(kl_handle_t h, int key, int value) {
             if (value < -1 || value > 2) return KL_ERR_INVALID;
             h->opt_cg_onepass = value;
             break;
+        case KL_OPT_X0:
+            if (value != 0 && value != 1) return KL_ERR_INVALID;
+            h->opt_x0 = value;
+            break;
         default: return KL_ERR_INVALID;
     }
     return KL_OK;
@@ -679,6 +683,7 @@ int kl_get_option(kl_handle_t h, int key, int *value) {
         case KL_OPT_PERSISTENT: *value = h->opt_persistent; break;
         case KL_OPT_PUSH_HALO: *value = h->opt_push_halo; break;
         case KL_OPT_CG_ONEPASS: *value = h->opt_cg_onepass; break;
+        case KL_OPT_X0: *value = h->opt_x0; break;
         default: return KL_ERR_INVALID;
     }
     return KL_OK;

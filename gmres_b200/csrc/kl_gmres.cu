@@ -577,6 +577,7 @@ int gmres_mgsr_solve(Ctx *c, const kl_operator_t *A, const double *b, double *x,
                             int mf) {
     if (!c || !A || !b || !x || !final_err || !v_err || !n_out_p || !restart_out_p) return KL_ERR_INVALID;
     if (m < 1 || m + 1 > kMaxCols) return c->fail(KL_ERR_INVALID, "restart length m out of range");
+    KL_TRY(x0_check(c, b, x));
     Prob P;
     KL_TRY(prob_init(&P, c, A, M, params, nparams, nx, ny));
     const bool prec = P.pc.kind != KL_PC_NONE;
@@ -615,7 +616,8 @@ int gmres_mgsr_solve(Ctx *c, const kl_operator_t *A, const double *b, double *x,
     G.m = m; G.ldh = ldh; G.mf = mf;
 
     if (!dev) KL_TRY(stage_in(c, db, b, n));
-    KL_CUDA(c, cudaMemsetAsync(dx, 0, n * sizeof(double), c->stream));          // x = 0 (:304)
+    if (c->opt_x0) KL_TRY(stage_in(c, dx, x, n));                               // x = x0 (KL_OPT_X0)
+    else KL_CUDA(c, cudaMemsetAsync(dx, 0, n * sizeof(double), c->stream));     // x = 0 (:304)
     KL_CUDA(c, cudaMemsetAsync(G.fe, 0, (m + 2) * sizeof(double), c->stream));  // final_err = 0
     KL_CUDA(c, cudaMemsetAsync(c->d_I, 0, sizeof(int) * I_COUNT, c->stream));
     {
@@ -630,6 +632,22 @@ int gmres_mgsr_solve(Ctx *c, const kl_operator_t *A, const double *b, double *x,
         set_gate(d, c, false);
         d.a = db; d.b = db; d.c = nullptr; d.d = nullptr;
         KL_TRY(launch_pointwise(c, d, n, PostStoreRed{c->d_S, S_BETA0, 1}));
+    }
+    if (c->opt_x0) {
+        // the first cycle's beta = ||M^-1 (b - A x0)|| against the ||b|| that final_err is measured with: x0 that
+        // already passes the test returns before a cycle (beta = 0 would make V_1 = w/0)
+        KL_TRY(op_resid(&P, dx, db, z, false));
+        if (prec) KL_TRY(pc_apply(&P, z, w, aux, aux2, 0, false, NoPost{}));
+        double beta = 0.0;
+        KL_TRY(x0_norm(c, prec ? w : z, n, &beta));
+        if (beta == 0.0 || beta / c->h_pinned[S_BETA0] < tol) {
+            KL_TRY(x0_zero_step(c));
+            for (int i = 0; i < m; ++i) final_err[i] = 0.0;
+            for (int i = 0; i <= m; ++i) v_err[i] = 0.0;
+            *n_out_p = 0;
+            *restart_out_p = 1;
+            return KL_OK;
+        }
     }
     KL_CUDA(c, cudaEventRecord(c->ev0, c->stream));
 

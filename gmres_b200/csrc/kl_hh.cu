@@ -448,6 +448,7 @@ int gmres_hh_solve(Ctx *c, const kl_operator_t *A, const double *b, double *x, i
     if (!c || !A || !b || !x || !final_err || !v_err || !n_out_p || !stages_out_p) return KL_ERR_INVALID;
     if (m < 1 || m + 1 > kMaxCols) return c->fail(KL_ERR_INVALID, "restart length m out of range");
     if (c->nranks > 1) return c->fail(KL_ERR_UNSUPPORTED, "Householder GMRES is single-GPU in this release");
+    KL_TRY(x0_check(c, b, x));
     Prob P;
     KL_TRY(prob_init(&P, c, A, prec_variant == 1 ? M : nullptr, params, nparams, nx, ny));
     const bool prec = P.pc.kind != KL_PC_NONE;
@@ -497,7 +498,8 @@ int gmres_hh_solve(Ctx *c, const kl_operator_t *A, const double *b, double *x, i
     }
 
     if (!dev) KL_TRY(stage_in(c, db, b, n));
-    KL_CUDA(c, cudaMemsetAsync(dx, 0, n * sizeof(double), c->stream));
+    if (c->opt_x0) KL_TRY(stage_in(c, dx, x, n));                               // x = x0 (KL_OPT_X0)
+    else KL_CUDA(c, cudaMemsetAsync(dx, 0, n * sizeof(double), c->stream));
     KL_CUDA(c, cudaMemsetAsync(G.fe, 0, (m + 2) * sizeof(double), c->stream));
     KL_CUDA(c, cudaMemsetAsync(c->d_I, 0, sizeof(int) * I_COUNT, c->stream));
     {
@@ -512,6 +514,21 @@ int gmres_hh_solve(Ctx *c, const kl_operator_t *A, const double *b, double *x, i
         set_gate(d, c, false);
         d.a = db; d.b = db; d.c = nullptr; d.d = nullptr;
         KL_TRY(launch_pointwise(c, d, n, PostStoreRed{c->d_S, S_BETA0, 1}));
+    }
+    if (c->opt_x0) {
+        // as in gmres_mgsr_solve: x0 whose ||M^-1 (b - A x0)|| / ||b|| already passes the test returns before a cycle
+        KL_TRY(op_resid(&P, dx, db, z, false));
+        if (prec) KL_TRY(pc_apply(&P, z, w, aux, aux2, 0, false, NoPost{}));
+        double beta = 0.0;
+        KL_TRY(x0_norm(c, prec ? w : z, n, &beta));
+        if (beta == 0.0 || beta / c->h_pinned[S_BETA0] < tol) {
+            KL_TRY(x0_zero_step(c));
+            for (int i = 0; i < m; ++i) final_err[i] = 0.0;
+            for (int i = 0; i <= m; ++i) v_err[i] = 0.0;
+            *n_out_p = 0;
+            *stages_out_p = 1;
+            return KL_OK;
+        }
     }
     KL_CUDA(c, cudaEventRecord(c->ev0, c->stream));
     const int max_stages = c->opt_max_restarts;

@@ -158,6 +158,8 @@ struct kl_context_s {
     int opt_stencil_tail = -1;  // lines per CTA in the tapered tail (-1 auto, 0 off), KL_OPT_STENCIL_TAIL
     int opt_pdl = 1;            // programmatic dependent launch between the fused CG kernels (KL_OPT_PDL)
     int opt_cg_onepass = -1;    // plain CG in chain passes (KL_OPT_CG_ONEPASS): -1 auto, 0 off, 1 one pass per iteration, 2 pairs
+    int opt_x0 = 0;             // x is the initial guess on entry (KL_OPT_X0); no environment variable: it turns an output
+                                // into an input
     // comm
     int rank = 0, nranks = 1;
     void *nccl_comm = nullptr;

@@ -385,6 +385,38 @@ int read_back(Ctx *c) {
     return KL_OK;
 }
 
+int x0_check(Ctx *c, const double *b, const double *x) {
+    if (!c->opt_x0) return KL_OK;
+    // multi-GPU: the plain-CG producer-push prologue pushes r0's boundary lines, a path that is not covered yet
+    if (c->nranks > 1) return c->fail(KL_ERR_UNSUPPORTED, "KL_OPT_X0 is single-GPU in this release");
+    if (c->pointer_mode == KL_POINTER_DEVICE && x == b)
+        return c->fail(KL_ERR_INVALID, "KL_OPT_X0: x is read as the initial guess and written as the solution, it must not be b");
+    return KL_OK;
+}
+
+int x0_norm(Ctx *c, const double *v, size_t n, double *norm) {
+    PDot2 d;
+    set_gate(d, c, false);
+    d.a = v; d.b = v; d.c = nullptr; d.d = nullptr;
+    KL_TRY(launch_pointwise(c, d, n, PostStoreRed{c->d_S, S_RES, 1}));
+    KL_TRY(read_back(c));
+    *norm = c->h_pinned[S_RES];
+    KL_CUDA(c, cudaMemsetAsync(c->d_S + S_RES, 0, sizeof(double), c->stream));
+    return KL_OK;
+}
+
+int x0_zero_step(Ctx *c) {
+    c->history.clear();
+    c->history_len = 0;
+    KL_CUDA(c, cudaEventRecord(c->ev3, c->stream));
+    KL_CUDA(c, cudaStreamSynchronize(c->stream));
+    KL_CUDA(c, cudaGetLastError());
+    float ms = 0;
+    cudaEventElapsedTime(&ms, c->ev2, c->ev3);
+    c->stats.total_ms = ms;
+    return KL_OK;
+}
+
 int fetch_history(Ctx *c) {
     KL_TRY(read_back(c));
     int len = c->h_pinned_i[I_HIST];

@@ -93,5 +93,13 @@ int read_back(Ctx *c);
 // copy history from the device and fill ctx->history
 int fetch_history(Ctx *c);
 
+// KL_OPT_X0 (x is the initial guess).  x0_check: the option's preconditions (one GPU; device mode: x is not b).
+int x0_check(Ctx *c, const double *b, const double *x);
+// ||v||, read back to the host, for the zero-step test before the first iteration.  S_RES, where the reduction
+// lands, is zeroed again, so the iteration starts from the scalar block of a cold solve.
+int x0_norm(Ctx *c, const double *v, size_t n, double *norm);
+// bookkeeping of a zero-step return (x0 already meets the stopping test): empty history, call time
+int x0_zero_step(Ctx *c);
+
 
 }  // namespace kl

@@ -38,7 +38,7 @@
 extern "C" {
 #endif
 
-#define KL_VERSION 100
+#define KL_VERSION 101
 
 typedef struct kl_context_s *kl_handle_t;
 
@@ -154,6 +154,18 @@ enum {
                                  bit-identical to 1), 0 = two stencil passes (64n B), -1 (default) = one pass from 2^20
                                  unknowns on (1.3-1.8x faster there on B200; smaller grids, which fit in L2, keep two
                                  passes), pairs from 2^24 on                                                          */
+    KL_OPT_X0 = 23,           /* solver entries (not kl_lanczos): 0 (default) = x is output only and the solve starts from
+                                 x = 0, as the reference does; 1 = x is read on entry as the initial guess x0 and
+                                 overwritten with the solution (host mode: the nx*ny doubles at x are uploaded and
+                                 counted in h2d_bytes; device mode: x is used in place and must not be b).  CG, PCG and
+                                 BiCGSTAB start from r0 = b - A x0 with the same absolute test ||r|| < tol; GMRES and
+                                 Householder GMRES start their first cycle from x0 and keep final_err = |g_j+1|/||b||;
+                                 iter, n_out, restart_out / stages_out and the history count this call only.  If the
+                                 initial residual norm of the stopping test (||r0||, or ||M^-1 (b - A x0)|| / ||b||
+                                 for GMRES) is below tol or zero, the call returns KL_OK at once with x = x0 untouched,
+                                 iter = 0 and res = ||r0|| (GMRES: n_out = 0, restart_out = 1, final_err = v_err = 0)
+                                 and an empty history.  One GPU only (KL_ERR_UNSUPPORTED on a multi-GPU handle); no
+                                 environment variable.                                                           */
     KL_OPT_PUSH_HALO = 16,    /* multi-GPU with peer memory: 1 (default) = the kernel that PRODUCES a vector pushes its
                                  boundary lines into the neighbours' halo slots (no halo kernel; the all-reduce that
                                  ends the kernel is the barrier); 0 = separate halo push before every operator apply */
@@ -202,7 +214,8 @@ int kl_apply_precond(kl_handle_t h, const kl_precond_t *M_inv, const kl_operator
                      int ny);
 
 /* ---- solvers -------------------------------------------------------------
- * Output sizes: x[nx*ny_local], final_err[m], v_err[m+1].                    */
+ * Output sizes: x[nx*ny_local], final_err[m], v_err[m+1].
+ * x is output only unless KL_OPT_X0 = 1, which makes it the initial guess as well.   */
 
 /* gmres_mgsr_omp(Ax_vec,b,x,m,tol,final_err,v_err,n_out,restart_out,M_inv,params)
  * src/gmres_mgsr.f90:277 */
