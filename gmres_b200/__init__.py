@@ -27,6 +27,7 @@ from .api import (  # noqa: F401
     aniso_var,
     cbpr2,
     cheb,
+    jacobi_cheb,
     no_precond,
     ORTHO_MGS2,
     ORTHO_CGS2,
@@ -42,9 +43,10 @@ from .api import (  # noqa: F401
     KL_OPT_PROFILE,
     KL_OPT_CHECK_EVERY,
     KL_OPT_X0,
+    KL_PC_JACOBI_CHEB,
 )
 
 __all__ = [
     "Handle", "KrylovError", "Operator", "Precond", "GmresResult", "CgResult", "stvec",
-    "stv_poisson", "aniso", "cbpr2", "cheb", "no_precond", "library_path", "load_library",
+    "stv_poisson", "aniso", "cbpr2", "cheb", "jacobi_cheb", "no_precond", "library_path", "load_library",
 ]

@@ -32,7 +32,7 @@ _LIBNAME = "libkrylov_b200.so"
 
 KL_OK, KL_NOT_CONVERGED, KL_BREAKDOWN = 0, 1, 2
 KL_OP_POISSON5, KL_OP_POISSON5_BRANCHY, KL_OP_ANISO5, KL_OP_ANISO5_VAR, KL_OP_USER = 0, 1, 2, 4, 100
-KL_PC_NONE, KL_PC_CBPR2, KL_PC_CHEB, KL_PC_USER = 0, 1, 2, 100
+KL_PC_NONE, KL_PC_CBPR2, KL_PC_CHEB, KL_PC_JACOBI_CHEB, KL_PC_USER = 0, 1, 2, 3, 100
 KL_POINTER_HOST, KL_POINTER_DEVICE = 0, 1
 (KL_OPT_ORTHO, KL_OPT_MAX_RESTARTS, KL_OPT_VERR, KL_OPT_CHECK_EVERY, KL_OPT_USE_GRAPH,
  KL_OPT_HH_MODE, KL_OPT_FUSE, KL_OPT_PROFILE) = range(1, 9)
@@ -241,6 +241,13 @@ def aniso_var(kx, ky) -> Operator:
 
 def cheb(degree: int) -> Precond:
     return Precond(KL_PC_CHEB, int(degree))
+
+
+def jacobi_cheb(degree: int) -> Precond:
+    """Chebyshev of the given degree on the Jacobi-scaled operator D^-1 A (KL_PC_JACOBI_CHEB), for aniso_var operators.
+    Degree 0 is point Jacobi (params ignored); degree k >= 1 takes params = (a, b), an interval of the spectrum of
+    D^-1 A, which lies in (0, 2]."""
+    return Precond(KL_PC_JACOBI_CHEB, int(degree))
 
 
 @dataclass

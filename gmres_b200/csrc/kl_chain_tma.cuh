@@ -51,6 +51,9 @@
 //        sd = side inputs (arrays side[0..NSIDE), read point-wise at the last level's output points only,
 //        valid for lv == L && out; the kernel prefetches them two lines ahead into registers)
 // level0 must map all-zero inputs to u = 0 (outside the domain TMA delivers zeros).
+// VAROP functors (ChJacCheb) take the diagonal of A at their points as well: level0(out, idx, raw, dg, u, cc, acc)
+// and level(lv, out, idx, up, au, dg, cin, raw, sd, u, cout, acc); their level-0 values outside the domain never
+// reach the domain (the checked march applies the boundary rule to neighbours).
 #pragma once
 #include <type_traits>
 
@@ -62,9 +65,10 @@ constexpr int kChainWarps = 4;
 constexpr int kChainThreads = kChainWarps * 32;
 constexpr int kChainMaxL = 6;
 
-template <int L>
+// VAR: the variable-coefficient operator needs one more halo column (its level 0 reads kx at columns -1 and +1)
+template <int L, bool VAR = false>
 struct ChainDims {
-    static constexpr int H = (L + 1) & ~1;              // halo columns per window side
+    static constexpr int H = (L + (VAR ? 1 : 0) + 1) & ~1;   // halo columns per window side
     static constexpr int WW = 64 - 2 * H;               // output columns per warp
     static constexpr int STRIP = kChainWarps * WW;      // output columns per CTA
     static constexpr int BW = STRIP + 2 * H;            // columns a CTA needs
@@ -78,12 +82,12 @@ struct ChainRing {
     static constexpr int SR = C::SR;
     static constexpr int NST = C::NST;
     static constexpr int NR = SR * NST;
-    static constexpr int RET = (C::LAG * C::L + SR - 1) / SR;
+    static constexpr int RET = (C::LAG * C::L + (C::VAROP ? 2 : 0) + SR - 1) / SR;
     static constexpr int P = 6;                         // unroll period of the march = lcm(3 field slots, 2 carried slots)
     static_assert(P % SR == 0, "an unroll period must hold whole stages");
     static_assert(NR % P == 0, "ring must hold whole periods");
     static_assert(NST - RET >= 2, "ring too shallow");
-    static constexpr size_t bytes = (size_t)C::NIN * NR * ChainDims<C::L>::BWP * sizeof(double) + 2 * NST * 8 + 64;
+    static constexpr size_t bytes = (size_t)C::NIN * NR * ChainDims<C::L, C::VAROP>::BWP * sizeof(double) + 2 * NST * 8 + 64;
 };
 
 struct ChainGeo {
@@ -98,6 +102,9 @@ struct ChainBase {
     static constexpr int NC = NC_;
     static constexpr int NRED = NRED_;
     static constexpr int NSIDE = 0;     // point-wise side inputs of the last level, prefetched 2 lines ahead
+    // VAROP: the chain applies KL_OP_ANISO5_VAR with in[1] = kx, in[2] = ky (see "Variable coefficients" above
+    // k_chain_tma); the functor's level0 / level then also receive the diagonal of A
+    static constexpr bool VAROP = false;
     // LAG: how many lines level l runs behind level l-1.  With LAG = 1 level l consumes the line level l-1
     // produced in the SAME march step, so a step is one dependent chain of 7L FP64 operations (~250 cycles of
     // latency at L = 4 with 4 warps per scheduler to hide it: the round-1 kernel ran the FP64 pipe at 44 %).
@@ -161,6 +168,46 @@ __device__ __forceinline__ double apply5c(double c, double l, double r, double d
     }
 }
 
+// Variable coefficients (C::VAROP, OPK = KL_OP_ANISO5_VAR, one GPU): every level computes its face weights from the
+// ring -- kx of its own line (columns -1 and +2 by shuffle), ky of lines rho-1, rho, rho+1 -- and hands A u and the
+// diagonal to the functor; level 0 gets the diagonal of its line too (for D^-1 r).  So that level 0 can see ky one
+// line ahead, ky is loaded one line down (ring line R holds ky line R+1; TMA zero-fills line ny), the march starts
+// two lines earlier (the ring's first ky line is then two lines above the first level-0 line that counts) and the
+// ring keeps two more lines.  Level 0 also needs kx one column outside its window, hence one more halo column
+// (ChainDims<L, true>).  The zeros TMA delivers outside the domain are not the boundary rule (a boundary face takes
+// the cell's own coefficient): the checked copy of the march applies the rule, lean hexads lie strictly inside the
+// domain and need none.
+// Face weights, diagonal and (AU) au = A u at the thread's two points of line `row`, same evaluation order as
+// oracle/krylov_extras.c ko_aniso_var.  u: cu = line row, up = row-1, dn = row+1.  All lanes must call it.
+template <bool AU, bool CHK>
+__device__ __forceinline__ void var_apply(const double2 kx, const double2 kyu, const double2 kyc, const double2 kyd,
+                                          const double (&cu)[2], const double (&up)[2], const double (&dn)[2],
+                                          const int gc, const int row, const int nx, const int ny, double (&au)[2],
+                                          double (&dg)[2]) {
+    const double kxs[4] = {__shfl_up_sync(0xffffffffu, kx.y, 1), kx.x, kx.y, __shfl_down_sync(0xffffffffu, kx.x, 1)};
+    double xs[4] = {0.0, cu[0], cu[1], 0.0};
+    if (AU) {
+        xs[0] = __shfl_up_sync(0xffffffffu, cu[1], 1);
+        xs[3] = __shfl_down_sync(0xffffffffu, cu[0], 1);
+    }
+    const double ku[2] = {kyu.x, kyu.y}, kc[2] = {kyc.x, kyc.y}, kd[2] = {kyd.x, kyd.y};
+#pragma unroll
+    for (int e = 0; e < 2; ++e) {
+        const int i = gc + e;
+        const bool hl = !CHK || i > 0, hr = !CHK || i < nx - 1, hu = !CHK || row > 0, hd = !CHK || row < ny - 1;
+        const double kxc = kxs[e + 1];
+        const double wl = hl ? 0.5 * (kxc + kxs[e]) : kxc, wr = hr ? 0.5 * (kxc + kxs[e + 2]) : kxc;
+        const double wu = hu ? 0.5 * (kc[e] + ku[e]) : kc[e], wd = hd ? 0.5 * (kc[e] + kd[e]) : kc[e];
+        dg[e] = ((wl + wr) + wd) + wu;
+        if (AU) {
+            const double xl = hl ? xs[e] : 0.0, xr = hr ? xs[e + 2] : 0.0;
+            const double xu = hu ? up[e] : 0.0, xd = hd ? dn[e] : 0.0;
+            const double s = fma(wl, xl, wr * xr), t = fma(wd, xd, wu * xu);
+            au[e] = fma(dg[e], cu[e], -(s + t));
+        }
+    }
+}
+
 // MG: multi-GPU instantiation (lines above / below the slab come from the neighbours' halo buffers).  It is a
 // template parameter because the patch code in the level-0 path (global loads + ring stores in all six unrolled
 // phases) cost the single-GPU kernels 10-28 % when it was a run-time branch.
@@ -172,7 +219,11 @@ k_chain_tma(const C c_in, const ChainGeo g, const RedCtl rc, const __grid_consta
     f.init();
     constexpr int NIN = C::NIN, L = C::L, NC = C::NC, NRED = C::NRED;
     constexpr int NR_ = NRED > 0 ? NRED : 1;
-    using D = ChainDims<L>;
+    static_assert(C::VAROP == (OPK == KL_OP_ANISO5_VAR) && (!C::VAROP || (NIN == 3 && !MG)), "variable-coefficient chain");
+    // variable coefficients: the march starts VX lines earlier -- ky is loaded one line down, so the first ky line
+    // in the ring is jstart + 1, and level 0 at line R needs ky line R - 1: level 0 is valid from jstart + 2 on
+    constexpr int VX = C::VAROP ? 2 : 0;
+    using D = ChainDims<L, C::VAROP>;
     using RG = ChainRing<C>;
     constexpr int NSIDE = C::NSIDE, NSD = NSIDE > 0 ? NSIDE : 1;
     constexpr int H = D::H, WW = D::WW, BWP = D::BWP;
@@ -184,7 +235,7 @@ k_chain_tma(const C c_in, const ChainGeo g, const RedCtl rc, const __grid_consta
     // rotation period lcm(3, 2) = 6.  (A period-3 march needs a third carried slot, 4 L NC more registers, which the
     // 128-register budget at L = 3, 4 does not have.)
     constexpr int P = RG::P, CCS = 2;
-    constexpr int NB = (LAG * L + P - 1) / P;      // how many periods back raw inputs are re-read
+    constexpr int NB = (LAG * L + (C::VAROP ? 2 : 0) + P - 1) / P;   // how many periods back raw inputs are re-read
     constexpr unsigned kStageBytes = NIN * SR * BWP * sizeof(double);
 
     extern __shared__ __align__(128) unsigned char smem_raw[];
@@ -200,8 +251,8 @@ k_chain_tma(const C c_in, const ChainGeo g, const RedCtl rc, const __grid_consta
     const bool outlane = lane >= H / 2 && lane < 32 - H / 2 && gc < g.nx;
     const int j0 = blockIdx.y * g.rows;
     const int j1 = min(j0 + g.rows, g.ny);
-    const int jstart = j0 - L;                       // grid line of march step 0
-    const int T = (j1 - j0) + L + LAG * L;           // march steps (level L emits line R - LAG*L)
+    const int jstart = j0 - L - VX;                  // grid line of march step 0
+    const int T = (j1 - j0) + L + LAG * L + VX;      // march steps (level L emits line R - LAG*L)
     const int nstg = (T + SR - 1) / SR;
 
     if (tid == 0) {
@@ -218,7 +269,8 @@ k_chain_tma(const C c_in, const ChainGeo g, const RedCtl rc, const __grid_consta
         mbar_expect_tx(&full[s], kStageBytes);
 #pragma unroll
         for (int a = 0; a < NIN; ++a)
-            tma_load_2d(ring + ((size_t)a * NR + (size_t)s * SR) * BWP, &tm.m[a], &full[s], i0 - H, jstart + q * SR);
+            tma_load_2d(ring + ((size_t)a * NR + (size_t)s * SR) * BWP, &tm.m[a], &full[s], i0 - H,
+                        jstart + q * SR + ((C::VAROP && a == 2) ? 1 : 0));
     };
     if (tid == 0) {
         for (int q = 0; q < NST && q < nstg; ++q) issue(q);
@@ -251,6 +303,11 @@ k_chain_tma(const C c_in, const ChainGeo g, const RedCtl rc, const __grid_consta
     for (int k = 0; k <= NB; ++k) rbase[k] = tb;
     const double *&cur = rbase[0];
     int q = 0;                        // stage of the current march step
+    // input a at ring line (current period + kk), kk >= -NB*P (compile time after unrolling)
+    auto ring_at = [&](int a, int kk) -> double2 {
+        const int bk = kk >= 0 ? 0 : (-kk + P - 1) / P;
+        return *reinterpret_cast<const double2 *>(rbase[bk] + ((size_t)a * NR + (size_t)(kk + bk * P)) * BWP);
+    };
 
     // one march step; PH = step index mod 6 (compile time), t = step index.  LEAN: the step belongs to a hexad
     // in which the last level's line is inside [j0, j1) for all six steps, of a CTA whose windows and lines all
@@ -296,7 +353,14 @@ k_chain_tma(const C c_in, const ChainGeo g, const RedCtl rc, const __grid_consta
                 }
             }
             const bool out = outlane && R >= j0 && R < j1;
-            f.level0(out, (size_t)R * g.nx + gc, raw, U[0][PH % 3], CC[0][PH % CCS], acc);
+            if constexpr (C::VAROP) {
+                double dg[2], au_unused[2];
+                var_apply<false, !LEAN>(ring_at(1, PH), ring_at(2, PH - 2), ring_at(2, PH - 1), ring_at(2, PH),
+                                        U[0][PH % 3], U[0][PH % 3], U[0][PH % 3], gc, R, g.nx, g.ny, au_unused, dg);
+                f.level0(out, (size_t)R * g.nx + gc, raw, dg, U[0][PH % 3], CC[0][PH % CCS], acc);
+            } else {
+                f.level0(out, (size_t)R * g.nx + gc, raw, U[0][PH % 3], CC[0][PH % CCS], acc);
+            }
         };
         if (LAG == 1) level_zero();
         // ---- levels 1..L (LAG 1: ascending, each consumes what its predecessor just produced; LAG 2: descending,
@@ -312,13 +376,19 @@ k_chain_tma(const C c_in, const ChainGeo g, const RedCtl rc, const __grid_consta
             const double(&cu)[2] = U[l - 1][sl_cu];
             const double(&up)[2] = U[l - 1][sl_up];
             const double(&dn)[2] = U[l - 1][sl_dn];
-            double lf = __shfl_up_sync(0xffffffffu, cu[1], 1);
-            double rt = __shfl_down_sync(0xffffffffu, cu[0], 1);
-            double au[2];
-            au[0] = apply5c<OPK>(cu[0], lf, cu[1], dn[0], up[0], f.coef);
-            au[1] = apply5c<OPK>(cu[1], cu[0], rt, dn[1], up[1], f.coef);
+            double au[2], dg[2];
             // raw inputs of line rho from the ring (an earlier hexad when PH < LAG*l)
             const int kb = PH - LAG * l;
+            if constexpr (C::VAROP) {
+                // ring line m of ky holds ky line m+1
+                var_apply<true, !LEAN>(ring_at(1, kb), ring_at(2, kb - 2), ring_at(2, kb - 1), ring_at(2, kb), cu, up, dn,
+                                       gc, rho, g.nx, g.ny, au, dg);
+            } else {
+                double lf = __shfl_up_sync(0xffffffffu, cu[1], 1);
+                double rt = __shfl_down_sync(0xffffffffu, cu[0], 1);
+                au[0] = apply5c<OPK>(cu[0], lf, cu[1], dn[0], up[0], f.coef);
+                au[1] = apply5c<OPK>(cu[1], cu[0], rt, dn[1], up[1], f.coef);
+            }
             const int back = kb >= 0 ? 0 : (-kb + P - 1) / P;    // periods back (compile time after unrolling)
             const double *rb = rbase[back] + (size_t)(kb + back * P) * BWP;
             auto rawget = [&](int a) -> double2 {
@@ -332,7 +402,8 @@ k_chain_tma(const C c_in, const ChainGeo g, const RedCtl rc, const __grid_consta
                 sd[a][0] = SD[a][PH % 3][0];
                 sd[a][1] = SD[a][PH % 3][1];
             }
-            f.level(l, out, (size_t)rho * g.nx + gc, cu, au, CC[l - 1][cs_in], rawget, sd, un, cn, acc);
+            if constexpr (C::VAROP) f.level(l, out, (size_t)rho * g.nx + gc, cu, au, dg, CC[l - 1][cs_in], rawget, sd, un, cn, acc);
+            else f.level(l, out, (size_t)rho * g.nx + gc, cu, au, CC[l - 1][cs_in], rawget, sd, un, cn, acc);
             if (l < L) {
                 const bool rowin = LEAN || (rho >= g.row_lo && rho < g.row_hi);
                 const bool m0 = LEAN || (rowin & colin0), m1 = LEAN || (rowin & colin1);
@@ -379,8 +450,9 @@ k_chain_tma(const C c_in, const ChainGeo g, const RedCtl rc, const __grid_consta
     using FF = std::false_type;
 
     // a CTA is lean when every column of its four windows and every line it touches is inside the domain
-    const bool lean_cta = i0 - H >= 0 && i0 - H + kChainWarps * WW + 2 * H <= g.nx && jstart >= 0 && jstart + T <= g.ny;
-    constexpr int kLeanT0 = L + LAG * L;      // first step whose last-level line is >= j0
+    // (variable coefficients: and VX lines below, so that no line a lean hexad reads ky from is a boundary line)
+    const bool lean_cta = i0 - H >= 0 && i0 - H + kChainWarps * WW + 2 * H <= g.nx && jstart >= 0 && jstart + T + VX <= g.ny;
+    constexpr int kLeanT0 = L + LAG * L + VX; // first step whose last-level line is >= j0
 
     // Two copies of the march per kernel: a fast one for whole hexads and the generic, step-by-step checked one.
     //   LEAN kernels : fast = lean hexads of interior CTAs ; generic = first hexads, the partial last one, edge CTAs
@@ -454,9 +526,9 @@ k_chain_tma(const C c_in, const ChainGeo g, const RedCtl rc, const __grid_consta
 int tmap_encode_box(Ctx *c, CUtensorMap *out, const double *base, int nx, int ny, int box_x, int box_y);
 
 // lines per CTA: the redundant work is 2L / rows; keep it below ~10 % but leave >= ~3 CTAs per SM.
-template <int L>
+template <int L, bool VAR = false>
 inline bool chain_geometry(Ctx *c, int nx, int ny, ChainGeo *g, dim3 *grid, bool single_input = false) {
-    const long gx = (nx + ChainDims<L>::STRIP - 1) / ChainDims<L>::STRIP;
+    const long gx = (nx + ChainDims<L, VAR>::STRIP - 1) / ChainDims<L, VAR>::STRIP;
     if (gx > kMaxBlocks) return false;
     // measured at 8192^2 (profiles/r02_chain_rows_sweep.txt): L <= 3 is flat between 24L and 64L lines; from L = 4 on
     // the single-input chains like longer marches (fewer redundant lines, more lean hexads): L = 4: 392 / 384 / 381 /
@@ -486,11 +558,11 @@ inline bool chain_geometry(Ctx *c, int nx, int ny, ChainGeo *g, dim3 *grid, bool
 template <class C, class Post>
 inline int launch_chain(Ctx *c, const kl_operator_t *op, C f, int nx, int ny, const Post &post, int red_src = 0) {
     constexpr int L = C::L;
-    using D = ChainDims<L>;
+    using D = ChainDims<L, C::VAROP>;
     using RG = ChainRing<C>;
     ChainGeo g;
     dim3 grid;
-    if (!chain_geometry<L>(c, nx, ny, &g, &grid, C::NIN == 1))
+    if (!chain_geometry<L, C::VAROP>(c, nx, ny, &g, &grid, C::NIN == 1))
         return c->fail(KL_ERR_UNSUPPORTED, "grid too wide for the reduction buffer");
     // lines of the neighbour ranks are unknowns too (recomputed redundantly level by level)
     if (f.lo[0]) g.row_lo = -L;
@@ -511,10 +583,16 @@ inline int launch_chain(Ctx *c, const kl_operator_t *op, C f, int nx, int ny, co
     }
 #define KL_CH_LAUNCH(OPK)                                                                              \
     if (f.lo[0] || f.hi[0]) KL_CH_LAUNCH1(OPK, true) else KL_CH_LAUNCH1(OPK, false)
-    switch (op->kind) {
-        case KL_OP_POISSON5: KL_CH_LAUNCH(KL_OP_POISSON5) break;
-        case KL_OP_ANISO5: KL_CH_LAUNCH(KL_OP_ANISO5) break;
-        default: return c->fail(KL_ERR_INVALID, "launch_chain: not a built-in operator");
+    if constexpr (C::VAROP) {
+        if (op->kind != KL_OP_ANISO5_VAR || f.lo[0] || f.hi[0])
+            return c->fail(KL_ERR_INVALID, "launch_chain: variable-coefficient chain on another operator");
+        KL_CH_LAUNCH1(KL_OP_ANISO5_VAR, false)
+    } else {
+        switch (op->kind) {
+            case KL_OP_POISSON5: KL_CH_LAUNCH(KL_OP_POISSON5) break;
+            case KL_OP_ANISO5: KL_CH_LAUNCH(KL_OP_ANISO5) break;
+            default: return c->fail(KL_ERR_INVALID, "launch_chain: not a built-in operator");
+        }
     }
 #undef KL_CH_LAUNCH
 #undef KL_CH_LAUNCH1
@@ -609,6 +687,55 @@ struct ChChebCont : ChainBase<3, L_, 1, 2> {
         }
         if (lv == L_ && out) {
             stg2(z + idx, u[0], u[1]);
+#pragma unroll
+            for (int e = 0; e < 2; ++e) {
+                acc[0] = fma(u[e], u[e], acc[0]);
+                acc[1] = fma(r2[e], u[e], acc[1]);
+            }
+        }
+    }
+};
+
+// ---------------------------------------------------------------------------
+// degree-L Jacobi-scaled Chebyshev on KL_OP_ANISO5_VAR in one pass (definition: tests/jacobi_cheb_twin.c):
+//   level 0: u = (r*dinv)/theta, d = u ;  level l: d = fma(c1[l], d, c2[l]*((r - A u)*dinv)) ; u = u + d ;  z = u_L
+// dinv = RN(1/diag) with the diagonal the kernel hands over.  Same arithmetic per point as k_jacobi_cheb_step
+// (kl_ops.cu).  in = {r, kx, ky}: 24n B in, 8n B out (16n with d_out).  Reductions as ChCheb.
+// ---------------------------------------------------------------------------
+template <int L_>
+struct ChJacCheb : ChainBase<3, L_, 1, 2> {
+    static constexpr bool VAROP = true;
+    static constexpr int SR = 2, NST = 6;       // 12-line ring: keeps up to L + 2 lines behind the march
+    static constexpr int MINB = L_ <= 4 ? 3 : 2;   // 60-74 KB of ring per CTA: 3 CTAs per SM at most; L = 5, 6 spill under
+                                                    // the 168-register cap of 3
+    double *z, *d_out;     // d_out != nullptr: also store d_L (continuation with k_jacobi_cheb_step beyond kChainMaxL)
+    int mode;              // 0: the sums are not used ; 1: z.z ; 2: r.z   (host side only)
+    double theta;
+    double c1[L_], c2[L_];
+    FastDiv fd;
+    __device__ __forceinline__ void init() { fd.set(theta); }
+    __device__ __forceinline__ void level0(bool, size_t, const double (&raw)[3][2], const double (&dg)[2],
+                                           double (&u)[2], double (&cc)[1][2], double *) const {
+        fd.div2(raw[0][0] * __drcp_rn(dg[0]), raw[0][1] * __drcp_rn(dg[1]), u[0], u[1]);
+        cc[0][0] = u[0];
+        cc[0][1] = u[1];
+    }
+    template <class RAW>
+    __device__ __forceinline__ void level(int lv, bool out, size_t idx, const double (&up)[2], const double (&au)[2],
+                                          const double (&dg)[2], const double (&cin)[1][2], RAW raw,
+                                          const double (&)[1][2], double (&u)[2], double (&cout)[1][2],
+                                          double *acc) const {
+        const double2 rr = raw(0);
+        const double r2[2] = {rr.x, rr.y};
+#pragma unroll
+        for (int e = 0; e < 2; ++e) {
+            const double d = fma(c1[lv - 1], cin[0][e], c2[lv - 1] * ((r2[e] - au[e]) * __drcp_rn(dg[e])));
+            u[e] = up[e] + d;
+            cout[0][e] = d;
+        }
+        if (lv == L_ && out) {
+            stg2(z + idx, u[0], u[1]);
+            if (d_out) stg2(d_out + idx, cout[0][0], cout[0][1]);
 #pragma unroll
             for (int e = 0; e < 2; ++e) {
                 acc[0] = fma(u[e], u[e], acc[0]);

@@ -2,6 +2,8 @@
 #include <math.h>
 #include <string.h>
 
+#include <cmath>
+
 #include "kl_ops.cuh"
 
 namespace kl {
@@ -35,6 +37,18 @@ int prob_init(Prob *P, Ctx *c, const kl_operator_t *op, const kl_precond_t *pc, 
     for (int i = 0; i < 8; ++i) P->params[i] = (params && i < P->nparams) ? params[i] : 0.0;
     if ((P->pc.kind == KL_PC_CBPR2 || P->pc.kind == KL_PC_CHEB) && P->nparams < 2)
         return c->fail(KL_ERR_INVALID, "Chebyshev preconditioners need params(1:2)");
+    if (P->pc.kind == KL_PC_JACOBI_CHEB) {
+        if (P->op.kind != KL_OP_ANISO5_VAR)
+            return c->fail(KL_ERR_UNSUPPORTED, "KL_PC_JACOBI_CHEB needs KL_OP_ANISO5_VAR; constant-diagonal operators use "
+                                               "KL_PC_CHEB with the interval scaled by their diagonal");
+        if (P->pc.degree < 0) return c->fail(KL_ERR_INVALID, "KL_PC_JACOBI_CHEB: degree >= 0");
+        if (P->pc.degree >= 1) {
+            if (P->nparams < 2) return c->fail(KL_ERR_INVALID, "KL_PC_JACOBI_CHEB of degree >= 1 needs params(1:2)");
+            const double a = P->params[0], b = P->params[1];
+            if (!(std::isfinite(a) && std::isfinite(b) && a > 0.0 && b > 0.0 && a != b))
+                return c->fail(KL_ERR_INVALID, "KL_PC_JACOBI_CHEB: params(1:2) must be distinct finite positive numbers");
+        }
+    }
     P->nx = nx;
     P->ny = ny;
     kl_partition(c, ny, &P->j0, &P->nyl);
@@ -103,6 +117,46 @@ k_aniso_var(const double *__restrict__ x, double *__restrict__ y, const double *
     const double diag = ((wl + wr) + wd) + wu;
     const double s = fma(wl, xl, wr * xr), t = fma(wd, xd, wu * xu);
     y[idx] = fma(diag, xc, -(s + t));
+}
+
+// Jacobi-scaled Chebyshev on KL_OP_ANISO5_VAR, one pass per step (definition: tests/jacobi_cheb_twin.c;
+// same arithmetic per point as the chained ChJacCheb, kl_chain_tma.cuh).  Serves odd nx, nx < 64, the chain switched
+// off (KL_OPT_TMA / KL_OPT_FUSE / KL_OPT_CHAIN) and every step beyond kChainMaxL.  dinv = RN(1/diag) is recomputed
+// from kx, ky in every pass.  kind 2: z = r*dinv (degree 0) ; kind 1: the start, d = z = (r*dinv)/theta ;
+// kind 0: one step, d = fma(c1, d, c2*((r - A zin)*dinv)), z = zin + d.  Step: 56n B (r, zin, d, kx, ky in; d, z out).
+__global__ void __launch_bounds__(256)
+k_jacobi_cheb_step(const double *__restrict__ r, const double *__restrict__ zin, double *__restrict__ d,
+                   double *__restrict__ z, const double *__restrict__ kx, const double *__restrict__ ky, const int nx,
+                   const int ny, const double theta, const double c1, const double c2, const int kind,
+                   const int *__restrict__ flags) {
+    if (flags && flags[I_CONV_AT] >= 0) return;
+    const int i = blockIdx.x * 256 + threadIdx.x, j = blockIdx.y;
+    if (i >= nx) return;
+    const size_t idx = (size_t)i + (size_t)j * nx;
+    const double kxc = __ldg(kx + idx), kyc = __ldg(ky + idx);
+    const bool hl = i > 0, hr = i < nx - 1, hu = j > 0, hd = j < ny - 1;
+    const double wl = hl ? 0.5 * (kxc + __ldg(kx + idx - 1)) : kxc, wr = hr ? 0.5 * (kxc + __ldg(kx + idx + 1)) : kxc;
+    const double wu = hu ? 0.5 * (kyc + __ldg(ky + idx - nx)) : kyc, wd = hd ? 0.5 * (kyc + __ldg(ky + idx + nx)) : kyc;
+    const double diag = ((wl + wr) + wd) + wu;
+    const double dinv = __drcp_rn(diag), rc = __ldg(r + idx);
+    if (kind == 2) {
+        z[idx] = rc * dinv;
+        return;
+    }
+    if (kind == 1) {
+        const double d0 = (rc * dinv) / theta;
+        d[idx] = d0;
+        z[idx] = d0;
+        return;
+    }
+    const double xc = __ldg(zin + idx);
+    const double xl = hl ? __ldg(zin + idx - 1) : 0.0, xr = hr ? __ldg(zin + idx + 1) : 0.0;
+    const double xd = hd ? __ldg(zin + idx + nx) : 0.0, xu = hu ? __ldg(zin + idx - nx) : 0.0;
+    const double s = fma(wl, xl, wr * xr), t = fma(wd, xd, wu * xu);
+    const double az = fma(diag, xc, -(s + t));
+    const double dn = fma(c1, d[idx], c2 * ((rc - az) * dinv));
+    d[idx] = dn;
+    z[idx] = xc + dn;
 }
 
 int op_apply(Prob *P, const double *x, double *y, bool gated) {
@@ -193,10 +247,84 @@ struct FChebStep : StencilBase<1, (MODE ? 1 : 0)> {
     }
 };
 
+// KL_PC_JACOBI_CHEB (prob_init admits it on KL_OP_ANISO5_VAR only, which runs on one GPU)
+static int pc_jacobi_cheb(Prob *P, const double *r, double *z, double *aux, double *aux2, int mode, bool gated,
+                          const PostAny &post) {
+    Ctx *c = P->c;
+    const kl_aniso_var_t *cf = (const kl_aniso_var_t *)P->op.user;
+    const int k = P->pc.degree;
+    const dim3 grid((unsigned)((P->nx + 255) / 256), (unsigned)P->nyl);
+    const int *flags = gated ? c->d_I : nullptr;
+    auto pass = [&](const double *zin, double *zout, double theta, double c1, double c2, int kind) {
+        k_jacobi_cheb_step<<<grid, 256, 0, c->stream>>>(r, zin, aux2, zout, cf->kx, cf->ky, P->nx, P->nyl, theta, c1, c2,
+                                                        kind, flags);
+        c->stats.kernel_launches++;
+    };
+    if (k == 0) {
+        pass(nullptr, z, 0.0, 0.0, 0.0, 2);
+    } else {
+        // Saad Alg. 12.1 on D^-1 A; coefficients on the host (same arithmetic as the oracle and KL_PC_CHEB)
+        const double ea = P->params[0], eb = P->params[1];
+        const double theta = (eb + ea) / 2.0, delta = fabs(eb - ea) / 2.0;
+        const double sigma = theta / delta;
+        double rho_prev = 1.0 / sigma;
+        // ping-pong so that the final result lands in z: z_s lives in zb[(k - s) & 1], d in aux2
+        double *zb[2] = {z, aux};
+        const int kc = k < kChainMaxL ? k : kChainMaxL;
+        int s0 = 0;
+        if (chain_ok(P, kc)) {
+            // the first min(k, 6) steps in ONE pass over r, kx, ky (kl_chain_tma.cuh ChJacCheb): 32n B
+            double c1s[kChainMaxL], c2s[kChainMaxL];
+            for (int s = 0; s < kc; ++s) {
+                const double rho = 1.0 / (2.0 * sigma - rho_prev);
+                c1s[s] = rho * rho_prev;
+                c2s[s] = 2.0 * rho / delta;
+                rho_prev = rho;
+            }
+            const double *in[3] = {r, cf->kx, cf->ky};
+            const Halo H = {};
+            double *dst = (kc == k) ? z : zb[(k - kc) & 1];
+#define KL_JC(LL)                                                                       \
+    case LL: {                                                                          \
+        ChJacCheb<LL> f;                                                                \
+        set_io(f, P, in, H);                                                            \
+        set_gate(f, c, gated);                                                          \
+        f.z = dst; f.d_out = (kc == k) ? nullptr : aux2; f.mode = (kc == k) ? mode : 0; \
+        f.theta = theta;                                                                \
+        for (int s = 0; s < LL; ++s) { f.c1[s] = c1s[s]; f.c2[s] = c2s[s]; }            \
+        if (kc == k && mode != 0) { KL_TRY(launch_chain(c, &P->op, f, P->nx, P->nyl, post, mode == 2 ? 1 : 0)); } \
+        else { KL_TRY(launch_chain(c, &P->op, f, P->nx, P->nyl, NoPost{})); }           \
+    } break;
+            switch (kc) {
+                KL_JC(1) KL_JC(2) KL_JC(3) KL_JC(4) KL_JC(5) KL_JC(6)
+                default: return c->fail(KL_ERR_INVALID, "jacobi-chebyshev chain length");
+            }
+#undef KL_JC
+            if (kc == k) return KL_OK;
+            s0 = kc;
+        } else {
+            pass(nullptr, zb[k & 1], theta, 0.0, 0.0, 1);
+        }
+        for (int s = s0; s < k; ++s) {
+            const double rho = 1.0 / (2.0 * sigma - rho_prev);
+            pass(zb[(k - s) & 1], zb[(k - s - 1) & 1], theta, rho * rho_prev, 2.0 * rho / delta, 0);
+            rho_prev = rho;
+        }
+    }
+    if (mode != 0) {
+        PDot2 dt;
+        set_gate(dt, c, gated);
+        dt.a = (mode == 1) ? z : r; dt.b = z; dt.c = nullptr; dt.d = nullptr;
+        KL_TRY(launch_pointwise(c, dt, P->n, post));
+    }
+    return KL_OK;
+}
+
 int pc_apply_any(Prob *P, const double *r, double *z, double *aux, double *aux2, int mode, bool gated,
                  const PostAny &post) {
     Ctx *c = P->c;
     const int kind = P->pc.kind;
+    if (kind == KL_PC_JACOBI_CHEB) return pc_jacobi_cheb(P, r, z, aux, aux2, mode, gated, post);
     if (kind == KL_PC_CBPR2 && P->builtin_op()) {
         Cbpr2Coef cf = cbpr2_coef(P->params);
         Halo H;

@@ -72,7 +72,7 @@ int gmres_hh_solve(Ctx *c, const kl_operator_t *A, const double *b, double *x, i
 // z = b - A x
 int op_resid(Prob *P, const double *x, const double *b, double *z, bool gated);
 // z = M^-1 r ; mode 0: no reduction, 1: S_RED[0] = sum z*z, 2: S_RED[0] = sum r*z.
-// aux/aux2: scratch vectors (aux2 only needed for KL_PC_CHEB).  For KL_PC_NONE
+// aux/aux2: scratch vectors (aux2 only needed for KL_PC_CHEB and KL_PC_JACOBI_CHEB).  For KL_PC_NONE
 // z = r is a copy.  `post` runs after the reduction (mode != 0).
 // (compiled once, in kl_ops.cu: the post functor is a run-time PostAny, so the Chebyshev chain kernels and the
 // cbpr2 / Chebyshev-step stencil kernels are instantiated in ONE translation unit instead of in every solver's)

@@ -89,11 +89,21 @@ enum {
     KL_PC_NONE = 0,
     KL_PC_CBPR2 = 1,  /* chebyshev_precond::cbpr2  src/preconds/chebyshev.f90:8-38 */
     KL_PC_CHEB = 2,   /* degree-k Chebyshev iteration (new; README.md:11)          */
+    KL_PC_JACOBI_CHEB = 3, /* degree-k Chebyshev iteration on the Jacobi-scaled operator D^-1 A, D = diag(A), for
+                          KL_OP_ANISO5_VAR only (new).  degree 0: z = D^-1 r (point Jacobi), params ignored; degree
+                          k >= 1: params = (a, b), an interval of the spectrum of D^-1 A in either order.  That
+                          spectrum lies in (0, 2] for every positive coefficient field (Gershgorin: the off-diagonal
+                          row sums of A are at most its diagonal), so b = 2 needs no estimate, and
+                          kl_cheb_interval_from_ritz(2.0 / 1.025, k) yields (2, 2/ratio(k)) from the measured ratio
+                          table.  Degree k <= 6 runs as ONE temporally blocked pass (r, kx, ky in, z out: 32n B)
+                          on even nx >= 64 with KL_OPT_TMA, KL_OPT_FUSE and KL_OPT_CHAIN on; otherwise, and for
+                          the steps beyond the sixth, one pass per step.  Constant-diagonal operators use
+                          KL_PC_CHEB with the interval scaled by their diagonal.                              */
     KL_PC_USER = 100
 };
 typedef struct {
     int kind;
-    int degree;        /* KL_PC_CHEB */
+    int degree;        /* KL_PC_CHEB, KL_PC_JACOBI_CHEB */
     kl_precond_fn fn;  /* KL_PC_USER */
     void *user;
 } kl_precond_t;

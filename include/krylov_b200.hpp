@@ -40,6 +40,8 @@ inline kl_operator_t aniso(double ex, double ey) { return kl_operator_t{KL_OP_AN
 inline const kl_precond_t cbpr2{KL_PC_CBPR2, 0, nullptr, nullptr};
 inline const kl_precond_t no_precond{KL_PC_NONE, 0, nullptr, nullptr};
 inline kl_precond_t cheb(int degree) { return kl_precond_t{KL_PC_CHEB, degree, nullptr, nullptr}; }
+// Chebyshev on the Jacobi-scaled operator D^-1 A (variable-coefficient operators only; degree 0 = point Jacobi)
+inline kl_precond_t jacobi_cheb(int degree) { return kl_precond_t{KL_PC_JACOBI_CHEB, degree, nullptr, nullptr}; }
 
 class Handle {
 public:
