@@ -25,6 +25,9 @@ from .api import (  # noqa: F401
     stv_poisson,
     aniso,
     aniso_var,
+    stencil5,
+    convdiff,
+    stencil5_spectrum,
     cbpr2,
     cheb,
     jacobi_cheb,
@@ -44,9 +47,10 @@ from .api import (  # noqa: F401
     KL_OPT_CHECK_EVERY,
     KL_OPT_X0,
     KL_PC_JACOBI_CHEB,
+    KL_OP_STENCIL5,
 )
 
 __all__ = [
     "Handle", "KrylovError", "Operator", "Precond", "GmresResult", "CgResult", "stvec",
-    "stv_poisson", "aniso", "cbpr2", "cheb", "jacobi_cheb", "no_precond", "library_path", "load_library",
+    "stv_poisson", "aniso", "stencil5", "convdiff", "stencil5_spectrum", "cbpr2", "cheb", "jacobi_cheb", "no_precond", "library_path", "load_library",
 ]

@@ -31,7 +31,8 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 _LIBNAME = "libkrylov_b200.so"
 
 KL_OK, KL_NOT_CONVERGED, KL_BREAKDOWN = 0, 1, 2
-KL_OP_POISSON5, KL_OP_POISSON5_BRANCHY, KL_OP_ANISO5, KL_OP_ANISO5_VAR, KL_OP_USER = 0, 1, 2, 4, 100
+KL_OP_POISSON5, KL_OP_POISSON5_BRANCHY, KL_OP_ANISO5, KL_OP_ANISO5_VAR, KL_OP_STENCIL5, KL_OP_USER = 0, 1, 2, 4, 5, 100
+KL_ERR_INVALID, KL_ERR_UNSUPPORTED = -1, -5
 KL_PC_NONE, KL_PC_CBPR2, KL_PC_CHEB, KL_PC_JACOBI_CHEB, KL_PC_USER = 0, 1, 2, 3, 100
 KL_POINTER_HOST, KL_POINTER_DEVICE = 0, 1
 (KL_OPT_ORTHO, KL_OPT_MAX_RESTARTS, KL_OPT_VERR, KL_OPT_CHECK_EVERY, KL_OPT_USE_GRAPH,
@@ -57,6 +58,10 @@ class kl_operator_t(C.Structure):
 
 class kl_aniso_var_t(C.Structure):
     _fields_ = [("kx", C.c_void_p), ("ky", C.c_void_p)]
+
+
+class kl_stencil5_t(C.Structure):
+    _fields_ = [("c", C.c_double), ("wl", C.c_double), ("wr", C.c_double), ("wd", C.c_double), ("wu", C.c_double)]
 
 
 class kl_precond_t(C.Structure):
@@ -132,6 +137,7 @@ def load_library():
     L.kl_lanczos.argtypes = [C.c_void_p, C.POINTER(kl_operator_t), C.c_int, C.c_int, C.c_int, _dp, _dp]
     L.kl_cheb_params_from_ritz.argtypes = [C.c_double, C.c_double, _dp]
     L.kl_cheb_interval_from_ritz.argtypes = [C.c_double, C.c_int, _dp]
+    L.kl_stencil5_spectrum.argtypes = [C.POINTER(kl_stencil5_t), C.c_int, C.c_int, _dp, _dp]
     L.kl_get_history.argtypes = [C.c_void_p, _dp, C.c_int, _ip]
     L.kl_get_stats.argtypes = [C.c_void_p, C.POINTER(kl_stats_t)]
     L.kl_get_profile.argtypes = [C.c_void_p, C.c_int, C.POINTER(C.c_char_p), _dp, C.POINTER(C.c_longlong), _dp]
@@ -154,6 +160,7 @@ class Operator:
     eps_y: float = 1.0
     fn: Optional[object] = None  # python callable(d_x:int, d_y:int, nx, ny_local, stream:int) for KL_OP_USER
     coef: Optional[tuple] = None  # (kx, ky) CUDA float64 tensors for KL_OP_ANISO5_VAR
+    w5: Optional[tuple] = None    # (c, wl, wr, wd, wu) for KL_OP_STENCIL5
 
     def _c(self):
         o = kl_operator_t()
@@ -162,6 +169,9 @@ class Operator:
         if self.kind == KL_OP_ANISO5_VAR:
             kx, ky = self.coef
             keep = kl_aniso_var_t(C.c_void_p(kx.data_ptr()), C.c_void_p(ky.data_ptr()))
+            o.user = C.cast(C.pointer(keep), C.c_void_p)
+        if self.kind == KL_OP_STENCIL5:
+            keep = kl_stencil5_t(*self.w5)
             o.user = C.cast(C.pointer(keep), C.c_void_p)
         if self.kind == KL_OP_USER:
             f = self.fn
@@ -237,6 +247,59 @@ def aniso_var(kx, ky) -> Operator:
         return torch.from_numpy(np.ascontiguousarray(a, dtype=np.float64).reshape(-1)).cuda()
 
     return Operator(KL_OP_ANISO5_VAR, coef=(dev(kx), dev(ky)))
+
+
+def stencil5(c: float, wl: float, wr: float, wd: float, wu: float) -> Operator:
+    """General constant-coefficient 5-point operator with zero Dirichlet boundary (KL_OP_STENCIL5):
+        y(i,j) = c x(i,j) - (wl x(i-1,j) + wr x(i+1,j) + wd x(i,j+1) + wu x(i,j-1)),   idx = i + j*nx
+    ("d" is the next line idx+nx, "u" the previous one idx-nx).  Every weight must be a finite real number.  It is
+    nonsymmetric unless wl == wr and wd == wu; CG, PCG and lanczos refuse it then.  One GPU only."""
+    w = []
+    for name, v in (("c", c), ("wl", wl), ("wr", wr), ("wd", wd), ("wu", wu)):
+        if isinstance(v, (bool, np.bool_)) or not isinstance(v, (int, float, np.integer, np.floating)):
+            raise KrylovError(f"stencil5: weight {name} must be a real number, got {type(v).__name__}")
+        f = float(v)
+        if not np.isfinite(f):
+            raise KrylovError(f"stencil5: weight {name} must be finite, got {f}")
+        w.append(f)
+    return Operator(KL_OP_STENCIL5, w5=tuple(w))
+
+
+def convdiff(px: float, py: float, upwind: bool = False) -> Operator:
+    """Convection-diffusion -lap(u) + b.grad(u) on a grid of spacing h, scaled by h^2 (KL_OP_STENCIL5), in terms of the
+    cell Peclet numbers px = bx*h/2 and py = by*h/2.
+      central: c = 4, wl = 1 + px, wr = 1 - px, wu = 1 + py, wd = 1 - py.  The spectrum is real iff |px|, |py| <= 1.
+      upwind (first order): c = (4 + 2|px|) + 2|py|; the upstream weight (wl for px > 0, wr for px < 0; wu for py > 0,
+      wd for py < 0) is 1 + 2|p|, the other one 1.  The spectrum is always real."""
+    for name, v in (("px", px), ("py", py)):
+        if isinstance(v, (bool, np.bool_)) or not isinstance(v, (int, float, np.integer, np.floating)) or \
+                not np.isfinite(float(v)):
+            raise KrylovError(f"convdiff: {name} must be a finite real number")
+    px, py = float(px), float(py)
+    if not upwind:
+        return stencil5(4.0, 1.0 + px, 1.0 - px, 1.0 - py, 1.0 + py)
+    ax, ay = abs(px), abs(py)
+    wl, wr = (1.0 + 2.0 * ax, 1.0) if px >= 0 else (1.0, 1.0 + 2.0 * ax)
+    wu, wd = (1.0 + 2.0 * ay, 1.0) if py >= 0 else (1.0, 1.0 + 2.0 * ay)
+    return stencil5((4.0 + 2.0 * ax) + 2.0 * ay, wl, wr, wd, wu)
+
+
+def stencil5_spectrum(op: Operator, nx: int, ny: int):
+    """(lam_min, lam_max): the exact extremes of the Dirichlet spectrum of a stencil5 operator on an nx x ny grid
+    (kl_stencil5_spectrum, host arithmetic, no GPU needed).  Raises KrylovError when the spectrum is complex
+    (wl*wr < 0 or wd*wu < 0).  (lam_min, lam_max) is the exact interval for cheb(k)."""
+    if not isinstance(op, Operator) or op.kind != KL_OP_STENCIL5:
+        raise KrylovError("stencil5_spectrum: op must be a stencil5 / convdiff operator")
+    if int(nx) < 1 or int(ny) < 1:
+        raise KrylovError("stencil5_spectrum: nx, ny >= 1")
+    w = kl_stencil5_t(*op.w5)
+    lo, hi = C.c_double(), C.c_double()
+    rc = load_library().kl_stencil5_spectrum(C.byref(w), int(nx), int(ny), C.byref(lo), C.byref(hi))
+    if rc == KL_ERR_UNSUPPORTED:
+        raise KrylovError("stencil5_spectrum: the spectrum is complex (wl*wr < 0 or wd*wu < 0)")
+    if rc != 0:
+        raise KrylovError(f"kl_stencil5_spectrum failed with {rc}")
+    return lo.value, hi.value
 
 
 def cheb(degree: int) -> Precond:

@@ -317,6 +317,9 @@ static int cg_solve(Ctx *c, const kl_operator_t *A, const double *b, double *x, 
     KL_TRY(x0_check(c, b, x));
     Prob P;
     KL_TRY(prob_init(&P, c, A, M, params, nparams, nx, ny));
+    if (!P.symmetric())
+        return c->fail(KL_ERR_UNSUPPORTED, "CG / PCG need a symmetric operator: KL_OP_STENCIL5 with wl != wr or wd != wu "
+                                           "takes GMRES or BiCGSTAB");
     const bool prec = P.pc.kind != KL_PC_NONE;
     const bool fused = c->opt_fuse && P.builtin_op();
     const size_t n = P.n;
@@ -599,7 +602,7 @@ static int cg_solve(Ctx *c, const kl_operator_t *A, const double *b, double *x, 
         Ctx::GraphEntry *ge = nullptr;
         if (use_graph && batch % 2 == 0 && done % 2 == 0) {
             GraphKey gk;
-            gk.add('C').add(nx).add(ny).add(batch).add(P.op.kind).add(P.op.eps_x).add(P.op.eps_y).add(P.pc.kind)
+            gk.add('C').add(nx).add(ny).add(batch).add(P.op.kind).add(P.op.eps_x).add(P.op.eps_y).add(P.w5).add(P.pc.kind)
                 .add(P.pc.degree).add(P.params).add(c->opt_tma).add(c->opt_chain).add(c->opt_stencil_rows)
                 .add(c->opt_stencil_tail).add(c->opt_stencil_stagger).add(c->opt_pdl).add(c->opt_reverse).add(c->opt_persistent)
                 .add(c->ws).add(dx).add(r).add(pold)

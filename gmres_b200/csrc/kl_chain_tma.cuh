@@ -161,6 +161,9 @@ __device__ __forceinline__ double apply5c(double c, double l, double r, double d
         return fma(4.0, c, -(((l + r) + dn) + up));
     } else if (OPK == KL_OP_POISSON5_BRANCHY) {
         return ((fma(4.0, c, -l) - r) - up) - dn;
+    } else if (OPK == KL_OP_STENCIL5) {
+        double s = fma(k.ex, l, k.exr * r), t = fma(k.ey, dn, k.eyu * up);
+        return fma(k.cc, c, -(s + t));
     } else {
         double sx = l + r, sy = dn + up;
         double t = fma(k.ex, sx, k.ey * sy);
@@ -567,7 +570,7 @@ inline int launch_chain(Ctx *c, const kl_operator_t *op, C f, int nx, int ny, co
     // lines of the neighbour ranks are unknowns too (recomputed redundantly level by level)
     if (f.lo[0]) g.row_lo = -L;
     if (f.hi[0]) g.row_hi = ny + L;
-    f.coef = OpCoef{op->eps_x, op->eps_y, 2.0 * (op->eps_x + op->eps_y)};
+    f.coef = op_coef(op);
     RedCtl rc = redctl(c);
     TMaps<C::NIN> tm;
     for (int a = 0; a < C::NIN; ++a) KL_TRY(tmap_encode_box(c, &tm.m[a], f.in[a], nx, ny, D::BWP, RG::SR));
@@ -591,6 +594,10 @@ inline int launch_chain(Ctx *c, const kl_operator_t *op, C f, int nx, int ny, co
         switch (op->kind) {
             case KL_OP_POISSON5: KL_CH_LAUNCH(KL_OP_POISSON5) break;
             case KL_OP_ANISO5: KL_CH_LAUNCH(KL_OP_ANISO5) break;
+            case KL_OP_STENCIL5:   // one GPU (prob_init): no multi-GPU instantiation
+                if (f.lo[0] || f.hi[0]) return c->fail(KL_ERR_UNSUPPORTED, "launch_chain: KL_OP_STENCIL5 is single-GPU");
+                KL_CH_LAUNCH1(KL_OP_STENCIL5, false)
+                break;
             default: return c->fail(KL_ERR_INVALID, "launch_chain: not a built-in operator");
         }
     }

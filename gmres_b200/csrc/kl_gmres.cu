@@ -808,7 +808,7 @@ int gmres_mgsr_solve(Ctx *c, const kl_operator_t *A, const double *b, double *x,
                            (P.pc.kind == KL_PC_NONE || P.pc.kind == KL_PC_CBPR2 || P.pc.kind == KL_PC_CHEB);
     GraphKey gk;
     if (use_graph) {
-        gk.add('G').add(nx).add(ny).add(m).add(mf).add(P.op.kind).add(P.op.eps_x).add(P.op.eps_y).add(P.pc.kind)
+        gk.add('G').add(nx).add(ny).add(m).add(mf).add(P.op.kind).add(P.op.eps_x).add(P.op.eps_y).add(P.w5).add(P.pc.kind)
             .add(P.pc.degree).add(P.params).add(c->opt_ortho).add(c->opt_reorth_eta_permille).add(c->opt_tma)
             .add(c->opt_chain).add(c->opt_stencil_rows).add(c->opt_stencil_tail).add(c->opt_stencil_stagger)
             .add(c->opt_pdl).add(c->opt_coop).add(c->opt_reverse).add(c->opt_persistent).add(c->ws).add(db).add(dx).add(V).add(G.H);

@@ -651,7 +651,7 @@ int gmres_hh_solve(Ctx *c, const kl_operator_t *A, const double *b, double *x, i
                            (P.pc.kind == KL_PC_NONE || P.pc.kind == KL_PC_CBPR2 || P.pc.kind == KL_PC_CHEB);
     GraphKey gk;
     if (use_graph) {
-        gk.add('H').add(nx).add(ny).add(m).add(prec_variant).add(P.op.kind).add(P.op.eps_x).add(P.op.eps_y)
+        gk.add('H').add(nx).add(ny).add(m).add(prec_variant).add(P.op.kind).add(P.op.eps_x).add(P.op.eps_y).add(P.w5)
             .add(P.pc.kind).add(P.pc.degree).add(P.params).add(c->opt_hh_mode).add(c->opt_tma).add(c->opt_chain)
             .add(c->opt_stencil_rows).add(c->opt_stencil_tail).add(c->opt_stencil_stagger).add(c->opt_verr).add(c->opt_pdl)
             .add(c->opt_reverse).add(c->opt_persistent)

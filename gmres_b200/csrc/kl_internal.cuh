@@ -474,9 +474,19 @@ __device__ __forceinline__ void griddep_launch() { asm volatile("griddepcontrol.
 //   missing neighbours are passed as 0.0 (adding/subtracting 0.0 is exact, so
 //   this reproduces every edge/corner formula of poisson.f90:47-76).
 // ------------------------------------------------------------------------
+// KL_OP_ANISO5: ex = eps_x, ey = eps_y, cc = 2(eps_x + eps_y) ; KL_OP_STENCIL5: ex = wl, ey = wd, cc = c and the two
+// weights of the other side, exr = wr, eyu = wu (op_coef)
 struct OpCoef {
     double ex, ey, cc;
+    double exr, eyu;
 };
+inline OpCoef op_coef(const kl_operator_t *op) {
+    if (op->kind == KL_OP_STENCIL5) {
+        const kl_stencil5_t *w = (const kl_stencil5_t *)op->user;
+        return OpCoef{w->wl, w->wd, w->c, w->wr, w->wu};
+    }
+    return OpCoef{op->eps_x, op->eps_y, 2.0 * (op->eps_x + op->eps_y), 0.0, 0.0};
+}
 template <int OPK>
 __device__ __forceinline__ double apply5(double c, double l, double r, double dn, double up,
                                          const OpCoef &k) {
@@ -486,6 +496,10 @@ __device__ __forceinline__ double apply5(double c, double l, double r, double dn
     } else if (OPK == KL_OP_POISSON5_BRANCHY) {
         // poisson.f90:88-92  ((((4x - x(idx-1)) - x(idx+1)) - x(idx-n)) - x(idx+n))
         return (((4.0 * c - l) - r) - up) - dn;
+    } else if (OPK == KL_OP_STENCIL5) {
+        // krylov_b200.h kl_stencil5_t (the order of k_aniso_var)
+        double s = fma(k.ex, l, k.exr * r), t = fma(k.ey, dn, k.eyu * up);
+        return fma(k.cc, c, -(s + t));
     } else {
         double sx = l + r, sy = dn + up;
         double t = fma(k.ex, sx, k.ey * sy);
@@ -493,8 +507,12 @@ __device__ __forceinline__ double apply5(double c, double l, double r, double dn
     }
 }
 
-// the same with the operator chosen at run time (generic, non-TMA kernel: small and odd grids, KL_OPT_TMA = 0)
+// the same with the operator chosen at run time (generic, non-TMA kernel: small and odd grids, KL_OPT_TMA = 0).
+// S5: KL_OP_STENCIL5, chosen at compile time -- its functors are wrapped in S5<F> (launch_stencil), so that the
+// generic kernels of the other operators carry no fourth branch (it cost them registers and spills)
+template <bool S5 = false>
 __device__ __forceinline__ double apply5_rt(int opk, double c, double l, double r, double dn, double up, const OpCoef &k) {
+    if (S5) return apply5<KL_OP_STENCIL5>(c, l, r, dn, up, k);
     if (opk == KL_OP_POISSON5) return apply5<KL_OP_POISSON5>(c, l, r, dn, up, k);
     if (opk == KL_OP_POISSON5_BRANCHY) return apply5<KL_OP_POISSON5_BRANCHY>(c, l, r, dn, up, k);
     return apply5<KL_OP_ANISO5>(c, l, r, dn, up, k);
@@ -565,6 +583,8 @@ struct StencilBase {
     static constexpr bool kLateWait = false;
     // kReverse: march the grid from its last lines to its first (see Geo::reverse)
     static constexpr bool kReverse = false;
+    // kS5: the generic kernel applies KL_OP_STENCIL5 (set by the S5<F> wrapper only)
+    static constexpr bool kS5 = false;
     __device__ __forceinline__ void late_init() {}
     const double *in[NIN_];
     const double *lo[NIN_];
@@ -578,6 +598,12 @@ struct StencilBase {
         int ca = flags[I_CONV_AT];
         return !(ca < 0 || (run_on_conv && ca == step));
     }
+};
+
+// KL_OP_STENCIL5 on the generic kernel: the functor F with the operator fixed at compile time (apply5_rt<true>)
+template <class F>
+struct S5 : F {
+    static constexpr bool kS5 = true;
 };
 
 constexpr int kStencilThreads = 128;
@@ -693,10 +719,10 @@ k_stencil(const F f_in, const Geo g, const RedCtl rc, const PostAny post, const 
         if (act) {
             double au[VEC];
             if (VEC == 1) {
-                au[0] = apply5_rt(opk, cu[0], l, r, dn[0], up[0], f.coef);
+                au[0] = apply5_rt<F::kS5>(opk, cu[0], l, r, dn[0], up[0], f.coef);
             } else {
-                au[0] = apply5_rt(opk, cu[0], l, cu[VEC - 1], dn[0], up[0], f.coef);
-                au[VEC - 1] = apply5_rt(opk, cu[VEC - 1], cu[0], r, dn[VEC - 1], up[VEC - 1], f.coef);
+                au[0] = apply5_rt<F::kS5>(opk, cu[0], l, cu[VEC - 1], dn[0], up[0], f.coef);
+                au[VEC - 1] = apply5_rt<F::kS5>(opk, cu[VEC - 1], cu[0], r, dn[VEC - 1], up[VEC - 1], f.coef);
             }
             if constexpr (F::kPush)
                 f.template store<VEC>((size_t)j * g.nx + i0, rawCu.c, cu, au, acc, (j == 0 ? 1 : 0) | (j == g.ny - 1 ? 2 : 0));
@@ -932,12 +958,13 @@ template <class F, class Post>
 inline int launch_stencil(Ctx *c, const kl_operator_t *op, F f, int nx, int ny, const Post &post, bool pdl = false) {
     const int vec = (nx % 2 == 0) ? 2 : 1;
     const bool tma = c->opt_tma && vec == 2 && nx >= 64;
-    const int strip = tma ? kTmaStrip : kStencilThreads * vec;
+    // KL_OP_STENCIL5 runs the generic kernel with one column per thread only (S5<F>, VEC = 1: half the instantiations)
+    const int strip = tma ? kTmaStrip : kStencilThreads * (op->kind == KL_OP_STENCIL5 ? 1 : vec);
     Geo g{};
     g.nx = nx; g.ny = ny;
     const int reverse = (F::kReverse && c->opt_reverse) ? 1 : 0;
     dim3 grid;
-    f.coef = OpCoef{op->eps_x, op->eps_y, 2.0 * (op->eps_x + op->eps_y)};
+    f.coef = op_coef(op);
     RedCtl rc = redctl(c);
     const bool inl = F::NRED > 0 && redctl_inline_allreduce(c, rc, F::NRED);
     const int fuse = c->nranks == 1 || inl;
@@ -985,7 +1012,7 @@ inline int launch_stencil(Ctx *c, const kl_operator_t *op, F f, int nx, int ny, 
         cfg.gridDim = grid;                                                                         \
         cfg.dynamicSmemBytes = SMEM;                                                                \
     }
-    if (opk != KL_OP_POISSON5 && opk != KL_OP_POISSON5_BRANCHY && opk != KL_OP_ANISO5)
+    if (opk != KL_OP_POISSON5 && opk != KL_OP_POISSON5_BRANCHY && opk != KL_OP_ANISO5 && opk != KL_OP_STENCIL5)
         return c->fail(KL_ERR_INVALID, "launch_stencil: not a built-in operator");
     // the TMA kernel is specialised per operator (its inner loop is the hot path); the generic kernel takes it as
     // a run-time argument
@@ -997,7 +1024,13 @@ inline int launch_stencil(Ctx *c, const kl_operator_t *op, F f, int nx, int ny, 
     if (tma) {
         if (opk == KL_OP_POISSON5) KL_ST_TMA(KL_OP_POISSON5)
         else if (opk == KL_OP_POISSON5_BRANCHY) KL_ST_TMA(KL_OP_POISSON5_BRANCHY)
+        else if (opk == KL_OP_STENCIL5) KL_ST_TMA(KL_OP_STENCIL5)
         else KL_ST_TMA(KL_OP_ANISO5)
+    } else if (opk == KL_OP_STENCIL5) {
+        S5<F> f5;
+        static_cast<F &>(f5) = f;
+        KL_ST_GEO((k_stencil<S5<F>, 1>), 0)
+        KL_CUDA(c, cudaLaunchKernelEx(&cfg, k_stencil<S5<F>, 1>, f5, g, rc, pa, fuse, opk));
     } else if (vec == 2) {
         KL_ST_GEO((k_stencil<F, 2>), 0)
         KL_CUDA(c, cudaLaunchKernelEx(&cfg, k_stencil<F, 2>, f, g, rc, pa, fuse, opk));

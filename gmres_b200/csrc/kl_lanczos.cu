@@ -100,6 +100,9 @@ extern "C" int kl_lanczos(kl_handle_t h, const kl_operator_t *A, int nx, int ny,
     Ctx *c = h;
     Prob P;
     KL_TRY(prob_init(&P, c, A, nullptr, nullptr, 0, nx, ny));
+    if (!P.symmetric())
+        return c->fail(KL_ERR_UNSUPPORTED, "kl_lanczos needs a symmetric operator: for KL_OP_STENCIL5 use "
+                                           "kl_stencil5_spectrum");
     const size_t n = P.n;
     KL_TRY(ws_reserve(c, 3 * ws_need(n)));
     ws_reset(c);

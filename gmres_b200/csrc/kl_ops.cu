@@ -18,11 +18,26 @@ int prob_init(Prob *P, Ctx *c, const kl_operator_t *op, const kl_precond_t *pc, 
     } else if (nx < 2 || ny < 2) return c->fail(KL_ERR_INVALID, "grid must be at least 2x2");
     P->c = c;
     P->op = *op;
+    P->w5 = kl_stencil5_t{0.0, 0.0, 0.0, 0.0, 0.0};
     if (pc) P->pc = *pc;
     else P->pc = kl_precond_t{KL_PC_NONE, 0, nullptr, nullptr};
     if (P->op.kind != KL_OP_POISSON5 && P->op.kind != KL_OP_POISSON5_BRANCHY && P->op.kind != KL_OP_ANISO5 &&
-        P->op.kind != KL_OP_USER && P->op.kind != KL_OP_DENSE && P->op.kind != KL_OP_ANISO5_VAR)
+        P->op.kind != KL_OP_USER && P->op.kind != KL_OP_DENSE && P->op.kind != KL_OP_ANISO5_VAR &&
+        P->op.kind != KL_OP_STENCIL5)
         return c->fail(KL_ERR_INVALID, "unknown operator kind");
+    if (P->op.kind == KL_OP_STENCIL5) {
+        const kl_stencil5_t *w = (const kl_stencil5_t *)op->user;
+        if (!w) return c->fail(KL_ERR_INVALID, "KL_OP_STENCIL5 without weights");
+        if (!(std::isfinite(w->c) && std::isfinite(w->wl) && std::isfinite(w->wr) && std::isfinite(w->wd) &&
+              std::isfinite(w->wu)))
+            return c->fail(KL_ERR_INVALID, "KL_OP_STENCIL5: the weights must be finite");
+        if (c->nranks > 1) return c->fail(KL_ERR_UNSUPPORTED, "KL_OP_STENCIL5 is single-GPU in this release");
+        P->w5 = *w;
+        P->op.user = &P->w5;     // the kernels' coefficients (op_coef) come from this copy
+        if ((P->pc.kind == KL_PC_CBPR2 || P->pc.kind == KL_PC_CHEB) && (w->wl * w->wr < 0.0 || w->wd * w->wu < 0.0))
+            return c->fail(KL_ERR_UNSUPPORTED, "KL_OP_STENCIL5 with a complex spectrum (wl*wr < 0 or wd*wu < 0): "
+                                               "the Chebyshev preconditioners need a real interval");
+    }
     if (P->op.kind == KL_OP_ANISO5_VAR) {
         const kl_aniso_var_t *cf = (const kl_aniso_var_t *)P->op.user;
         if (!cf || !cf->kx || !cf->ky) return c->fail(KL_ERR_INVALID, "KL_OP_ANISO5_VAR without coefficient arrays");
@@ -563,6 +578,25 @@ int fetch_history(Ctx *c) {
 using namespace kl;
 
 extern "C" {
+
+// The operator is the Kronecker sum of two tridiagonal Toeplitz matrices, tridiag(-wl, c/2, -wr) (x) I + I (x)
+// tridiag(-wu, c/2, -wd).  With wl*wr >= 0 and wd*wu >= 0 each factor is diagonally similar to a symmetric one, with
+// eigenvalues c/2 - 2 sqrt(wl*wr) cos(k pi/(nx+1)), k = 1..nx (and the same in y); the extremes are k = 1 and k = nx.
+int kl_stencil5_spectrum(const kl_stencil5_t *w, int nx, int ny, double *lam_min, double *lam_max) {
+    if (!w || !lam_min || !lam_max) return KL_ERR_INVALID;
+    *lam_min = *lam_max = NAN;
+    if (nx < 1 || ny < 1) return KL_ERR_INVALID;
+    if (!(std::isfinite(w->c) && std::isfinite(w->wl) && std::isfinite(w->wr) && std::isfinite(w->wd) &&
+          std::isfinite(w->wu)))
+        return KL_ERR_INVALID;
+    const double gx = w->wl * w->wr, gy = w->wd * w->wu;
+    if (gx < 0.0 || gy < 0.0) return KL_ERR_UNSUPPORTED;
+    const double pi = 3.14159265358979323846;
+    const double ax = 2.0 * std::sqrt(gx) * std::cos(pi / (nx + 1)), ay = 2.0 * std::sqrt(gy) * std::cos(pi / (ny + 1));
+    *lam_min = (w->c - ax) - ay;
+    *lam_max = (w->c + ax) + ay;
+    return KL_OK;
+}
 
 int kl_apply_operator(kl_handle_t h, const kl_operator_t *A_x, const double *x, double *y, int nx, int ny) {
     if (!h || !A_x || !x || !y) return KL_ERR_INVALID;

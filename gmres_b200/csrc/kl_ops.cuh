@@ -14,9 +14,15 @@ struct Prob {
     int nx, ny;        // global grid
     int nyl, j0;       // this rank's slab
     size_t n;          // nx * nyl
+    // KL_OP_STENCIL5: the caller's weights, copied at the start of the call (op.user points here); all zero for the
+    // other kinds.  Part of every CUDA-graph key.
+    kl_stencil5_t w5;
     bool builtin_op() const {   // the stencil operators (fused kernels); user callbacks and dense matrices take the generic path
-        return op.kind == KL_OP_POISSON5 || op.kind == KL_OP_POISSON5_BRANCHY || op.kind == KL_OP_ANISO5;
+        return op.kind == KL_OP_POISSON5 || op.kind == KL_OP_POISSON5_BRANCHY || op.kind == KL_OP_ANISO5 ||
+               op.kind == KL_OP_STENCIL5;
     }
+    // false only for a KL_OP_STENCIL5 that is not symmetric (CG, PCG and Lanczos refuse it)
+    bool symmetric() const { return op.kind != KL_OP_STENCIL5 || (w5.wl == w5.wr && w5.wd == w5.wu); }
 };
 
 int prob_init(Prob *P, Ctx *c, const kl_operator_t *op, const kl_precond_t *pc, const double *params,
@@ -37,7 +43,8 @@ inline bool chain_ok(const Prob *P, int L) {
     const Ctx *c = P->c;
     if (!(c->opt_tma && c->opt_fuse && c->opt_chain) || P->nx % 2 != 0 || P->nx < 64) return false;
     // stv_poisson (the reference's branchy variant, unused by its drivers) runs one pass per application: the
-    // temporally blocked kernels are only instantiated for stvec and the anisotropic operator
+    // temporally blocked kernels are only instantiated for stvec and the constant-coefficient operators
+    // (KL_OP_ANISO5, and KL_OP_STENCIL5 on one GPU)
     if (P->op.kind == KL_OP_POISSON5_BRANCHY) return false;
     if (c->nranks == 1) return true;
     return P->ny / c->nranks >= L && (size_t)L * P->nx <= 65536;   // L-line halo fits the exchange buffers

@@ -66,6 +66,12 @@ enum {
                                     set up by kl_gmres_mgsr_dense / kl_gmres_hh_dense (single GPU only)   */
     KL_OP_ANISO5_VAR = 4,        /* variable-coefficient anisotropic diffusion, self-adjoint finite-volume form
                                     (README.md:46 WIP, new): `user` points to a kl_aniso_var_t (single GPU only) */
+    KL_OP_STENCIL5 = 5,          /* general constant-coefficient 5-point operator, e.g. convection-diffusion (new):
+                                    `user` points to a HOST kl_stencil5_t, read at the start of each call (single GPU
+                                    only).  Nonsymmetric unless wl == wr and wd == wu: CG, PCG and kl_lanczos refuse it
+                                    then (KL_ERR_UNSUPPORTED), and KL_PC_CBPR2 / KL_PC_CHEB refuse it when its spectrum
+                                    is complex (wl*wr < 0 or wd*wu < 0).  It runs through the same fused and temporally
+                                    blocked kernels as KL_OP_ANISO5.                                                 */
     KL_OP_USER = 100             /* user callback on device pointers (single GPU only) */
 };
 /* coefficient fields of KL_OP_ANISO5_VAR: cell values kx(i,j), ky(i,j), idx = i + j*nx, DEVICE pointers (kl_vec_alloc /
@@ -73,6 +79,24 @@ enum {
 typedef struct {
     const double *kx, *ky;
 } kl_aniso_var_t;
+/* weights of KL_OP_STENCIL5, finite numbers (idx = i + j*nx, "d" = idx+nx is line j+1, "u" = idx-nx is line j-1, the
+ * reference's naming in poisson.f90:42):
+ *   y(i,j) = c x(idx) - ( wl x(idx-1) + wr x(idx+1) + wd x(idx+nx) + wu x(idx-nx) ),   missing neighbours = 0
+ * evaluation order (every kernel, and the same as KL_OP_ANISO5_VAR's):
+ *   s = fma(wl, xl, wr*xr) ; t = fma(wd, xd, wu*xu) ; y = fma(c, xc, -(s + t))
+ * so c = ((a+a)+b)+b, wl = wr = a, wd = wu = b gives KL_OP_ANISO5_VAR on constant fields kx = a, ky = b bit for bit.
+ * Convection-diffusion -lap(u) + (bx, by).grad(u) on a grid of spacing h, scaled by h^2, with the cell Peclet numbers
+ * px = bx*h/2, py = by*h/2: central differences c = 4, wl = 1+px, wr = 1-px, wu = 1+py, wd = 1-py (real spectrum iff
+ * |px|, |py| <= 1); first-order upwind (px, py >= 0) c = 4+2px+2py, wl = 1+2px, wr = 1, wu = 1+2py, wd = 1.           */
+typedef struct {
+    double c, wl, wr, wd, wu;
+} kl_stencil5_t;
+/* Exact extremes of the Dirichlet spectrum of KL_OP_STENCIL5 on an nx x ny grid (host arithmetic, no handle).  When
+ * wl*wr >= 0 and wd*wu >= 0 the operator is similar to a symmetric one by a diagonal scaling and its spectrum is real:
+ *   lambda = c -+ 2 sqrt(wl*wr) cos(pi/(nx+1)) -+ 2 sqrt(wd*wu) cos(pi/(ny+1))
+ * (KL_OK).  Otherwise the spectrum is complex: KL_ERR_UNSUPPORTED and both outputs NaN.  Pass [lam_min, lam_max] to
+ * KL_PC_CHEB as its interval.                                                                                         */
+int kl_stencil5_spectrum(const kl_stencil5_t *w, int nx, int ny, double *lam_min, double *lam_max);
 typedef struct {
     int kind;
     double eps_x, eps_y;  /* KL_OP_ANISO5 */

@@ -23,6 +23,7 @@
 #include <cmath>
 #include <stdexcept>
 #include <string>
+#include <utility>
 #include <vector>
 
 #include "krylov_b200.h"
@@ -37,6 +38,25 @@ struct Error : std::runtime_error {
 inline const kl_operator_t stvec{KL_OP_POISSON5, 1.0, 1.0, nullptr, nullptr};
 inline const kl_operator_t stv_poisson{KL_OP_POISSON5_BRANCHY, 1.0, 1.0, nullptr, nullptr};
 inline kl_operator_t aniso(double ex, double ey) { return kl_operator_t{KL_OP_ANISO5, ex, ey, nullptr, nullptr}; }
+// general constant-coefficient 5-point operator (KL_OP_STENCIL5, krylov_b200.h kl_stencil5_t).  It converts to the
+// kl_operator_t every entry takes; that descriptor points at this object's weights, so the object must outlive the
+// calls it is passed to.
+struct stencil5 {
+    kl_stencil5_t w;
+    kl_operator_t op;
+    stencil5(double c, double wl, double wr, double wd, double wu)
+        : w{c, wl, wr, wd, wu}, op{KL_OP_STENCIL5, 1.0, 1.0, nullptr, &w} {}
+    stencil5(const stencil5 &o) : stencil5(o.w.c, o.w.wl, o.w.wr, o.w.wd, o.w.wu) {}
+    stencil5 &operator=(const stencil5 &o) { w = o.w; return *this; }
+    operator const kl_operator_t &() const { return op; }
+    // exact extremes of the spectrum on an nx x ny grid (kl_stencil5_spectrum); throws if it is complex
+    std::pair<double, double> spectrum(int nx, int ny) const {
+        double lo, hi;
+        const int rc = kl_stencil5_spectrum(&w, nx, ny, &lo, &hi);
+        if (rc != KL_OK) throw Error(rc, "kl_stencil5_spectrum: complex spectrum (wl*wr < 0 or wd*wu < 0) or bad arguments");
+        return {lo, hi};
+    }
+};
 inline const kl_precond_t cbpr2{KL_PC_CBPR2, 0, nullptr, nullptr};
 inline const kl_precond_t no_precond{KL_PC_NONE, 0, nullptr, nullptr};
 inline kl_precond_t cheb(int degree) { return kl_precond_t{KL_PC_CHEB, degree, nullptr, nullptr}; }
