@@ -154,7 +154,9 @@ enum {
     KL_OPT_MAX_RESTARTS = 2,  /* default 1000 = max_restarts (gmres_mgsr.f90:6) / stages (gmres_hh.f90:8) */
     KL_OPT_VERR = 3,          /* 1 (default): compute the v_err epilogue; 0: skip it */
     KL_OPT_CHECK_EVERY = 4,   /* CG/BiCGSTAB: iterations enqueued between host polls (default 32) */
-    KL_OPT_USE_GRAPH = 5,     /* reserved (CUDA-graph replay of an iteration batch); currently a no-op */
+    KL_OPT_USE_GRAPH = 5,     /* 1 (default): CG / PCG iteration batches and GMRES-MGSR / Householder GMRES restart cycles
+                                 are captured once and replayed as CUDA graphs (cached per handle; fused kernels, no or
+                                 a built-in preconditioner, KL_OPT_PROFILE off); 0: eager launches, same results */
     KL_OPT_HH_MODE = 6,       /* Householder application, see below                  */
     KL_OPT_FUSE = 7,          /* 1 (default): fused kernels; 0: one kernel per reference loop */
     KL_OPT_PROFILE = 8,       /* 1: CUDA-event pairs around every hot kernel (kl_get_profile)  */
