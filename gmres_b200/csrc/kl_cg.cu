@@ -4,7 +4,9 @@
 // All four share one device implementation (the serial and OpenMP variants
 // compute the same quantities; only their summation order differs).
 //
-// Plain CG, one GPU, from 2^24 unknowns on (default): 36n B per iteration, PAIRS of temporally blocked passes
+// Plain CG, one GPU, from 2^27 unknowns on (default): 24n B per iteration, GROUPS of four temporally blocked passes
+//   (16n + 16n + 16n + 48n, ChCgLook<J, STORE> below; r, p and x are stored every fourth iteration only).
+// Plain CG, one GPU, 2^24 .. 2^27 unknowns (default): 36n B per iteration, PAIRS of temporally blocked passes
 //   (24n + 48n, ChCgPass<kCgPairA / kCgPairB> below; p and x are stored every second iteration only).
 // Plain CG, one GPU, 2^20 .. 2^24 unknowns (default): 48n B per iteration, ONE temporally blocked pass (ChCg below).
 // Plain CG otherwise: 64n B per iteration, see FCgDirX2 / FCgRUpdate below (A applied twice, A p never stored).
@@ -158,7 +160,7 @@ struct FCgRUpdate : StencilBase<2, 1> {
 //     as the two fmas of two one-pass iterations              reads r_{k+1}, p_k, x_k   writes r_{k+2}, p_{k+2}, x_{k+2}
 // 24n + 48n B per pair.  Every stored value and every sum is the one-pass path's fma chain on the same operands,
 // and NIN, L (hence the CTA grid and the block-partial reduction order) are ChCg's: the results are bit-identical.
-// Pass B takes alpha_k, beta_k from S_ALPHA_PREV / S_BETA_PREV (cg_onepass_scalars).
+// Pass B takes alpha_k, beta_k from S_ALPHA_HIST / S_BETA_HIST (cg_onepass_scalars).
 enum CgPass { kCgOne, kCgPairA, kCgPairB };
 template <int MODE>
 struct ChCgPass : ChainBase<2, 2, 1, 4> {
@@ -171,8 +173,8 @@ struct ChCgPass : ChainBase<2, 2, 1, 4> {
         alpha = S[S_ALPHA];
         beta = S[S_BETA];
         if (MODE == kCgPairB) {
-            alpha0 = S[S_ALPHA_PREV];
-            beta0 = S[S_BETA_PREV];
+            alpha0 = S[S_ALPHA_HIST];
+            beta0 = S[S_BETA_HIST];
         }
     }
     __device__ __forceinline__ void level0(bool, size_t, const double (&raw)[2][2], double (&u)[2],
@@ -231,6 +233,134 @@ struct ChCgPass : ChainBase<2, 2, 1, 4> {
     }
 };
 using ChCg = ChCgPass<kCgOne>;
+
+// ---- plain CG in GROUPS of G passes (16n (G-1) + 48n B per G iterations, KL_OPT_CG_ONEPASS = 3) ------------------
+// Recompute instead of store.  A group starts from r_k, p_k, x_k in HBM; its pass j = 1..G replays the j iterations
+// k .. k+j-1 from them (J = j) and finds alpha_{k+j} and the predicted beta_{k+j} as the one-pass path does:
+//   level 0:         u = p_k
+//   level l = 1..J:  A p_{k+l-1} ; r_{k+l} = r_{k+l-1} - alpha_{k+l-1} A p_{k+l-1} ; p_{k+l} = r_{k+l} + beta_{k+l-1} p_{k+l-1}
+//                    (r_k from the ring at level 1, then carried point-wise from level to level)
+//                    STORE: x_{k+l} = x_k + alpha_k p_k + .. + alpha_{k+l-1} p_{k+l-1} (x_k from the ring at level 1,
+//                    then carried), stored with r_{k+J} and p_{k+J} at level J
+//   level J + 1:     A p_{k+J} ; rho, gamma, sigma, delta as ChCg's last level
+// Passes 1..G-1 store nothing (reads r_k, p_k: 16n B); pass G stores (reads r_k, p_k, x_k, writes r, p, x: 48n B).
+// Every point-wise value is the one-pass path's fma on the same operands.  The CTA grid is that of J + 1 levels, so
+// the block-partial sums, hence alpha and beta, differ from the one-pass path's at rounding level.
+// back = 0: the pass follows iteration k + J - 1, so alpha_{k+J-1} is S_ALPHA and the older ones are in the history;
+// back = 1: the store pass that finishes a group after convergence at its pass J (one more iteration recorded).
+template <int J, bool STORE>
+struct ChCgLook : ChainBase<STORE ? 3 : 2, J + 1, STORE ? 2 : 1, 4> {
+    static_assert(J >= 1 && J <= kCgHist + 1, "group depth");
+    static constexpr bool SINGLE_GPU = true;
+    // from three levels on: 2-line stages (a 12-line ring).  With 1-line stages the L retained lines leave only
+    // 6 - L lines of lookahead, too few to cover the DRAM latency (measured at 16384^2 with G = 4: the 4-level store
+    // pass took 2407 us against 2089 us for the 5-level one, which had 2-line stages)
+    static constexpr int SR = J + 1 >= 3 ? 2 : 1;
+    // store passes from four levels on: three 12-line inputs take 60-70 KB of ring, so at most 3 CTAs fit an SM
+    // anyway; their register budget (168) then holds the four levels without spills (128 spilled 28-84 B)
+    static constexpr int MINB = (STORE && J + 1 >= 4) ? 3 : ChainBase<STORE ? 3 : 2, J + 1, STORE ? 2 : 1, 4>::MINB;
+    static constexpr int NC = STORE ? 2 : 1;
+    double *r_new, *p_new, *x_new;
+    const double *S;
+    int back;
+    double al[J], be[J];      // alpha_{k+l}, beta_{k+l}, l = 0..J-1
+    __device__ __forceinline__ void init() {
+#pragma unroll
+        for (int l = 0; l < J; ++l) {
+            const int d = J - 1 - l + back;     // iterations before the current one
+            al[l] = d == 0 ? S[S_ALPHA] : S[S_ALPHA_HIST + d - 1];
+            be[l] = d == 0 ? S[S_BETA] : S[S_BETA_HIST + d - 1];
+        }
+    }
+    __device__ __forceinline__ void level0(bool, size_t, const double (&raw)[STORE ? 3 : 2][2], double (&u)[2],
+                                           double (&cc)[NC][2], double *) const {
+#pragma unroll
+        for (int e = 0; e < 2; ++e) {
+            u[e] = raw[1][e];                                                            // p_k
+#pragma unroll
+            for (int k = 0; k < NC; ++k) cc[k][e] = 0.0;
+        }
+    }
+    template <class RAW>
+    __device__ __forceinline__ void level(int lv, bool out, size_t idx, const double (&up)[2], const double (&au)[2],
+                                          const double (&cin)[NC][2], RAW raw, const double (&)[1][2], double (&u)[2],
+                                          double (&cout)[NC][2], double *acc) const {
+        if (lv <= J) {
+            double rk[2], xk[2];
+            if (lv == 1) {
+                const double2 rv = raw(0);
+                rk[0] = rv.x; rk[1] = rv.y;
+                if (STORE) {
+                    const double2 xv = raw(STORE ? 2 : 0);
+                    xk[0] = xv.x; xk[1] = xv.y;
+                }
+            } else {
+                rk[0] = cin[0][0]; rk[1] = cin[0][1];
+                xk[0] = cin[NC - 1][0]; xk[1] = cin[NC - 1][1];
+            }
+#pragma unroll
+            for (int e = 0; e < 2; ++e) {
+                cout[0][e] = fma(-al[lv - 1], au[e], rk[e]);                             // cg.f90:130
+                u[e] = fma(be[lv - 1], up[e], cout[0][e]);                               // direction update
+                if (STORE) cout[NC - 1][e] = fma(al[lv - 1], up[e], xk[e]);              // cg.f90:128
+            }
+            if (STORE && lv == J && out) {
+                stg2(r_new + idx, cout[0][0], cout[0][1]);
+                stg2(p_new + idx, u[0], u[1]);
+                stg2(x_new + idx, cout[NC - 1][0], cout[NC - 1][1]);
+            }
+        } else {
+            u[0] = u[1] = 0.0;
+#pragma unroll
+            for (int k = 0; k < NC; ++k) cout[k][0] = cout[k][1] = 0.0;
+            if (out) {
+#pragma unroll
+                for (int e = 0; e < 2; ++e) {
+                    acc[0] = fma(cin[0][e], cin[0][e], acc[0]);                          // rho   = r'.r'
+                    acc[1] = fma(au[e], up[e], acc[1]);                                  // gamma = p'.Ap'
+                    acc[2] = fma(au[e], cin[0][e], acc[2]);                              // sigma = r'.Ap'
+                    acc[3] = fma(au[e], au[e], acc[3]);                                  // delta = Ap'.Ap'
+                }
+            }
+        }
+    }
+};
+constexpr int kCgGroupMax = kCgHist + 1;
+
+// Pass j of a group (store: also r, p, x), or the finishing store pass (back = 1, ungated, no post).  The names are
+// the profile's (KL_OPT_PROFILE): classes 0..2 store nothing, 3..6 store at depth 1..4, 7 finishes a group.
+static const char *const kCgLookName[2][kCgGroupMax] = {
+    {"cg_group_look1 (chain, 2 levels: replay 1 iteration from r_k, p_k; A p; 4 dots; stores nothing)",
+     "cg_group_look2 (chain, 3 levels: replay 2 iterations from r_k, p_k; A p; 4 dots; stores nothing)",
+     "cg_group_look3 (chain, 4 levels: replay 3 iterations from r_k, p_k; A p; 4 dots; stores nothing)",
+     nullptr},
+    {"cg_group_store1 (chain, 2 levels: replay 1 iteration from r_k, p_k, x_k; store r, p, x; A p; 4 dots)",
+     "cg_group_store2 (chain, 3 levels: replay 2 iterations from r_k, p_k, x_k; store r, p, x; A p; 4 dots)",
+     "cg_group_store3 (chain, 4 levels: replay 3 iterations from r_k, p_k, x_k; store r, p, x; A p; 4 dots)",
+     "cg_group_store4 (chain, 5 levels: replay 4 iterations from r_k, p_k, x_k; store r, p, x; A p; 4 dots)"}};
+static const char kCgFinishName[] = "cg_group_finish (chain: x after convergence inside a group)";
+
+template <int J, bool STORE>
+static int cg_look_launch(Ctx *c, Prob *P, const double *r, const double *p, const double *x, double *r_new,
+                          double *p_new, double *x_new, int back, bool gated) {
+    Halo H{};
+    const double *vecs[3] = {r, p, x};
+    ChCgLook<J, STORE> f;
+    set_io(f, P, vecs, H);
+    set_gate(f, c, gated);
+    f.r_new = r_new; f.p_new = p_new; f.x_new = x_new; f.S = c->d_S; f.back = back;
+    if (back) return launch_chain(c, &P->op, f, P->nx, P->nyl, NoPost{});
+    return launch_chain(c, &P->op, f, P->nx, P->nyl, PostCgOnePass{c->d_S, c->d_I, c->d_hist, c->hist_cap});
+}
+static int cg_look(Ctx *c, Prob *P, int J, bool store, const double *r, const double *p, const double *x,
+                   double *r_new, double *p_new, double *x_new, int back, bool gated) {
+#define KL_LOOK(JJ, ST) \
+    if (J == JJ && store == ST) return cg_look_launch<JJ, ST>(c, P, r, p, x, r_new, p_new, x_new, back, gated);
+    KL_LOOK(1, false) KL_LOOK(2, false) KL_LOOK(3, false)
+    KL_LOOK(1, true) KL_LOOK(2, true) KL_LOOK(3, true) KL_LOOK(4, true)
+#undef KL_LOOK
+    return c->fail(KL_ERR_INVALID, "cg_look: group depth");
+}
 
 // Prologue of the one-pass path: the four sums of ChCg's last level for p_0 = r_0 (= b), no store.
 struct FCgOnePassInit : StencilBase<1, 4> {
@@ -309,6 +439,8 @@ constexpr size_t kCgOnePassMin = (size_t)1 << 20;
 // ... and pairs of passes (36n B per iteration) from this many on (scripts/cg_pair_sweep.py,
 // profiles/r04_cg_pair_sweep.json).
 constexpr size_t kCgPairMin = (size_t)1 << 24;
+// ... and groups of passes from this many on (scripts/cg_group_sweep.py, profiles/r08_cg_group_sweep.json)
+constexpr size_t kCgGroupMin = (size_t)1 << 27;
 
 static int cg_solve(Ctx *c, const kl_operator_t *A, const double *b, double *x, int nx, int ny,
                     double tol, int *iter, double *res_out, const kl_precond_t *M, const double *params,
@@ -335,10 +467,13 @@ static int cg_solve(Ctx *c, const kl_operator_t *A, const double *b, double *x, 
     const bool twice = defer_x && !prec && c->opt_chain;       // plain CG: apply A twice, never store A p (64n B)
     // plain CG in one chain pass per iteration (48n B) or in pairs of passes (36n B): single GPU (the chain needs a
     // two-line halo, which the multi-GPU producer-push protocol does not deliver)
-    const int cg_pass = !(twice && c->nranks == 1 && chain_ok(&P, 2)) ? 0
-                        : c->opt_cg_onepass >= 0 ? c->opt_cg_onepass
-                        : (n >= kCgPairMin ? 2 : (n >= kCgOnePassMin ? 1 : 0));
-    const bool onepass = cg_pass == 1, pair = cg_pass == 2;
+    // groups of G passes need G + 1 levels
+    const int G = c->opt_cg_group;
+    int cg_pass = !(twice && c->nranks == 1 && chain_ok(&P, 2)) ? 0
+                  : c->opt_cg_onepass >= 0 ? c->opt_cg_onepass
+                  : (n >= kCgGroupMin ? 3 : (n >= kCgPairMin ? 2 : (n >= kCgOnePassMin ? 1 : 0)));
+    if (cg_pass == 3 && !chain_ok(&P, G + 1)) cg_pass = 2;
+    const bool onepass = cg_pass == 1, pair = cg_pass == 2, group = cg_pass == 3;
     const int nvec = 4 + (dev ? 0 : 1) + (prec ? 3 : 0) + ((fuse_pc || twice) ? 1 : 0) + (twice ? 1 : 0);
     KL_TRY(ws_reserve(c, nvec * ws_need(n)));
     ws_reset(c);
@@ -350,8 +485,11 @@ static int cg_solve(Ctx *c, const kl_operator_t *A, const double *b, double *x, 
     double *x_cur = dx, *x_alt = twice ? ws_take<double>(c, n) : nullptr;
     // one-pass: x is ping-ponged from the first iteration on; start it where an odd / even maxit ends in dx
     // pairs: x moves once per pair; start it where maxit / 2 pairs end in dx (an odd maxit ends in a flush to dx)
-    if ((onepass && (maxit & 1)) || (pair && ((maxit / 2) & 1))) std::swap(x_cur, x_alt);
+    // groups: x moves once per group; start it where the ceil(maxit / G) store passes end in dx
+    if ((onepass && (maxit & 1)) || (pair && ((maxit / 2) & 1)) || (group && (((maxit + G - 1) / G) & 1)))
+        std::swap(x_cur, x_alt);
     double *const x_start = x_cur, *const x_other = x_alt;
+    double *const r_start = r, *const r_other = r_alt;
     const Cbpr2Coef cf = fuse_pc ? cbpr2_coef(P.params) : Cbpr2Coef{1.0, 0.0};
     if (prec) {
         z = ws_take<double>(c, n);
@@ -381,8 +519,9 @@ static int cg_solve(Ctx *c, const kl_operator_t *A, const double *b, double *x, 
         KL_TRY(stage_in(c, r, b, n));
         KL_CUDA(c, cudaMemsetAsync(x_cur, 0, n * sizeof(double), c->stream));
     }
-    // pairs: p_0 = r_0 gets a buffer of its own, as pass B of the first pair overwrites r_0's with r_2
-    if (pair) KL_CUDA(c, cudaMemcpyAsync(p0, r, n * sizeof(double), cudaMemcpyDeviceToDevice, c->stream));
+    // pairs: p_0 = r_0 gets a buffer of its own, as pass B of the first pair overwrites r_0's with r_2 (groups: so
+    // that r and p ping-pong alike from the first group on)
+    if (pair || group) KL_CUDA(c, cudaMemcpyAsync(p0, r, n * sizeof(double), cudaMemcpyDeviceToDevice, c->stream));
     else KL_CUDA(c, cudaMemsetAsync(p0, 0, n * sizeof(double), c->stream));
     KL_CUDA(c, cudaMemsetAsync(c->d_I, 0, sizeof(int) * I_COUNT, c->stream));
     {
@@ -405,7 +544,7 @@ static int cg_solve(Ctx *c, const kl_operator_t *A, const double *b, double *x, 
     // one-pass: rr, p.Ap, r.Ap and Ap.Ap for p_0 = r_0, then alpha_0 and the predicted beta_0
     if (prec) {
         KL_TRY(pc_apply(&P, r, z, aux, aux2, 2, false, PostStoreRed{c->d_S, S_RR, 0}));
-    } else if (onepass || pair) {
+    } else if (onepass || pair || group) {
         Halo H{};
         const double *vecs[1] = {r};
         FCgOnePassInit d;
@@ -429,6 +568,21 @@ static int cg_solve(Ctx *c, const kl_operator_t *A, const double *b, double *x, 
     auto enqueue_iterations = [&](const int done0, const int batch) -> int {
         const int done = done0;
         for (int k = 0; k < batch; ++k) {
+            if (group) {
+                // pass j of its group replays j iterations from the group's r_k, p_k (x_k); the last pass of a group,
+                // and of a group truncated by maxit, stores r, p and x, which then move to the other buffers
+                const int it = done + k, j = it % G + 1;
+                const bool store = j == G || it + 1 == maxit;
+                ProfScope ps(c, store ? 2 + j : j - 1, kCgLookName[store][j - 1], (store ? 48.0 : 16.0) * n);
+                KL_TRY(cg_look(c, &P, j, store, r, pold, x_cur, r_alt, pnew, x_alt, 0, true));
+                if (store) {
+                    std::swap(r, r_alt);
+                    std::swap(x_cur, x_alt);
+                    std::swap(pold, pnew);
+                }
+                z = r;
+                continue;
+            }
             if (pair && ((done + k) & 1) == 0) {
                 // pass A: p_0 is in p0 from the prologue on, p alternates between p1 (written by the first pair) and p0
                 ProfScope ps(c, 0, "cg_pair_a (chain: r-=alpha*A p; p=r+beta*p; A p; 4 dots)", 24.0 * n);
@@ -600,13 +754,18 @@ static int cg_solve(Ctx *c, const kl_operator_t *A, const double *b, double *x, 
         int batch = c->opt_check_every;
         if (batch > maxit - done) batch = maxit - done;
         Ctx::GraphEntry *ge = nullptr;
-        if (use_graph && batch % 2 == 0 && done % 2 == 0) {
+        // groups: the buffer roles alternate once per group, so a replayable batch (whose replay does not run the
+        // host-side swaps of enqueue_iterations) is an even number of whole groups from phase 0 on.  Batches starting
+        // mid-group run eagerly.
+        const int period = group ? G : 2;
+        if (use_graph && batch % (group ? 2 * G : 2) == 0 && done % period == 0) {
             GraphKey gk;
             gk.add('C').add(nx).add(ny).add(batch).add(P.op.kind).add(P.op.eps_x).add(P.op.eps_y).add(P.w5).add(P.pc.kind)
                 .add(P.pc.degree).add(P.params).add(c->opt_tma).add(c->opt_chain).add(c->opt_stencil_rows)
                 .add(c->opt_stencil_tail).add(c->opt_stencil_stagger).add(c->opt_pdl).add(c->opt_reverse).add(c->opt_persistent)
                 .add(c->ws).add(dx).add(r).add(pold)
-                .add(x_cur).add(cg_pass).add(onepass && done == 0);     // (one-pass: iteration 1 reads r as p)
+                .add(x_cur).add(cg_pass).add(onepass && done == 0)      // (one-pass: iteration 1 reads r as p)
+                .add(group ? G : 0).add(done % period);
             ge = graph_find(c, gk.s);
             if (!ge && polls >= 1) {     // the first batch of a handle's first solve runs eagerly
                 const long long l0 = c->stats.kernel_launches;
@@ -636,18 +795,35 @@ static int cg_solve(Ctx *c, const kl_operator_t *A, const double *b, double *x, 
             break;
         }
     }
-    if (pair) {
+    if (group) {
+        // after `its` passes (the passes after the convergence step were gated off), m = its / G groups stored x_{mG}
+        // in x_start (m even) or the other buffer (m odd).  A group truncated by maxit stored x_{its} into dx.  If its
+        // pass j < G raised the flag, one ungated store pass of depth j from the group's r_k, p_k, x_k forms x_{its}.
+        if (status == KL_NOT_CONVERGED) KL_TRY(read_back(c));     // (maxit = 0: no poll ran)
+        const int its_done = c->h_pinned_i[I_ITER], m = its_done / G, j = its_done % G;
+        const double *xres = (m & 1) ? x_other : x_start;
+        if (j != 0 && its_done == maxit) {
+            xres = (m & 1) ? x_start : x_other;
+        } else if (j != 0) {
+            ProfScope ps(c, 7, kCgFinishName, 48.0 * n);
+            double *xo = (m & 1) ? x_start : x_other;
+            KL_TRY(cg_look(c, &P, j, true, (m & 1) ? r_other : r_start, (m & 1) ? p1 : p0, xres,
+                           (m & 1) ? r_start : r_other, (m & 1) ? p0 : p1, xo, 1, false));
+            xres = xo;
+        }
+        if (xres != dx) KL_CUDA(c, cudaMemcpyAsync(dx, xres, n * sizeof(double), cudaMemcpyDeviceToDevice, c->stream));
+    } else if (pair) {
         // after `its` passes (the passes after the convergence step were gated off) x_{2m}, m = its / 2, is in
         // x_start (m even) or the other buffer (m odd), and p_{2m} in p0 (m even) or p1 (m odd).  An odd `its` ended
         // on a pass A: x_{its} = x_{2m} + alpha_{2m} p_{2m}, the one-pass path's fma, with alpha_{2m} in
-        // S_ALPHA_PREV.
+        // S_ALPHA_HIST.
         if (status == KL_NOT_CONVERGED) KL_TRY(read_back(c));     // (maxit = 0: no poll ran)
         const int its_done = c->h_pinned_i[I_ITER], m = its_done / 2;
         const double *xres = (m & 1) ? x_other : x_start;
         if (its_done & 1) {
             PAxpy u;
             set_gate(u, c, false);
-            u.a = xres; u.b = (m & 1) ? p1 : p0; u.y = dx; u.S = c->d_S; u.s_idx = S_ALPHA_PREV; u.sign = 1.0;
+            u.a = xres; u.b = (m & 1) ? p1 : p0; u.y = dx; u.S = c->d_S; u.s_idx = S_ALPHA_HIST; u.sign = 1.0;
             KL_TRY(launch_pointwise(c, u, n, NoPost{}));
         } else if (xres != dx) {
             KL_CUDA(c, cudaMemcpyAsync(dx, xres, n * sizeof(double), cudaMemcpyDeviceToDevice, c->stream));
@@ -690,7 +866,13 @@ static int cg_solve(Ctx *c, const kl_operator_t *A, const double *b, double *x, 
     c->stats.cycles = polls;
     c->stats.solve_ms = ms;
     c->stats.total_ms = ms_tot;
-    c->stats.algorithmic_bytes = pair ? (24.0 * ((its + 1) / 2) + 48.0 * (its / 2) + 24.0 * (its & 1)) * (double)n
+    // groups: 16n B per pass that stores nothing, 48n B per store pass; a group cut short by maxit ends on a store
+    // pass, one cut short by convergence on a pass that stores nothing and the finishing store pass
+    const int gt = group ? its % G : 0;
+    c->stats.algorithmic_bytes =
+        group ? (double)(its / G) * (16.0 * (G - 1) + 48.0) * (double)n +
+                    (gt == 0 ? 0.0 : (16.0 * (its == maxit ? gt - 1 : gt) + 48.0) * (double)n)
+        : pair ? (24.0 * ((its + 1) / 2) + 48.0 * (its / 2) + 24.0 * (its & 1)) * (double)n
                                       : (double)its * (fuse_pc ? 80.0 : (prec ? 96.0 : (onepass ? 48.0 : (twice ? 64.0 : (defer_x ? 72.0 : 80.0))))) * (double)n;
     *res_out = c->h_pinned[S_RES];
     if (status == KL_OK) *iter = c->h_pinned_i[I_CONV_AT];   // count on exit; unchanged if not converged

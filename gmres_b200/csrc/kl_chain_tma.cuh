@@ -105,6 +105,8 @@ struct ChainBase {
     // VAROP: the chain applies KL_OP_ANISO5_VAR with in[1] = kx, in[2] = ky (see "Variable coefficients" above
     // k_chain_tma); the functor's level0 / level then also receive the diagonal of A
     static constexpr bool VAROP = false;
+    // SINGLE_GPU: no multi-GPU instantiation (a functor whose solver path runs on one GPU only)
+    static constexpr bool SINGLE_GPU = false;
     // LAG: how many lines level l runs behind level l-1.  With LAG = 1 level l consumes the line level l-1
     // produced in the SAME march step, so a step is one dependent chain of 7L FP64 operations (~250 cycles of
     // latency at L = 4 with 4 warps per scheduler to hide it: the round-1 kernel ran the FP64 pipe at 44 %).
@@ -585,7 +587,9 @@ inline int launch_chain(Ctx *c, const kl_operator_t *op, C f, int nx, int ny, co
         k_chain_tma<C, OPK, MG><<<grid, kChainThreads, smem, c->stream>>>(f, g, rc, tm);               \
     }
 #define KL_CH_LAUNCH(OPK)                                                                              \
-    if (f.lo[0] || f.hi[0]) KL_CH_LAUNCH1(OPK, true) else KL_CH_LAUNCH1(OPK, false)
+    if constexpr (C::SINGLE_GPU) KL_CH_LAUNCH1(OPK, false)                                             \
+    else if (f.lo[0] || f.hi[0]) KL_CH_LAUNCH1(OPK, true) else KL_CH_LAUNCH1(OPK, false)
+    if (C::SINGLE_GPU && (f.lo[0] || f.hi[0])) return c->fail(KL_ERR_UNSUPPORTED, "launch_chain: single-GPU chain");
     if constexpr (C::VAROP) {
         if (op->kind != KL_OP_ANISO5_VAR || f.lo[0] || f.hi[0])
             return c->fail(KL_ERR_INVALID, "launch_chain: variable-coefficient chain on another operator");

@@ -499,7 +499,8 @@ int kl_create(kl_handle_t *h, int device) {
     if (const char *e = getenv("KL_STENCIL_TAIL")) c->opt_stencil_tail = atoi(e);
     if (const char *e = getenv("KL_STENCIL_STAGGER")) c->opt_stencil_stagger = atoi(e) != 0;
     if (const char *e = getenv("KL_REVERSE")) c->opt_reverse = atoi(e) != 0;
-    if (const char *e = getenv("KL_CG_ONEPASS")) c->opt_cg_onepass = atoi(e) < 0 ? -1 : std::min(atoi(e), 2);
+    if (const char *e = getenv("KL_CG_ONEPASS")) c->opt_cg_onepass = atoi(e) < 0 ? -1 : std::min(atoi(e), 3);
+    if (const char *e = getenv("KL_CG_GROUP")) c->opt_cg_group = std::max(2, std::min(atoi(e), 4));
     if (const char *e = getenv("KL_COOP")) c->opt_coop = atoi(e) != 0;
     if (const char *e = getenv("KL_PERSISTENT")) c->opt_persistent = atoi(e) != 0;
     if (const char *e = getenv("KL_PERSIST_OCC")) c->opt_persist_occ = atoi(e);
@@ -538,7 +539,10 @@ int kl_destroy(kl_handle_t h) {
     if (!h) return KL_OK;
     Ctx *c = h;
     cudaSetDevice(c->device);
-    if (c->stream) cudaStreamSynchronize(c->stream);
+    // a borrowed stream (kl_set_stream) may already be destroyed by its owner -- e.g. another handle whose stream this
+    // one was set to and which was destroyed first -- so it is not touched: wait for the device instead
+    if (c->own_stream && c->stream) cudaStreamSynchronize(c->stream);
+    else cudaDeviceSynchronize();
     for (int r = 0; r < 16; ++r)
         if (c->cb_peer[r] && c->cb_peer[r] != c->cb_local) cudaIpcCloseMemHandle(c->cb_peer[r]);
     cudaFree(c->cb_local);
@@ -646,7 +650,7 @@ int kl_set_option(kl_handle_t h, int key, int value) {
         case KL_OPT_PERSISTENT: h->opt_persistent = value != 0; break;
         case KL_OPT_PUSH_HALO: h->opt_push_halo = value != 0; break;
         case KL_OPT_CG_ONEPASS:
-            if (value < -1 || value > 2) return KL_ERR_INVALID;
+            if (value < -1 || value > 3) return KL_ERR_INVALID;
             h->opt_cg_onepass = value;
             break;
         case KL_OPT_X0:

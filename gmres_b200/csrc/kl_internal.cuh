@@ -38,8 +38,10 @@ constexpr int kMaxDevices = 16;      // per-device launch state (function attrib
 enum SIdx {
     S_ALPHA = 0, S_BETA, S_OMEGA, S_RR, S_PAP, S_RES, S_TOL, S_BETA0, S_HVAL, S_NORM, S_TMP0,
     S_TMP1, S_TMP2, S_TMP3, S_CD, S_CALPHA, S_RHO, S_RHOPREV, S_C1, S_C2, S_THETA, S_SCALE,
-    S_ALPHA_PREV, S_BETA_PREV,     // CG pair mode: alpha and beta of the previous iteration (cg_onepass_scalars)
-    S_RED = 32,            // kMaxRed all-reduced sums land here (S_RED .. S_RED+7)
+    // CG pairs and groups: alpha and beta of the kCgHist iterations before the current one, most recent first
+    // (cg_onepass_scalars)
+    S_ALPHA_HIST, S_BETA_HIST = S_ALPHA_HIST + 3,
+    S_RED = 32,           // kMaxRed all-reduced sums land here (S_RED .. S_RED+7)
     S_LAN = 64,            // lanczos alphas/betas etc.
     S_COUNT = 1024
 };
@@ -157,7 +159,9 @@ struct kl_context_s {
     int opt_stencil_stagger = 0; // staggered tile heights (KL_OPT_STENCIL_STAGGER): measured neutral, off by default
     int opt_stencil_tail = -1;  // lines per CTA in the tapered tail (-1 auto, 0 off), KL_OPT_STENCIL_TAIL
     int opt_pdl = 1;            // programmatic dependent launch between the fused CG kernels (KL_OPT_PDL)
-    int opt_cg_onepass = -1;    // plain CG in chain passes (KL_OPT_CG_ONEPASS): -1 auto, 0 off, 1 one pass per iteration, 2 pairs
+    int opt_cg_onepass = -1;    // plain CG in chain passes (KL_OPT_CG_ONEPASS): -1 auto, 0 off, 1 one pass per iteration, 2 pairs,
+                                // 3 groups
+    int opt_cg_group = 4;       // passes per group of KL_OPT_CG_ONEPASS = 3 (2..4; environment KL_CG_GROUP)
     int opt_x0 = 0;             // x is the initial guess on entry (KL_OPT_X0); no environment variable: it turns an output
                                 // into an input
     // comm

@@ -187,9 +187,12 @@ enum {
     KL_OPT_CG_ONEPASS = 22,   /* plain CG on one GPU with a built-in 5-point operator: 1 = one temporally blocked pass per
                                  iteration (48n B, one reduction; beta predicted from three dot products of the same
                                  pass), 2 = pairs of such passes that store p and x every second iteration only (36n B,
-                                 bit-identical to 1), 0 = two stencil passes (64n B), -1 (default) = one pass from 2^20
-                                 unknowns on (1.3-1.8x faster there on B200; smaller grids, which fit in L2, keep two
-                                 passes), pairs from 2^24 on                                                          */
+                                 bit-identical to 1), 3 = groups of 4 passes: three replay 1..3 iterations from the
+                                 group's stored r, p and store nothing, the fourth replays 4 and stores r, p and x (24n
+                                 B; within rounding of 1: the partial sums of alpha and beta are added in another
+                                 order), 0 = two stencil passes (64n B), -1 (default) = one pass from 2^20 unknowns on
+                                 (1.3-1.8x faster there on B200; smaller grids, which fit in L2, keep two passes), pairs
+                                 from 2^24 on, groups from 2^27 on                                                    */
     KL_OPT_X0 = 23,           /* solver entries (not kl_lanczos): 0 (default) = x is output only and the solve starts from
                                  x = 0, as the reference does; 1 = x is read on entry as the initial guess x0 and
                                  overwritten with the solution (host mode: the nx*ny doubles at x are uploaded and
