@@ -28,6 +28,7 @@ from .api import (  # noqa: F401
     stencil5,
     convdiff,
     stencil5_spectrum,
+    csr,
     cbpr2,
     cheb,
     jacobi_cheb,
@@ -48,9 +49,10 @@ from .api import (  # noqa: F401
     KL_OPT_X0,
     KL_PC_JACOBI_CHEB,
     KL_OP_STENCIL5,
+    KL_OP_CSR,
 )
 
 __all__ = [
     "Handle", "KrylovError", "Operator", "Precond", "GmresResult", "CgResult", "stvec",
-    "stv_poisson", "aniso", "stencil5", "convdiff", "stencil5_spectrum", "cbpr2", "cheb", "jacobi_cheb", "no_precond", "library_path", "load_library",
+    "stv_poisson", "aniso", "stencil5", "convdiff", "stencil5_spectrum", "csr", "cbpr2", "cheb", "jacobi_cheb", "no_precond", "library_path", "load_library",
 ]

@@ -32,6 +32,7 @@ _LIBNAME = "libkrylov_b200.so"
 
 KL_OK, KL_NOT_CONVERGED, KL_BREAKDOWN = 0, 1, 2
 KL_OP_POISSON5, KL_OP_POISSON5_BRANCHY, KL_OP_ANISO5, KL_OP_ANISO5_VAR, KL_OP_STENCIL5, KL_OP_USER = 0, 1, 2, 4, 5, 100
+KL_OP_CSR = 6
 KL_ERR_INVALID, KL_ERR_UNSUPPORTED = -1, -5
 KL_PC_NONE, KL_PC_CBPR2, KL_PC_CHEB, KL_PC_JACOBI_CHEB, KL_PC_USER = 0, 1, 2, 3, 100
 KL_POINTER_HOST, KL_POINTER_DEVICE = 0, 1
@@ -62,6 +63,10 @@ class kl_aniso_var_t(C.Structure):
 
 class kl_stencil5_t(C.Structure):
     _fields_ = [("c", C.c_double), ("wl", C.c_double), ("wr", C.c_double), ("wd", C.c_double), ("wu", C.c_double)]
+
+
+class kl_csr_t(C.Structure):
+    _fields_ = [("nnz", C.c_int64), ("row_ptr", C.c_void_p), ("col_ind", C.c_void_p), ("val", C.c_void_p)]
 
 
 class kl_precond_t(C.Structure):
@@ -161,6 +166,7 @@ class Operator:
     fn: Optional[object] = None  # python callable(d_x:int, d_y:int, nx, ny_local, stream:int) for KL_OP_USER
     coef: Optional[tuple] = None  # (kx, ky) CUDA float64 tensors for KL_OP_ANISO5_VAR
     w5: Optional[tuple] = None    # (c, wl, wr, wd, wu) for KL_OP_STENCIL5
+    csr: Optional[tuple] = None   # (n, row_ptr int64, col_ind int32, val float64) CUDA tensors for KL_OP_CSR
 
     def _c(self):
         o = kl_operator_t()
@@ -172,6 +178,10 @@ class Operator:
             o.user = C.cast(C.pointer(keep), C.c_void_p)
         if self.kind == KL_OP_STENCIL5:
             keep = kl_stencil5_t(*self.w5)
+            o.user = C.cast(C.pointer(keep), C.c_void_p)
+        if self.kind == KL_OP_CSR:
+            _, rp, ci, v = self.csr
+            keep = kl_csr_t(v.numel(), rp.data_ptr(), ci.data_ptr(), v.data_ptr())
             o.user = C.cast(C.pointer(keep), C.c_void_p)
         if self.kind == KL_OP_USER:
             f = self.fn
@@ -284,6 +294,75 @@ def convdiff(px: float, py: float, upwind: bool = False) -> Operator:
     return stencil5((4.0 + 2.0 * ax) + 2.0 * ay, wl, wr, wd, wu)
 
 
+def csr(A, n: Optional[int] = None) -> Operator:
+    """A sparse n x n matrix in CSR form (KL_OP_CSR): a scipy.sparse matrix (converted with tocsr()), a CUDA
+    torch.sparse_csr_tensor, or a tuple (indptr, indices, data) with n given.  Columns need not be sorted and duplicate
+    entries add up.  The arrays are checked here, before anything reaches the device: square, n >= 2 and n < 2^31,
+    values convertible to float64 and finite, indptr starting at 0, nondecreasing and ending at nnz, columns in
+    [0, n).  nnz may exceed 2^31.  The matrix is kept on the device by the returned descriptor (int64 row pointers,
+    int32 columns, float64 values); pass nx = n, ny = 1 where a call takes a grid (the solvers default to it).  One GPU
+    only.  CG, PCG and lanczos trust the caller that the matrix is symmetric."""
+    import torch
+
+    def host(a, what):
+        if hasattr(a, "detach"):
+            a = a.detach().cpu().numpy()
+        try:
+            return np.asarray(a)
+        except Exception as e:  # pragma: no cover
+            raise KrylovError(f"csr: {what} is not an array ({e})")
+
+    if hasattr(A, "tocsr") and hasattr(A, "shape"):
+        M = A.tocsr()
+        shape = M.shape
+        indptr, indices, data = M.indptr, M.indices, M.data
+    elif hasattr(A, "layout") and A.layout == torch.sparse_csr:
+        if not A.is_cuda:
+            raise KrylovError("csr: a torch.sparse_csr_tensor must be on a CUDA device")
+        shape = tuple(A.shape)
+        indptr, indices, data = A.crow_indices(), A.col_indices(), A.values()
+    elif isinstance(A, (tuple, list)) and len(A) == 3:
+        if n is None:
+            raise KrylovError("csr: (indptr, indices, data) needs n")
+        indptr, indices, data = A
+        shape = (int(n), int(n))
+    else:
+        raise KrylovError(f"csr: expected a scipy.sparse matrix, a CUDA torch.sparse_csr_tensor or (indptr, indices, "
+                          f"data), got {type(A).__name__}")
+    if len(shape) != 2 or shape[0] != shape[1]:
+        raise KrylovError(f"csr: the matrix must be square, got shape {shape}")
+    if n is not None and int(n) != shape[0]:
+        raise KrylovError(f"csr: n = {n} but the matrix is {shape[0]} x {shape[1]}")
+    n = int(shape[0])
+    if n < 2 or n >= 2 ** 31:
+        raise KrylovError(f"csr: n = {n} must satisfy 2 <= n < 2^31")
+    ip, ix, dv = host(indptr, "indptr"), host(indices, "indices"), host(data, "data")
+    if ip.ndim != 1 or ix.ndim != 1 or dv.ndim != 1:
+        raise KrylovError("csr: indptr, indices and data must be one-dimensional")
+    if not (np.issubdtype(ip.dtype, np.integer) and np.issubdtype(ix.dtype, np.integer)):
+        raise KrylovError("csr: indptr and indices must be integer arrays")
+    try:
+        dv = np.asarray(dv, dtype=np.float64)
+    except (TypeError, ValueError) as e:
+        raise KrylovError(f"csr: the values are not convertible to float64 ({e})")
+    nnz = dv.size
+    if ip.size != n + 1:
+        raise KrylovError(f"csr: indptr has {ip.size} entries, n + 1 = {n + 1} expected")
+    if ix.size != nnz:
+        raise KrylovError(f"csr: {ix.size} column indices for {nnz} values")
+    ip = ip.astype(np.int64)
+    if ip[0] != 0 or ip[-1] != nnz or np.any(np.diff(ip) < 0):
+        raise KrylovError("csr: indptr must start at 0, be nondecreasing and end at nnz")
+    if nnz and (ix.min() < 0 or ix.max() >= n):
+        raise KrylovError(f"csr: a column index lies outside [0, {n})")
+    if not np.all(np.isfinite(dv)):
+        raise KrylovError("csr: the values must be finite")
+    dev = torch.device("cuda", torch.cuda.current_device())
+    return Operator(KL_OP_CSR, csr=(n, torch.from_numpy(ip).to(dev),
+                                    torch.from_numpy(ix.astype(np.int32)).to(dev),
+                                    torch.from_numpy(np.ascontiguousarray(dv)).to(dev)))
+
+
 def stencil5_spectrum(op: Operator, nx: int, ny: int):
     """(lam_min, lam_max): the exact extremes of the Dirichlet spectrum of a stencil5 operator on an nx x ny grid
     (kl_stencil5_spectrum, host arithmetic, no GPU needed).  Raises KrylovError when the spectrum is complex
@@ -307,9 +386,11 @@ def cheb(degree: int) -> Precond:
 
 
 def jacobi_cheb(degree: int) -> Precond:
-    """Chebyshev of the given degree on the Jacobi-scaled operator D^-1 A (KL_PC_JACOBI_CHEB), for aniso_var operators.
-    Degree 0 is point Jacobi (params ignored); degree k >= 1 takes params = (a, b), an interval of the spectrum of
-    D^-1 A, which lies in (0, 2]."""
+    """Chebyshev of the given degree on the Jacobi-scaled operator D^-1 A (KL_PC_JACOBI_CHEB), for aniso_var and csr
+    operators.  Degree 0 is point Jacobi (params ignored); degree k >= 1 takes params = (a, b), an interval of the
+    spectrum of D^-1 A.  For aniso_var that spectrum lies in (0, 2].  For csr the caller supplies the interval: with a
+    positive diagonal the Gershgorin bound is b = max_i sum_j |a_ij| / a_ii.  A csr matrix with a missing or zero
+    diagonal entry is refused."""
     return Precond(KL_PC_JACOBI_CHEB, int(degree))
 
 
@@ -523,8 +604,10 @@ class Handle:
         return x, xp
 
     @staticmethod
-    def _grid(b, nx, ny):
+    def _grid(b, nx, ny, A=None):
         n = b.numel() if hasattr(b, "numel") else b.size
+        if nx is None and isinstance(A, Operator) and A.kind == KL_OP_CSR:
+            return int(n), 1
         if nx is None:
             # nsize = int(sqrt(real(n)))  (gmres_mgsr.f90:298) -- single precision sqrt
             nx = ny = int(np.sqrt(np.float32(n)))
@@ -558,7 +641,7 @@ class Handle:
     def _gmres(self, fn, A, b, m, tol, M, params, nx, ny, with_pc=True, x0=None):
         self._check_x0(x0, b)
         ba, bp, dev = self._in(b)
-        nx, ny = self._grid(ba, nx, ny)
+        nx, ny = self._grid(ba, nx, ny, A)
         x, xp = self._x_out(ba, dev, x0)
         fe = np.zeros(m)
         ve = np.zeros(m + 1)
@@ -642,7 +725,7 @@ class Handle:
     def _cg(self, fn, A, b, tol, it, M, params, nx, ny, with_pc, x0=None):
         self._check_x0(x0, b)
         ba, bp, dev = self._in(b)
-        nx, ny = self._grid(ba, nx, ny)
+        nx, ny = self._grid(ba, nx, ny, A)
         x, xp = self._x_out(ba, dev, x0)
         itc, res = C.c_int(int(it)), C.c_double(0.0)
         o, keep = A._c()

@@ -56,6 +56,7 @@ enum IIdx {
     I_SKIP3,         // selective reorthogonalisation: 1 = the second update pass of this step is skipped
     I_NSKIP,         // number of skipped second passes ; I_NSKIPCOLS = sum of their column counts
     I_NSKIPCOLS,
+    I_CSR_BAD,       // KL_OP_CSR: the result of k_csr_check (kl_csr.cu csr_validate)
     I_COUNT = 64
 };
 

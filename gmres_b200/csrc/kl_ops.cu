@@ -9,22 +9,34 @@
 namespace kl {
 
 int prob_init(Prob *P, Ctx *c, const kl_operator_t *op, const kl_precond_t *pc, const double *params,
-              int nparams, int nx, int ny) {
+              int nparams, int nx, int ny, bool validate) {
     if (!c || !op) return KL_ERR_INVALID;
     if (op->kind == KL_OP_DENSE) {
         if (nx < 2 || ny != 1) return c->fail(KL_ERR_INVALID, "dense operator: nx = n >= 2, ny = 1");
         if (!op->user) return c->fail(KL_ERR_INVALID, "KL_OP_DENSE without a matrix");
         if (c->nranks > 1) return c->fail(KL_ERR_UNSUPPORTED, "dense operators are single-GPU only");
+    } else if (op->kind == KL_OP_CSR) {
+        if (nx < 2 || ny != 1) return c->fail(KL_ERR_INVALID, "KL_OP_CSR: nx = n >= 2, ny = 1");
+        const kl_csr_t *m = (const kl_csr_t *)op->user;
+        if (!m) return c->fail(KL_ERR_INVALID, "KL_OP_CSR without a matrix");
+        if (m->nnz < 0 || !m->row_ptr || (m->nnz > 0 && (!m->col_ind || !m->val)))
+            return c->fail(KL_ERR_INVALID, "KL_OP_CSR: nnz >= 0, row_ptr and (nnz > 0) col_ind and val non-null");
+        if (c->nranks > 1) return c->fail(KL_ERR_UNSUPPORTED, "KL_OP_CSR is single-GPU only");
     } else if (nx < 2 || ny < 2) return c->fail(KL_ERR_INVALID, "grid must be at least 2x2");
     P->c = c;
     P->op = *op;
     P->w5 = kl_stencil5_t{0.0, 0.0, 0.0, 0.0, 0.0};
+    P->csr = kl_csr_t{0, nullptr, nullptr, nullptr};
     if (pc) P->pc = *pc;
     else P->pc = kl_precond_t{KL_PC_NONE, 0, nullptr, nullptr};
     if (P->op.kind != KL_OP_POISSON5 && P->op.kind != KL_OP_POISSON5_BRANCHY && P->op.kind != KL_OP_ANISO5 &&
         P->op.kind != KL_OP_USER && P->op.kind != KL_OP_DENSE && P->op.kind != KL_OP_ANISO5_VAR &&
-        P->op.kind != KL_OP_STENCIL5)
+        P->op.kind != KL_OP_STENCIL5 && P->op.kind != KL_OP_CSR)
         return c->fail(KL_ERR_INVALID, "unknown operator kind");
+    if (P->op.kind == KL_OP_CSR) {
+        P->csr = *(const kl_csr_t *)op->user;
+        P->op.user = &P->csr;
+    }
     if (P->op.kind == KL_OP_STENCIL5) {
         const kl_stencil5_t *w = (const kl_stencil5_t *)op->user;
         if (!w) return c->fail(KL_ERR_INVALID, "KL_OP_STENCIL5 without weights");
@@ -53,9 +65,9 @@ int prob_init(Prob *P, Ctx *c, const kl_operator_t *op, const kl_precond_t *pc, 
     if ((P->pc.kind == KL_PC_CBPR2 || P->pc.kind == KL_PC_CHEB) && P->nparams < 2)
         return c->fail(KL_ERR_INVALID, "Chebyshev preconditioners need params(1:2)");
     if (P->pc.kind == KL_PC_JACOBI_CHEB) {
-        if (P->op.kind != KL_OP_ANISO5_VAR)
-            return c->fail(KL_ERR_UNSUPPORTED, "KL_PC_JACOBI_CHEB needs KL_OP_ANISO5_VAR; constant-diagonal operators use "
-                                               "KL_PC_CHEB with the interval scaled by their diagonal");
+        if (P->op.kind != KL_OP_ANISO5_VAR && P->op.kind != KL_OP_CSR)
+            return c->fail(KL_ERR_UNSUPPORTED, "KL_PC_JACOBI_CHEB needs KL_OP_ANISO5_VAR or KL_OP_CSR; constant-diagonal "
+                                               "operators use KL_PC_CHEB with the interval scaled by their diagonal");
         if (P->pc.degree < 0) return c->fail(KL_ERR_INVALID, "KL_PC_JACOBI_CHEB: degree >= 0");
         if (P->pc.degree >= 1) {
             if (P->nparams < 2) return c->fail(KL_ERR_INVALID, "KL_PC_JACOBI_CHEB of degree >= 1 needs params(1:2)");
@@ -70,6 +82,7 @@ int prob_init(Prob *P, Ctx *c, const kl_operator_t *op, const kl_precond_t *pc, 
     if (P->nyl < 1) return c->fail(KL_ERR_INVALID, "more ranks than grid lines");
     P->n = (size_t)nx * P->nyl;
     KL_CUDA(c, cudaSetDevice(c->device));
+    if (P->op.kind == KL_OP_CSR && validate) KL_TRY(csr_validate(c, &P->csr, nx, P->pc.kind == KL_PC_JACOBI_CHEB));
     if (c->nranks > 1) {
         size_t need = (size_t)nx * 8 * kChainMaxL;  // 4 slots x {lo,hi} x up to kChainMaxL lines (chained kernels)
         if (c->halo_doubles < need) {
@@ -184,6 +197,7 @@ int op_apply(Prob *P, const double *x, double *y, bool gated) {
         return KL_OK;
     }
     if (P->op.kind == KL_OP_DENSE) return launch_gemv(c, (const double *)P->op.user, P->nx, x, y, gated);
+    if (P->op.kind == KL_OP_CSR) return launch_csr_spmv(c, &P->csr, P->nx, x, y, gated);
     if (!P->builtin_op()) {
         // user callbacks cannot be gated on the device flag; they run unconditionally
         int rc = P->op.fn(P->op.user, x, y, P->nx, P->nyl, (void *)c->stream);
@@ -262,15 +276,20 @@ struct FChebStep : StencilBase<1, (MODE ? 1 : 0)> {
     }
 };
 
-// KL_PC_JACOBI_CHEB (prob_init admits it on KL_OP_ANISO5_VAR only, which runs on one GPU)
+// KL_PC_JACOBI_CHEB (prob_init admits it on KL_OP_ANISO5_VAR and KL_OP_CSR only, which run on one GPU)
 static int pc_jacobi_cheb(Prob *P, const double *r, double *z, double *aux, double *aux2, int mode, bool gated,
                           const PostAny &post) {
     Ctx *c = P->c;
-    const kl_aniso_var_t *cf = (const kl_aniso_var_t *)P->op.user;
+    const bool csr = P->op.kind == KL_OP_CSR;
+    const kl_aniso_var_t *cf = (const kl_aniso_var_t *)P->op.user;   // KL_OP_ANISO5_VAR only
     const int k = P->pc.degree;
     const dim3 grid((unsigned)((P->nx + 255) / 256), (unsigned)P->nyl);
     const int *flags = gated ? c->d_I : nullptr;
     auto pass = [&](const double *zin, double *zout, double theta, double c1, double c2, int kind) {
+        if (csr) {
+            launch_csr_jacobi_cheb_step(c, &P->csr, P->nx, r, zin, aux2, zout, theta, c1, c2, kind, gated);
+            return;
+        }
         k_jacobi_cheb_step<<<grid, 256, 0, c->stream>>>(r, zin, aux2, zout, cf->kx, cf->ky, P->nx, P->nyl, theta, c1, c2,
                                                         kind, flags);
         c->stats.kernel_launches++;
@@ -287,7 +306,8 @@ static int pc_jacobi_cheb(Prob *P, const double *r, double *z, double *aux, doub
         double *zb[2] = {z, aux};
         const int kc = k < kChainMaxL ? k : kChainMaxL;
         int s0 = 0;
-        if (chain_ok(P, kc)) {
+        // chain_ok looks at the grid only; the chained ChJacCheb reads the aniso_var coefficient fields
+        if (!csr && chain_ok(P, kc)) {
             // the first min(k, 6) steps in ONE pass over r, kx, ky (kl_chain_tma.cuh ChJacCheb): 32n B
             double c1s[kChainMaxL], c2s[kChainMaxL];
             for (int s = 0; s < kc; ++s) {
@@ -602,7 +622,8 @@ int kl_apply_operator(kl_handle_t h, const kl_operator_t *A_x, const double *x, 
     if (!h || !A_x || !x || !y) return KL_ERR_INVALID;
     Ctx *c = h;
     Prob P;
-    KL_TRY(prob_init(&P, c, A_x, nullptr, nullptr, 0, nx, ny));
+    // device pointer mode stays enqueue-only (it may run inside a KL_PC_USER callback): no KL_OP_CSR check
+    KL_TRY(prob_init(&P, c, A_x, nullptr, nullptr, 0, nx, ny, c->pointer_mode != KL_POINTER_DEVICE));
     if (c->pointer_mode == KL_POINTER_DEVICE) {
         KL_TRY(op_apply(&P, x, y, false));
         return KL_OK;
@@ -623,7 +644,7 @@ int kl_apply_precond(kl_handle_t h, const kl_precond_t *M_inv, const kl_operator
     if (!h || !A_x || !M_inv || !r || !z) return KL_ERR_INVALID;
     Ctx *c = h;
     Prob P;
-    KL_TRY(prob_init(&P, c, A_x, M_inv, params, nparams, nx, ny));
+    KL_TRY(prob_init(&P, c, A_x, M_inv, params, nparams, nx, ny, c->pointer_mode != KL_POINTER_DEVICE));
     KL_TRY(ws_reserve(c, 4 * ws_need(P.n)));
     ws_reset(c);
     if (c->pointer_mode == KL_POINTER_DEVICE && r != z) {

@@ -17,6 +17,8 @@ struct Prob {
     // KL_OP_STENCIL5: the caller's weights, copied at the start of the call (op.user points here); all zero for the
     // other kinds.  Part of every CUDA-graph key.
     kl_stencil5_t w5;
+    // KL_OP_CSR: the caller's descriptor, copied at the start of the call (op.user points here)
+    kl_csr_t csr;
     bool builtin_op() const {   // the stencil operators (fused kernels); user callbacks and dense matrices take the generic path
         return op.kind == KL_OP_POISSON5 || op.kind == KL_OP_POISSON5_BRANCHY || op.kind == KL_OP_ANISO5 ||
                op.kind == KL_OP_STENCIL5;
@@ -25,8 +27,19 @@ struct Prob {
     bool symmetric() const { return op.kind != KL_OP_STENCIL5 || (w5.wl == w5.wr && w5.wd == w5.wu); }
 };
 
+// `validate`: a KL_OP_CSR matrix is checked on the device (csr_validate, one synchronisation).  Only the
+// device-pointer-mode apply calls pass false: they must stay enqueue-only.
 int prob_init(Prob *P, Ctx *c, const kl_operator_t *op, const kl_precond_t *pc, const double *params,
-              int nparams, int nx, int ny);
+              int nparams, int nx, int ny, bool validate = true);
+
+// KL_OP_CSR (kl_csr.cu).  csr_width: the matrix-wide lane count per row W (krylov_b200.h kl_csr_t).
+int csr_width(int n, long long nnz);
+int launch_csr_spmv(Ctx *c, const kl_csr_t *m, int n, const double *x, double *y, bool gated);
+// one k_csr_jacobi_cheb_step pass (kinds as in k_jacobi_cheb_step)
+int launch_csr_jacobi_cheb_step(Ctx *c, const kl_csr_t *m, int n, const double *r, const double *zin, double *d,
+                                double *z, double theta, double c1, double c2, int kind, bool gated);
+// k_csr_check, read back: KL_ERR_INVALID for malformed index arrays, or (jacobi) a missing or zero diagonal entry
+int csr_validate(Ctx *c, const kl_csr_t *m, int n, bool jacobi);
 
 // Halo buffers: slot s in [0,4) -> lo/hi line of nx doubles each.
 struct Halo {

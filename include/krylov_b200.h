@@ -72,6 +72,10 @@ enum {
                                     then (KL_ERR_UNSUPPORTED), and KL_PC_CBPR2 / KL_PC_CHEB refuse it when its spectrum
                                     is complex (wl*wr < 0 or wd*wu < 0).  It runs through the same fused and temporally
                                     blocked kernels as KL_OP_ANISO5.                                                 */
+    KL_OP_CSR = 6,               /* sparse n x n matrix in CSR form (new): `user` points to a HOST kl_csr_t, nx = n >= 2,
+                                    ny = 1, single GPU only (KL_ERR_UNSUPPORTED on a multi-rank handle).  It takes the
+                                    generic solver path (one kernel per reference loop), like KL_OP_DENSE.  CG, PCG and
+                                    kl_lanczos trust the caller that the matrix is symmetric (positive definite).  */
     KL_OP_USER = 100             /* user callback on device pointers (single GPU only) */
 };
 /* coefficient fields of KL_OP_ANISO5_VAR: cell values kx(i,j), ky(i,j), idx = i + j*nx, DEVICE pointers (kl_vec_alloc /
@@ -97,6 +101,26 @@ typedef struct {
  * (KL_OK).  Otherwise the spectrum is complex: KL_ERR_UNSUPPORTED and both outputs NaN.  Pass [lam_min, lam_max] to
  * KL_PC_CHEB as its interval.                                                                                         */
 int kl_stencil5_spectrum(const kl_stencil5_t *w, int nx, int ny, double *lam_min, double *lam_max);
+/* the matrix of KL_OP_CSR: row i holds the entries k in [row_ptr[i], row_ptr[i+1]), column col_ind[k], value val[k].
+ * DEVICE pointers (row_ptr: n+1 values, col_ind and val: nnz values) that stay valid for the duration of the call.
+ * row_ptr[0] = 0, row_ptr nondecreasing, row_ptr[n] = nnz, 0 <= col_ind[k] < n.  Columns need not be sorted within a
+ * row; duplicate entries add up.  Every solver call, and kl_apply_operator / kl_apply_precond in host pointer mode,
+ * checks these conditions on the device before the first iteration and returns KL_ERR_INVALID when one fails.  The
+ * device-pointer-mode apply calls only enqueue (they may run inside a KL_PC_USER callback) and skip the check; their
+ * kernels still load nothing outside [0, nnz) and [0, n): a row range is clamped to [0, nnz] and an entry whose column
+ * is out of range contributes nothing.
+ * evaluation order of y = A x (every kernel; a CPU twin reproduces it bit for bit):
+ *   W = the smallest power of two >= ceil(nnz / n), clamped to [1, 32]: one width for the whole matrix.
+ *   Row i is served by W lanes.  Lane l sums k = row_ptr[i] + l, + W, + 2W, ... < row_ptr[i+1] in storage order:
+ *     s = 0 ; s = fma(val[k], x[col_ind[k]], s)
+ *   the lanes' sums are combined by an xor butterfly, s = s + shfl_xor(s, off) for off = W/2, ..., 1 (commutative, so
+ *   every lane ends with the same bits), and y[i] = s.                                                               */
+typedef struct {
+    int64_t nnz;
+    const int64_t *row_ptr;
+    const int32_t *col_ind;
+    const double *val;
+} kl_csr_t;
 typedef struct {
     int kind;
     double eps_x, eps_y;  /* KL_OP_ANISO5 */
@@ -114,7 +138,7 @@ enum {
     KL_PC_CBPR2 = 1,  /* chebyshev_precond::cbpr2  src/preconds/chebyshev.f90:8-38 */
     KL_PC_CHEB = 2,   /* degree-k Chebyshev iteration (new; README.md:11)          */
     KL_PC_JACOBI_CHEB = 3, /* degree-k Chebyshev iteration on the Jacobi-scaled operator D^-1 A, D = diag(A), for
-                          KL_OP_ANISO5_VAR only (new).  degree 0: z = D^-1 r (point Jacobi), params ignored; degree
+                          KL_OP_ANISO5_VAR and KL_OP_CSR (new).  degree 0: z = D^-1 r (point Jacobi), params ignored; degree
                           k >= 1: params = (a, b), an interval of the spectrum of D^-1 A in either order.  That
                           spectrum lies in (0, 2] for every positive coefficient field (Gershgorin: the off-diagonal
                           row sums of A are at most its diagonal), so b = 2 needs no estimate, and
@@ -122,7 +146,15 @@ enum {
                           table.  Degree k <= 6 runs as ONE temporally blocked pass (r, kx, ky in, z out: 32n B)
                           on even nx >= 64 with KL_OPT_TMA, KL_OPT_FUSE and KL_OPT_CHAIN on; otherwise, and for
                           the steps beyond the sixth, one pass per step.  Constant-diagonal operators use
-                          KL_PC_CHEB with the interval scaled by their diagonal.                              */
+                          KL_PC_CHEB with the interval scaled by their diagonal.
+                          KL_OP_CSR: D comes from the stored diagonal entries, duplicates summed in the row order of
+                          kl_csr_t (each lane adds its diagonal entries, then the butterfly), dinv = RN(1/a_ii)
+                          recomputed in every pass from the same row scan as A z; one pass per step (r, z, d and the
+                          matrix).  There is no interval for free: the spectrum of D^-1 A lies in (0, b] with the
+                          Gershgorin bound b = max_i sum_j |a_ij| / a_ii for a positive diagonal, and the caller supplies
+                          (a, b).  A missing or zero diagonal entry gives KL_ERR_INVALID (checked with the matrix).
+                          KL_PC_CHEB on KL_OP_CSR gives KL_ERR_UNSUPPORTED, as on every operator that is not a
+                          built-in stencil; KL_PC_CBPR2 runs through the generic path.                        */
     KL_PC_USER = 100
 };
 typedef struct {

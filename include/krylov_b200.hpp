@@ -57,10 +57,22 @@ struct stencil5 {
         return {lo, hi};
     }
 };
+// sparse n x n matrix in CSR form (KL_OP_CSR, krylov_b200.h kl_csr_t): row_ptr, col_ind and val are DEVICE arrays of
+// n+1, nnz and nnz entries.  Pass nx = n, ny = 1.  Like stencil5, the descriptor points at this object, which must
+// outlive the calls it is passed to.
+struct csr {
+    kl_csr_t m;
+    kl_operator_t op;
+    csr(int64_t nnz, const int64_t *row_ptr, const int32_t *col_ind, const double *val)
+        : m{nnz, row_ptr, col_ind, val}, op{KL_OP_CSR, 1.0, 1.0, nullptr, &m} {}
+    csr(const csr &o) : csr(o.m.nnz, o.m.row_ptr, o.m.col_ind, o.m.val) {}
+    csr &operator=(const csr &o) { m = o.m; return *this; }
+    operator const kl_operator_t &() const { return op; }
+};
 inline const kl_precond_t cbpr2{KL_PC_CBPR2, 0, nullptr, nullptr};
 inline const kl_precond_t no_precond{KL_PC_NONE, 0, nullptr, nullptr};
 inline kl_precond_t cheb(int degree) { return kl_precond_t{KL_PC_CHEB, degree, nullptr, nullptr}; }
-// Chebyshev on the Jacobi-scaled operator D^-1 A (variable-coefficient operators only; degree 0 = point Jacobi)
+// Chebyshev on the Jacobi-scaled operator D^-1 A (variable-coefficient and CSR operators only; degree 0 = point Jacobi)
 inline kl_precond_t jacobi_cheb(int degree) { return kl_precond_t{KL_PC_JACOBI_CHEB, degree, nullptr, nullptr}; }
 
 class Handle {
